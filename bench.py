@@ -2,7 +2,7 @@
 """bench.py -- filter-steps/sec of the batched sigma-point filter hot path on N B200s of one node.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload ukfom|usckf|msckf|fusion|ekf|msckf_ekf|safefusion|deadreckon]
-                  [--impl reference]
+                  [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path (predict + update) over one batch of synthetic inputs.  The
 default workload is BASELINE.json configs[3] (the north_star's): the Monte-Carlo USCKF fleet, 4M
@@ -35,6 +35,7 @@ if ROOT not in sys.path:
 from slam_localization_b200 import fleet, synth  # noqa: E402
 
 L2_BYTES = 126 * 1024 * 1024
+DUMP_BYTES = 60 * 10**6         # --dump-outputs: rows written at most; with the .npy headers the files stay under 64 MB
 
 
 def measured_peaks():
@@ -182,6 +183,10 @@ class UkfomWorkload:
     def status_ok(self):
         return all(sum(f.status_counts()) == 0 for f in self.fleets)
 
+    def outputs(self, k):
+        f = self.fleets[k % self.nfleets]
+        return {"mu": f.mu(), "P": f.P(), "status": f.status()}
+
     def stats_tensor(self):
         return self.fleets[0].ensemble_stats().t
 
@@ -240,6 +245,9 @@ class FusionWorkload:
 
     def status_ok(self):
         return True
+
+    def outputs(self, k):
+        return {"x": self.out[0].t, "C": self.out[1].t}
 
     def stats_tensor(self):
         return None
@@ -333,6 +341,9 @@ class UsckfWorkload:
 
     def status_ok(self):
         return sum(self.f.status_counts()) == 0
+
+    def outputs(self, k):
+        return {"mu": self.f.mu(), "P": self.f.P(), "status": self.f.status()}
 
     def stats_tensor(self):
         return self.f.ensemble_stats().t
@@ -434,6 +445,9 @@ class MsckfWorkload:
     def status_ok(self):
         return sum(self.f.status_counts()) == 0
 
+    def outputs(self, k):
+        return {"mu": self.f.mu(), "P": self.f.P(), "status": self.f.status(), "outliers": self.f.outliers()}
+
     def stats_tensor(self):
         return self.f.ensemble_stats().t
 
@@ -500,6 +514,25 @@ def cpu_baseline(wl, steps=3, warmup=1, budget_s=12.0):
                       (nsample, wl.units_per_step(), len(ts), warmup, cores)}, tot / len(ts) * 1e3
 
 
+def dump_outputs(wl, k, out_dir):
+    """Writes what step k of the timed path left for its caller (wl.outputs(k): arrays with one row per instance) as
+    out_dir/<name>.npy in float64, and out_dir/instance.npy with the instances the rows belong to: every instance when
+    all fit in DUMP_BYTES, otherwise a sorted sample drawn with a fixed seed.  Two builds run with the same arguments
+    see the same inputs, so their dumps compare array for array."""
+    import torch
+    arrays = wl.outputs(k)
+    n = wl.units_per_step()
+    assert all(a.shape[0] == n for a in arrays.values())
+    per = 8 * (1 + sum(int(np.prod(a.shape[1:])) for a in arrays.values()))
+    keep = min(n, DUMP_BYTES // per)
+    idx = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = a[torch.from_numpy(idx).to(a.device)].cpu().numpy() if isinstance(a, torch.Tensor) else a[idx]
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float64))
+    np.save(os.path.join(out_dir, "instance.npy"), idx.astype(np.float64))
+
+
 def run_reference(args, rank, world):
     if rank != 0:
         return 0
@@ -515,9 +548,10 @@ def run_reference(args, rank, world):
     return 0
 
 
-def measure(wl, args, ctx, sample_clocks):
+def measure(wl, args, ctx, sample_clocks, dump_dir=None):
     """Runs one workload's device-resident arm, end-to-end arm and stats gather; returns the result dict (rank 0)
-    or None (other ranks).  ctx = (torch, dist, engine, rank, world, local)."""
+    or None (other ranks).  ctx = (torch, dist, engine, rank, world, local).  With dump_dir, rank 0 writes the outputs
+    of the last timed step there (dump_outputs)."""
     torch, dist, engine, rank, world, local = ctx
 
     def barrier():
@@ -578,11 +612,12 @@ def measure(wl, args, ctx, sample_clocks):
     clocks = None
     if rank == 0 and sample_clocks:
         # a timed region shorter than a few sampling periods is followed by untimed steps of the same workload until at
-        # least 5 samples were taken under load; they are not part of any reported time
+        # least 5 samples were taken under load; they are not part of any reported time.  Not when the outputs of the
+        # last timed step are to be written: those steps would move the state on.
         extended = False
         t_end = time.monotonic() + 1.0
         kx = args.warmup + args.steps
-        while sampler.proc and sampler.count(t_load0, t_load1) < 5 and time.monotonic() < t_end:
+        while not dump_dir and sampler.proc and sampler.count(t_load0, t_load1) < 5 and time.monotonic() < t_end:
             for _ in range(8):
                 wl.step(kx)
                 kx += 1
@@ -591,6 +626,8 @@ def measure(wl, args, ctx, sample_clocks):
             extended = True
         clocks = sampler.stop(t_load0, t_load1)
         clocks["sampled_over"] = "timed region + untimed steps of the same workload" if extended else "timed region"
+    if dump_dir and rank == 0:      # before the end-to-end arm below steps the workload again
+        dump_outputs(wl, args.warmup + args.steps - 1, dump_dir)
     ms_max = rank_max(ms)
     units = wl.units_per_step() * args.steps * world
     value = units / (ms_max * 1e-3)
@@ -683,7 +720,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the nested runs of the other BASELINE configs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of the workload computed to DIR/<name>.npy (float64, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3
 
@@ -706,7 +749,7 @@ def main():
     ctx = (torch, dist, engine, rank, world, local)
 
     wl = WORKLOADS[args.workload](rank)
-    line = measure(wl, args, ctx, sample_clocks=True)
+    line = measure(wl, args, ctx, sample_clocks=True, dump_dir=args.dump_outputs)
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         line["cpu_baseline"], _ = cpu_baseline(wl)
     del wl

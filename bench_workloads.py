@@ -1,5 +1,6 @@
 """Bench workloads for the SURVEY 8(f) "next" rows (selected with bench.py --workload ekf|safefusion|deadreckon).
-Same contract as the classes in bench.py: one step = one pass of the row's hot path over one synthetic batch."""
+Same contract as the classes in bench.py: one step = one pass of the row's hot path over one synthetic batch;
+outputs(k) returns what step k left for its caller, one row per instance."""
 import time
 
 import numpy as np
@@ -88,6 +89,9 @@ class EkfWorkload:
     def status_ok(self):
         return bool(self.torch.isfinite(self.f.P.t[:: max(1, self.B // 64)]).all().item())
 
+    def outputs(self, k):
+        return {"err": self.f.err.t, "P": self.f.P.t, "ret": self.ret.t, "accepted": self.f.accepted}
+
     def stats_tensor(self):
         return None
 
@@ -149,6 +153,9 @@ class SafeFusionWorkload:
 
     def status_ok(self):
         return True
+
+    def outputs(self, k):
+        return {"x": self.out[0].t, "C": self.out[1].t}
 
     def stats_tensor(self):
         return None
@@ -220,6 +227,10 @@ class DeadReckonWorkload:
 
     def status_ok(self):
         return bool(self.torch.isfinite(self.pose[self.k & 1].t[:: max(1, self.B // 64)]).all().item())
+
+    def outputs(self, k):
+        b = self.k & 1
+        return {"pose": self.pose[b].t, "cov": self.cov[b].t, "delta_pose": self.dpose.t, "delta_cov": self.dcov.t}
 
     def stats_tensor(self):
         return None
@@ -303,6 +314,9 @@ class MsckfEkfWorkload:
     def status_ok(self):
         c = self.f.status_counts()   # gate rejections (bit 2) are expected; too few rows after the gate (QR_ROWS) is not
         return c[0] == 0 and c[1] == 0 and c[3] == 0 and c[4] == 0
+
+    def outputs(self, k):
+        return {"mu": self.f.mu(), "P": self.f.P(), "status": self.f.status(), "outliers": self.f.outliers()}
 
     def stats_tensor(self):
         return self.f.ensemble_stats().t

@@ -1,7 +1,10 @@
 """Host-side logic of bench.py that needs no GPU: the clock sampler keeps only the nvidia-smi lines that arrived while
-the GPU was under the workload's load, and summarises them (median SM clock, max clock, active throttle reasons)."""
+the GPU was under the workload's load, and summarises them (median SM clock, max clock, active throttle reasons);
+--dump-outputs writes every instance's outputs, or a fixed sample of them, as float64 within its byte budget."""
 import os
 import sys
+
+import numpy as np
 
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import bench  # noqa: E402
@@ -50,3 +53,55 @@ def test_workload_registry_matches_the_documented_names():
     assert sorted(bench.WORKLOADS) == sorted(["ukfom", "usckf", "msckf", "fusion", "ekf", "msckf_ekf", "safefusion", "deadreckon"])
     for name, cls in bench.WORKLOADS.items():
         assert cls.name == name and cls.unit and cls.metric
+        assert callable(getattr(cls, "outputs", None))
+
+
+class _Outputs:
+    """Stands in for a workload after its timed steps: host arrays and (CPU) torch tensors, one row per instance."""
+
+    def __init__(self, n):
+        import torch
+        rng = np.random.default_rng(3)
+        self.n = n
+        self.arrays = {"mu": rng.normal(size=(n, 5)), "P": torch.from_numpy(rng.normal(size=(n, 4, 4))),
+                       "status": np.arange(n, dtype=np.int32) % 3}
+
+    def units_per_step(self):
+        return self.n
+
+    def outputs(self, k):
+        return dict(self.arrays)
+
+
+def _load(d):
+    return {f[:-4]: np.load(os.path.join(d, f)) for f in sorted(os.listdir(d))}
+
+
+def test_dump_outputs_writes_every_instance_when_they_fit(tmp_path):
+    wl = _Outputs(100)
+    bench.dump_outputs(wl, 7, str(tmp_path))
+    got = _load(str(tmp_path))
+    assert sorted(got) == ["P", "instance", "mu", "status"]
+    assert all(a.dtype == np.float64 for a in got.values())
+    np.testing.assert_array_equal(got["instance"], np.arange(100))
+    np.testing.assert_array_equal(got["mu"], wl.arrays["mu"])
+    np.testing.assert_array_equal(got["P"], wl.arrays["P"].numpy())
+    np.testing.assert_array_equal(got["status"], wl.arrays["status"])
+
+
+def test_dump_outputs_samples_a_fixed_subset_within_the_budget(tmp_path, monkeypatch):
+    wl = _Outputs(5000)
+    per = 8 * (1 + 5 + 16 + 1)
+    monkeypatch.setattr(bench, "DUMP_BYTES", 300 * per + 7)
+    a, b = tmp_path / "a", tmp_path / "b"
+    bench.dump_outputs(wl, 0, str(a))
+    bench.dump_outputs(wl, 0, str(b))
+    ga, gb = _load(str(a)), _load(str(b))
+    idx = ga["instance"].astype(np.int64)
+    assert len(idx) == 300 and np.all(np.diff(idx) > 0) and idx[-1] < 5000 and idx[-1] > 2500
+    assert sum(v.nbytes for v in ga.values()) <= bench.DUMP_BYTES
+    np.testing.assert_array_equal(ga["mu"], wl.arrays["mu"][idx])
+    np.testing.assert_array_equal(ga["P"], wl.arrays["P"].numpy()[idx])
+    np.testing.assert_array_equal(ga["status"], wl.arrays["status"][idx])
+    for k in ga:
+        np.testing.assert_array_equal(ga[k], gb[k])
