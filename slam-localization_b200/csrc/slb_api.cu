@@ -59,7 +59,7 @@ __global__ void soa_to_dense_P(const double *soa, double *dense, int B0, int cnt
     if (c > r) { const int x = r; r = c; c = x; }
     dense[t] = soa[(size_t)(r * (r + 1) / 2 + c) * stride + B0 + i];
 }
-// USCKF / MSCKF kinds: instance-major records, P packed lower
+// USCKF / MSCKF kinds: instance-major records; P is packed lower (MSCKF, tri) or tiled (USCKF, prec)
 __global__ void aos_to_rec_mu(const double *aos, double *rec, int B0, int cnt, int QD, int qstride) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= cnt * QD) return;
@@ -72,20 +72,20 @@ __global__ void rec_to_aos_mu(const double *rec, double *aos, int B0, int cnt, i
     const int i = t / QD, c = t - i * QD;
     aos[t] = rec[(size_t)(B0 + i) * qstride + off + c];
 }
-__global__ void dense_to_rec_P(const double *dense, double *rec, int B0, int cnt, int N, int pstride) {
+__global__ void dense_to_rec_P(const double *dense, double *rec, int B0, int cnt, int N, int pstride, bool tiled) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= (int64_t)cnt * N * N) return;
     const int i = (int)(t / (N * N)), rc = (int)(t - (int64_t)i * N * N);
     const int r = rc / N, c = rc - r * N;
-    if (c <= r) rec[(size_t)(B0 + i) * pstride + r * (r + 1) / 2 + c] = dense[t];
+    if (c <= r) rec[(size_t)(B0 + i) * pstride + (tiled ? slbd::prec(N, r, c) : slbd::tri(r, c))] = dense[t];
 }
-__global__ void rec_to_dense_P(const double *rec, double *dense, int B0, int cnt, int N, int pstride) {
+__global__ void rec_to_dense_P(const double *rec, double *dense, int B0, int cnt, int N, int pstride, bool tiled) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= (int64_t)cnt * N * N) return;
     const int i = (int)(t / (N * N)), rc = (int)(t - (int64_t)i * N * N);
     int r = rc / N, c = rc - r * N;
     if (c > r) { const int x = r; r = c; c = x; }
-    dense[t] = rec[(size_t)(B0 + i) * pstride + r * (r + 1) / 2 + c];
+    dense[t] = rec[(size_t)(B0 + i) * pstride + (tiled ? slbd::prec(N, r, c) : slbd::tri(r, c))];
 }
 
 // fleet initialisation: instance i <- instance i % count (Monte-Carlo replicas of `count` priors)
@@ -356,7 +356,7 @@ int slb_device_ptr(slb_handle h, int field, void **dev) {
 static int transfer(slb_handle h, int field, void *host, size_t count, cudaStream_t s, bool up) {
     if (!h || !host) return set_error(SLB_ERR_INVALID, "slb_upload/download: null argument");
     DeviceGuard guard(h->cfg.device);
-    const bool soa = h->cfg.kind == SLB_KIND_UKF;
+    const bool soa = h->cfg.kind == SLB_KIND_UKF, tiled = h->cfg.kind == SLB_KIND_USCKF;
     if (field == SLB_FIELD_STATUS || field == SLB_FIELD_OUTLIERS) {
         if (up) return set_error(SLB_ERR_INVALID, "slb_upload: status fields are read-only");
         if (count != (size_t)h->B) return set_error(SLB_ERR_INVALID, "slb_download: count must equal batch");
@@ -387,7 +387,7 @@ static int transfer(slb_handle h, int field, void *host, size_t count, cudaStrea
                 else aos_to_rec_mu<<<grid, tpb, 0, s>>>(h->stage, h->mu, b0, cnt, h->QD, h->qstride);
             } else {
                 if (soa) dense_to_soa_P<<<grid, tpb, 0, s>>>(h->stage, h->P, b0, cnt, h->N, h->stride);
-                else dense_to_rec_P<<<grid, tpb, 0, s>>>(h->stage, h->P, b0, cnt, h->N, h->pstride);
+                else dense_to_rec_P<<<grid, tpb, 0, s>>>(h->stage, h->P, b0, cnt, h->N, h->pstride, tiled);
             }
             count_launch();
             SLB_CUDA(cudaGetLastError());
@@ -397,7 +397,7 @@ static int transfer(slb_handle h, int field, void *host, size_t count, cudaStrea
                 else rec_to_aos_mu<<<grid, tpb, 0, s>>>(h->mu, h->stage, b0, cnt, h->QD, h->qstride);
             } else {
                 if (soa) soa_to_dense_P<<<grid, tpb, 0, s>>>(h->P, h->stage, b0, cnt, h->N, h->stride);
-                else rec_to_dense_P<<<grid, tpb, 0, s>>>(h->P, h->stage, b0, cnt, h->N, h->pstride);
+                else rec_to_dense_P<<<grid, tpb, 0, s>>>(h->P, h->stage, b0, cnt, h->N, h->pstride, tiled);
             }
             count_launch();
             SLB_CUDA(cudaGetLastError());

@@ -16,6 +16,7 @@ struct ChkLayout {
     unsigned long long so3mask;   // bit b: block b is SO3
     int nfeat;                    // trailing plain scalars
     int N, QD, NP, pstride, qstride;
+    int tiled;                    // 1: P records in the USCKF tile layout (prec), 0: packed row-major (tri)
 };
 
 SLB_DEV double warp_max(double v) {
@@ -32,8 +33,10 @@ __global__ void __launch_bounds__(32) check_sigma_points_kernel(const double *mu
     double *Lp = sm, *Pa = Lp + NP, *D = Pa + NP, *mus = D + 32 * N, *ref = mus + QD, *md = ref + QD;
     for (int inst = blockIdx.x; inst < B; inst += gridDim.x) {
         const double *Pg = P + (size_t)inst * l.pstride, *mug = mu + (size_t)inst * l.qstride;
+        auto rec = [&](int i, int j) { return l.tiled ? prec(N, i, j) : tri(i, j); };   // P(i, j), i >= j, in the record
         __syncwarp();
-        for (int e = lane; e < NP; e += 32) { Lp[e] = Pg[e]; Pa[e] = 0.0; }
+        for (int i = 0; i < N; ++i)
+            for (int j = lane; j <= i; j += 32) { Lp[tri(i, j)] = Pg[rec(i, j)]; Pa[tri(i, j)] = 0.0; }
         for (int e = lane; e < QD; e += 32) { mus[e] = mug[e]; ref[e] = mug[e]; }
         __syncwarp();
         // ---- Eigen::LLT of Pk (lower triangle, Q8), right-looking, rows dealt to lanes -------------------------
@@ -152,7 +155,8 @@ __global__ void __launch_bounds__(32) check_sigma_points_kernel(const double *mu
         }
         __syncwarp();
         double dP = 0.0;
-        for (int e = lane; e < NP; e += 32) dP = fmax(dP, fabs(Pa[e] - Pg[e]));
+        for (int i = 0; i < N; ++i)
+            for (int j = lane; j <= i; j += 32) dP = fmax(dP, fabs(Pa[tri(i, j)] - Pg[rec(i, j)]));
         dP = warp_max(dP);
         // |muX [-] mu|_inf: ref [-] mus, block per lane
         double dm = 0.0;
@@ -193,6 +197,7 @@ int launch_check_sigma_points(const slb_batch_s *h, int32_t *flags, double *diff
     slbd::ChkLayout l;
     l.N = h->N; l.QD = h->QD; l.NP = h->NP; l.pstride = h->pstride; l.qstride = h->qstride;
     l.so3mask = 0;
+    l.tiled = h->cfg.kind == SLB_KIND_USCKF;
     if (h->cfg.kind == SLB_KIND_USCKF) {
         l.nblk = 12; l.nfeat = h->cfg.nk + h->cfg.nl;
         l.so3mask = (1ull << 1) | (1ull << 5) | (1ull << 9);

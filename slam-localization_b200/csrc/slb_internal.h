@@ -17,7 +17,8 @@ struct slb_batch_s {
     int pstride;  // USCKF/MSCKF: doubles per instance record of P (NP rounded up to 16 -> 128 B)
     int qstride;  // USCKF/MSCKF: doubles per instance record of mu (QD rounded up to 2 -> 16 B)
     double *mu;   // UKF: [QD][stride] SoA.  USCKF/MSCKF: [B][qstride]
-    double *P;    // UKF: [NP][stride] SoA packed lower.  USCKF/MSCKF: [B][pstride] packed lower
+    double *P;    // UKF: [NP][stride] SoA packed lower.  MSCKF: [B][pstride] packed lower (tri).  USCKF: [B][pstride]
+                  // 8 x 8 tiles in DMMA accumulator order (prec, slb_math.cuh), the same NP doubles
     int32_t *status;
     int32_t *outliers;
     // staging for the *_host entry points and upload/download

@@ -33,6 +33,18 @@ typedef Layout<4, 0x2> LayState12;  // pos, orient, velo, angvelo       (State)
 
 SLB_HD constexpr int tri(int i, int j) { return i * (i + 1) / 2 + j; }  // i >= j
 
+// Offset of P(i, j), i >= j, in a USCKF record of dimension N: the lower block triangle of 8 x 8 tiles, tile rows in
+// order, within a tile row the off-diagonal tiles first (row-major, 8 columns each), then the diagonal tile (its packed
+// lower triangle).  The last tile row holds only its h = N - 8 (ceil(N / 8) - 1) live rows (h x 8 tiles, an h-row
+// triangle), so tile row I starts where packed row 8 I would, at tri(8 I, 0), and the record is N (N + 1) / 2 doubles
+// like the packed triangle.  Row-major inside a tile is the DMMA m8n8k4 accumulator order: lane 4 b + a holds entries
+// (b, 2 a), (b, 2 a + 1) of a tile, i.e. doubles 2 lane and 2 lane + 1 of an off-diagonal tile, one aligned 16-byte
+// access.  (MSCKF records and UKF arrays keep the packed row-major triangle, tri().)
+SLB_HD constexpr int prec(int N, int i, int j) {
+    const int I = i >> 3, J = j >> 3, h = N - 8 * I < 8 ? N - 8 * I : 8;
+    return tri(8 * I, 0) + 8 * h * J + (J < I ? 8 * (i & 7) + (j & 7) : tri(i & 7, j & 7));
+}
+
 // ---- SO3 -----------------------------------------------------------------------------------------
 // Sigma-point deviations are small rotations, so exp / log almost always see small arguments.  Both
 // have a branch-free polynomial fast path (minimax fits, relative error < 5e-18 before rounding) that

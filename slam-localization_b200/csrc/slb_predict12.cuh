@@ -137,8 +137,8 @@ SLB_DEV void dmma884(double &d0, double &d1, double a, double b) {
 // =====================================================================================================
 // predict
 // =====================================================================================================
-constexpr int PRED_PR = 366;           // packed rows 24..35: T(36) - T(24) (USCKF; MSCKF uses 78 of it)
-constexpr int PRED_PF = 28 * 12;       // feature-row segments, nk + nl <= 28
+constexpr int PRED_PR = 520;           // USCKF: tile rows 3..4 (rows 24..39), prec(N, 40, 0) - prec(N, 24, 0); MSCKF uses 78 of it
+constexpr int PRED_PF = 8 * 12;        // USCKF: 12-wide segments of the feature rows below the span (rows 40..47)
 constexpr int PRED_DS = 20;            // row stride of the deviations D and of Fk (= 4 mod 16: conflict-free fragments)
 constexpr int PRED_LS = 78 + 16;       // factor, column-major packed (+ pad for the tile overhang)
 // doubles per warp (even: 16-B aligned warps for the bulk copy; last slot = mbarrier)
@@ -167,26 +167,41 @@ __global__ void __launch_bounds__(WPB * 32, 2) predict12_kernel(slb::FilterArgs 
     if (inst >= a.B) return;
     double *Pr = smem + (size_t)w * PRED_SM, *Pf = Pr + PRED_PR, *Ls = Pf + PRED_PF, *D = Ls + PRED_LS, *W = D + 28 * PRED_DS,
            *Fk = W + 144, *rsd = Fk + 12 * PRED_DS;
-    const int nf = CROSS ? a.nk + a.nl : 0;
-    constexpr int T0 = ROW0 * (ROW0 + 1) / 2, T1 = (ROW0 + 12) * (ROW0 + 13) / 2, SPAN = T1 - T0;
-    static_assert(SPAN <= PRED_PR, "row span");
+    // USCKF (CROSS) records are tiled (prec): the block's rows 24..35 lie in tile rows 3 and 4, which the span covers
+    // whole (rows 24..min(N, 40) - 1, feature rows 36..39 included); MSCKF records are packed (tri): rows ROW0..ROW0+11.
+    static_assert(!CROSS || ROW0 == 24, "the tiled span is tile rows 3..4");
+    const int nf = CROSS ? a.nk + a.nl : 0, N = CROSS ? 36 + nf : ROW0 + 12;
+    constexpr int T0 = ROW0 * (ROW0 + 1) / 2, T1 = (ROW0 + 12) * (ROW0 + 13) / 2;
+    constexpr int RS = CROSS ? 40 : ROW0 + 12;         // first record row after the span
+    constexpr int NFS = RS - 36;                        // CROSS: feature rows inside the span
+    const int SPAN = CROSS ? tri(min(N, RS), 0) - T0 : T1 - T0;
+    const int nfr = CROSS && nf > NFS ? nf - NFS : 0;   // feature rows below the span
+    static_assert(tri(RS, 0) - T0 <= PRED_PR && (!CROSS || 12 * (48 - RS) <= PRED_PF), "row span");
     double *Pg = a.P + (size_t)inst * a.pstride;
     double *mug = a.mu + (size_t)inst * a.qstride;
-    auto PR = [&](int r, int c) -> double & { return Pr[tri(ROW0 + r, c) - T0]; };  // row ROW0+r, col c
+    auto PR = [&](int r, int c) -> double & {   // row ROW0+r, col c
+        return Pr[(CROSS ? prec(N, ROW0 + r, c) : tri(ROW0 + r, c)) - T0];
+    };
+    auto PF = [&](int fr, int c) -> double & {   // feature row fr, col 24 + c
+        return fr < NFS ? PR(12 + fr, 24 + c) : Pf[(fr - NFS) * 12 + c];
+    };
     const int a_ = lane & 3, b_ = lane >> 2;  // 2D-cyclic tile coordinates == DMMA fragment coordinates (row, k)
 
-    // The block's rows are one contiguous span of the packed record: one TMA bulk copy (UBLKCP) brings it in,
-    // the 12-wide feature-row segments follow as LDGSTS; the mean and the control input load meanwhile.
-    static_assert((T0 * 8) % 16 == 0 && (SPAN * 8) % 16 == 0 && PRED_SM % 2 == 0, "bulk copy needs 16-byte alignment");
+    // The block's rows are one contiguous span of the record: one TMA bulk copy (UBLKCP) brings it in, the 12-wide
+    // segments of the feature rows below it follow as LDGSTS; the mean and the control input load meanwhile.  The
+    // USCKF shapes have N = 39 or N >= 40.
+    static_assert((T0 * 8) % 16 == 0 && ((T1 - T0) * 8) % 16 == 0 && PRED_SM % 2 == 0 &&
+                      (!CROSS || (((tri(RS, 0) - T0) * 8) % 16 == 0 && ((tri(39, 0) - T0) * 8) % 16 == 0)),
+                  "bulk copy needs 16-byte alignment");
     uint64_t *bar = reinterpret_cast<uint64_t *>(rsd + 16);
     if (lane == 0) {
         mbar_init(bar, 1);
         mbar_expect_tx(bar, SPAN * 8);
         bulk_g2s(Pr, Pg + T0, SPAN * 8, bar);
     }
-    for (int e = lane; e < nf * 12; e += 32) {
+    for (int e = lane; e < nfr * 12; e += 32) {
         const int r = e / 12, c = e - r * 12;
-        pred_cp_async8(Pf + e, Pg + tri(36 + r, 24 + c));
+        pred_cp_async8(Pf + e, Pg + prec(N, RS + r, 24 + c));
     }
     double mu[13];
 #pragma unroll
@@ -346,7 +361,7 @@ __global__ void __launch_bounds__(WPB * 32, 2) predict12_kernel(slb::FilterArgs 
                     const int fr = min(8 * I + b_, nf - 1);
 #pragma unroll
                     for (int k0 = 0; k0 < 12; k0 += 4) {
-                        const double av = Pf[fr * 12 + k0 + a_];
+                        const double av = PF(fr, k0 + a_);
                         dmma884(of[I][0][0], of[I][0][1], av, Fk[c0 * PRED_DS + k0 + a_]);  // B[k][n] = Fk[n][k]
                         dmma884(of[I][1][0], of[I][1][1], av, Fk[c1 * PRED_DS + k0 + a_]);
                     }
@@ -354,20 +369,21 @@ __global__ void __launch_bounds__(WPB * 32, 2) predict12_kernel(slb::FilterArgs 
             }
         }
         __syncwarp();
+        // rows 24..35 x cols 0..23 are off-diagonal tiles of tile rows 3 and 4: one 16-byte store per lane and tile
 #pragma unroll
         for (int I = 0; I < 2; ++I)
 #pragma unroll
-            for (int J = 0; J < 3; ++J) {
-                const int r = 8 * I + b_, c = 8 * J + 2 * a_;
-                if (r < 12) { PR(r, c) = oc[I][J][0]; PR(r, c + 1) = oc[I][J][1]; }
-            }
+            for (int J = 0; J < 3; ++J)
+                if (8 * I + b_ < 12)
+                    *reinterpret_cast<double2 *>(Pr + prec(N, ROW0 + 8 * I, 8 * J) - T0 + 2 * lane) =
+                        make_double2(oc[I][J][0], oc[I][J][1]);
 #pragma unroll
         for (int I = 0; I < 4; ++I)
             if (I < nft) {
 #pragma unroll
                 for (int J = 0; J < 2; ++J) {
                     const int fr = 8 * I + b_, c = 8 * J + 2 * a_;
-                    if (fr < nf && c < 12) { Pf[fr * 12 + c] = of[I][J][0]; Pf[fr * 12 + c + 1] = of[I][J][1]; }
+                    if (fr < nf && c < 12) { PF(fr, c) = of[I][J][0]; PF(fr, c + 1) = of[I][J][1]; }
                 }
             }
         __syncwarp();
@@ -376,9 +392,9 @@ __global__ void __launch_bounds__(WPB * 32, 2) predict12_kernel(slb::FilterArgs 
     }
     // ---- write back --------------------------------------------------------------------------------------
     for (int e = lane; e < SPAN; e += 32) Pg[T0 + e] = Pr[e];
-    for (int e = lane; e < nf * 12; e += 32) {
+    for (int e = lane; e < nfr * 12; e += 32) {
         const int r = e / 12, c = e - r * 12;
-        Pg[tri(36 + r, 24 + c)] = Pf[e];
+        Pg[prec(N, RS + r, 24 + c)] = Pf[e];
     }
     bool finite = true;
 #pragma unroll

@@ -2,11 +2,12 @@
 // setMeasurement (src/filters/Usckf.hpp), one filter instance per WARP.
 //
 // Instance record in HBM: mu[qstride] (statek 13 | statek_l 13 | statek_i 13 | featuresk | featuresk_l)
-// and the lower triangle of Pk packed row-major, P[T(i)+j], T(i) = i(i+1)/2, padded to 128 B.
+// and the lower triangle of Pk as 8 x 8 tiles in DMMA accumulator order, P[prec(N, i, j)] (slb_math.cuh): off-diagonal
+// tiles row-major, diagonal tiles packed lower, N(N+1)/2 doubles padded to 128 B.
 // A record is contiguous, so a warp streams it with one TMA bulk copy (cp.async.bulk -> UBLKCP).
 //
-// predict (Usckf.hpp:113-244) touches only statek_i: rows 24..35 of the packed triangle (one
-//   contiguous 366-double span) and the 12-wide segments of the feature rows.  Lane s evaluates sigma
+// predict (Usckf.hpp:113-244) touches only statek_i: rows 24..35, i.e. tile rows 3 and 4 (rows 24..39, one
+//   contiguous span of 520 doubles at N >= 40), and the 12-wide segments of the feature rows below.  Lane s evaluates sigma
 //   point s (25 of 32 lanes); Fk = Pxy^T Pii^-1 is obtained as W^T L^-1 with W = 0.5 (dY+ - dY-) by a
 //   triangular solve, because X_i [-] mu_old is +-L e_j by construction (same algebra as :152-154,
 //   without the explicit inverse).
@@ -28,7 +29,9 @@ __global__ void usckf_clone_kernel(slb::FilterArgs a, int mode) {
     if (t >= (int64_t)a.B * per) return;
     const int inst = (int)(t / per), e = (int)(t - (int64_t)inst * per);
     double *P = a.P + (size_t)inst * a.pstride, *mu = a.mu + (size_t)inst * a.qstride;
-    auto sym = [&](int r, int c) { return r >= c ? P[tri(r, c)] : P[tri(c, r)]; };
+    const int N = 36 + a.nk + a.nl;
+    auto at = [&](int r, int c) -> double & { return P[prec(N, r, c)]; };   // r >= c
+    auto sym = [&](int r, int c) { return r >= c ? at(r, c) : at(c, r); };
     if (e < 13) {
         if (mode == SLB_STATEK_I) mu[13 + e] = mu[26 + e];   // statek_l = statek_i (:401)
         else mu[e] = mu[13 + e];                              // statek = statek_l (:419)
@@ -39,26 +42,26 @@ __global__ void usckf_clone_kernel(slb::FilterArgs a, int mode) {
         if (blk == 0) {
             // Pk+l = Pk+i (:405) and Pk+i|k+l = Pk+i (:406-407)
             const double v = sym(24 + r, 24 + c);
-            if (c <= r) P[tri(12 + r, 12 + c)] = v;
-            P[tri(24 + r, 12 + c)] = v;
+            if (c <= r) at(12 + r, 12 + c) = v;
+            at(24 + r, 12 + c) = v;
         } else {
             // cross blocks with statek zeroed (:410-413)
-            P[tri(24 + r, c)] = 0.0;
-            P[tri(12 + r, c)] = 0.0;
+            at(24 + r, c) = 0.0;
+            at(12 + r, c) = 0.0;
         }
     } else if (blk == 0) {
         // Pk = Pk+l, Pk|k+l = Pk+l (:422-425)
         const double v = sym(12 + r, 12 + c);
-        if (c <= r) P[tri(r, c)] = v;
-        P[tri(12 + r, c)] = v;
+        if (c <= r) at(r, c) = v;
+        at(12 + r, c) = v;
     }
 }
 // The cloning kernel reads blocks other threads overwrite only in STATEK_I blk 0 (reads P_ii, writes
 // P_ll / P_il) and STATEK_L blk 0 (reads P_ll, writes P_kk / P_lk): sources and destinations are disjoint.
 
 __global__ void usckf_set_measurement_kernel(slb::FilterArgs a, int mode) {
-    const int N = 36 + a.nk + a.nl, NP = N * (N + 1) / 2;
-    const int nfe = NP - 666;  // packed entries of rows 36..N-1
+    const int N = 36 + a.nk + a.nl;
+    const int nfe = (N - 36) * N;  // rows 36..N-1 x all columns (entries above the diagonal do nothing)
     const int per = nfe + (mode == SLB_STATEK ? a.nk : a.nl);
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= (int64_t)a.B * per) return;
@@ -71,17 +74,16 @@ __global__ void usckf_set_measurement_kernel(slb::FilterArgs a, int mode) {
         mu[39 + f0 + c] = a.z[(size_t)inst * len + c];  // featuresk / featuresk_l = z (:335,:362)
         return;
     }
-    int r = 36;
-    while (tri(r + 1, 0) - 666 <= e) ++r;
-    const int c = e - (tri(r, 0) - 666);
+    const int r = 36 + e / N, c = e - (r - 36) * N;
+    if (c > r) return;
     const int fr = r - 36, fc = c - 36;
     double v = 0.0;  // Pk.setZero() (:348,:376): every state<->feature and k<->k+l cross term
     if (c >= 36) {
         const bool rin = fr >= f0 && fr < f0 + len, cin = fc >= f0 && fc < f0 + len;
         if (rin && cin) v = a.R[(fr - f0) * len + (fc - f0)];      // new block = R (:353,:381)
-        else if (!rin && !cin) v = P[tri(r, c)];                    // the block that stays (:355,:383)
+        else if (!rin && !cin) v = P[prec(N, r, c)];                // the block that stays (:355,:383)
     }
-    P[tri(r, c)] = v;
+    P[prec(N, r, c)] = v;
 }
 
 }  // namespace slbd
@@ -104,6 +106,23 @@ static int launch_predict_t(const FilterArgs &a, cudaStream_t s) {
 // (State.hpp:539-540, setMeasurement resizes Pk, Usckf.hpp:346-348); a batch has fixed sizes chosen at slb_create,
 // which rejects what is not in this list.  N = 36 + nk + nl <= 48 keeps the accumulator tiles in registers.
 #define SLB_USCKF_SHAPES(X) X(3, 0) X(3, 3) X(3, 6) X(3, 9) X(6, 0) X(6, 3) X(6, 6) X(9, 0) X(9, 3)
+// the tiled record layout (prec) places every entry of the lower triangle once inside the N(N+1)/2 doubles of the
+// packed one, and every off-diagonal tile row it holds starts on a 16-byte boundary
+static constexpr bool prec_fills_record(int N) {
+    bool seen[48 * 49 / 2] = {};
+    for (int i = 0; i < N; ++i)
+        for (int j = 0; j <= i; ++j) {
+            const int o = slbd::prec(N, i, j);
+            if (o < 0 || o >= N * (N + 1) / 2 || seen[o]) return false;
+            if ((j & 7) == 0 && (j >> 3) < (i >> 3) && o % 2 != 0) return false;
+            seen[o] = true;
+        }
+    return true;
+}
+#define SLB_USCKF_SHAPE(NK_, NL_) static_assert(prec_fills_record(36 + NK_ + NL_), "USCKF record layout");
+SLB_USCKF_SHAPES(SLB_USCKF_SHAPE)
+#undef SLB_USCKF_SHAPE
+
 bool usckf_shape_supported(int nk, int nl) {
 #define SLB_USCKF_SHAPE(NK_, NL_) \
     if (nk == NK_ && nl == NL_) return true;
@@ -192,7 +211,7 @@ int launch_usckf_set_measurement(int mode, const FilterArgs &a, cudaStream_t s) 
     const int N = 36 + a.nk + a.nl;
     const int len = mode == SLB_STATEK ? a.nk : a.nl;
     if (len == 0) return SLB_OK;
-    const int64_t work = (int64_t)a.B * (N * (N + 1) / 2 - 666 + len);
+    const int64_t work = (int64_t)a.B * ((N - 36) * N + len);
     slbd::usckf_set_measurement_kernel<<<(unsigned)((work + 255) / 256), 256, 0, s>>>(a, mode);
     count_launch();
     SLB_CUDA(cudaGetLastError());

@@ -1,7 +1,9 @@
 // slb_usckf_step.cuh -- localization::Usckf predict (Usckf.hpp:107-244) and update (:246-308) of one filter
-// instance per WARP with the instance record RESIDENT IN SHARED MEMORY: one TMA bulk load brings the packed lower
-// triangle of Pk (and the mean) in, predict and update work on it in place, one TMA bulk store writes it back, so a
-// fused predict+update step moves exactly the algorithmic bytes (record in + record out) through HBM.
+// instance per WARP with the instance record RESIDENT IN SHARED MEMORY: one TMA bulk load brings the lower triangle
+// of Pk (tiled, prec) and the mean in, predict and update work on it in place, one TMA bulk store writes it back, so a
+// fused predict+update step moves exactly the algorithmic bytes (record in + record out) through HBM.  The record's
+// off-diagonal 8 x 8 tiles are stored in accumulator order: moving one between the record and the DMMA accumulators
+// is one conflict-free 16-byte access per lane.
 //
 // update: the N x N factorisation is a BLOCKED right-looking one in the square-root-free form Pk = U D^-1 U^T
 //   (L(:,k) = U(:,k) / sqrt(d_k), see CholStep in slb_predict12.cuh for the scalar version): panels of 4 columns, the
@@ -397,17 +399,23 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
            *dl = Cs + NPAD * KP;
     UpdState<C> s;
     s.ok = true;
-    // ---- the lower triangle of Pk from the resident record into the accumulator tiles; diagonal tiles are filled
-    //      symmetrically, rows / columns beyond N (N % 8 != 0) are an identity block --------------------------------
+    // ---- the lower triangle of Pk from the resident record into the accumulator tiles: an off-diagonal tile is stored
+    //      in accumulator order (one 16-byte load per lane), diagonal tiles are filled symmetrically from their packed
+    //      triangle, rows / columns beyond N (N % 8 != 0) are an identity block ------------------------------------
     auto elem = [&](int i, int j) -> double {
         if (i >= N || j >= N) return i == j ? 1.0 : 0.0;
-        return i >= j ? Ps[tri(i, j)] : Ps[tri(j, i)];
+        return i >= j ? Ps[prec(N, i, j)] : Ps[prec(N, j, i)];
     };
 #pragma unroll
     for (int I = 0; I < NT; ++I)
 #pragma unroll
         for (int J = 0; J <= JLAST; ++J)
-            if (J <= I) {
+            if (J < I) {
+                double2 v = make_double2(0.0, 0.0);
+                if (8 * I + b_ < N) v = *reinterpret_cast<const double2 *>(Ps + prec(N, 8 * I, 8 * J) + 2 * lane);
+                s.c0[I][J] = v.x;
+                s.c1[I][J] = v.y;
+            } else if (J == I) {
                 const int i = 8 * I + b_, j = 8 * J + 2 * a_;
                 s.c0[I][J] = elem(i, j);
                 s.c1[I][J] = elem(i, j + 1);
@@ -537,12 +545,21 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
 #pragma unroll
             for (int J = 0; J <= I; ++J) {
                 const int i = 8 * I + b_, j = 8 * J + 2 * a_;
-                const bool w0 = i < N && j <= i, w1 = i < N && j + 1 <= i;
-                double p0 = w0 ? Ps[tri(i, j)] : 0.0, p1 = w1 ? Ps[tri(i, j + 1)] : 0.0;
+                if (J < I) {   // off-diagonal tile: one 16-byte read-modify-write per lane
+                    double2 *pp = reinterpret_cast<double2 *>(Ps + prec(N, 8 * I, 8 * J) + 2 * lane);
+                    const bool w = i < N;
+                    double2 p = w ? *pp : make_double2(0.0, 0.0);
 #pragma unroll
-                for (int kk = 0; kk < KP / 4; ++kk) dmma884(p0, p1, fa[I][kk], fb[J][kk]);
-                if (w0) Ps[tri(i, j)] = p0;
-                if (w1) Ps[tri(i, j + 1)] = p1;
+                    for (int kk = 0; kk < KP / 4; ++kk) dmma884(p.x, p.y, fa[I][kk], fb[J][kk]);
+                    if (w) *pp = p;
+                } else {
+                    const bool w0 = i < N && j <= i, w1 = i < N && j + 1 <= i;
+                    double p0 = w0 ? Ps[prec(N, i, j)] : 0.0, p1 = w1 ? Ps[prec(N, i, j + 1)] : 0.0;
+#pragma unroll
+                    for (int kk = 0; kk < KP / 4; ++kk) dmma884(p0, p1, fa[I][kk], fb[J][kk]);
+                    if (w0) Ps[prec(N, i, j)] = p0;
+                    if (w1) Ps[prec(N, i, j + 1)] = p1;
+                }
             }
     }
     return __all_sync(FULL, finite) ? 0 : SLB_ST_NONFINITE;
@@ -555,10 +572,10 @@ SLB_DEV int usckf_predict_smem(double *Ps, double *mus, double *scr, const doubl
                                bool &dirty) {
     typedef LayState12 L;
     typedef CycCfg<12> C;
-    constexpr int ROW0 = 24, MU0 = 26;
+    constexpr int ROW0 = 24, MU0 = 26, N = 36 + NF;
     double *Ls = scr, *D = Ls + PRED_LS, *W = D + 28 * PRED_DS, *Fk = W + 144, *rsd = Fk + 12 * PRED_DS, *slots = rsd + 16;
-    auto PR = [&](int r, int c) -> double & { return Ps[tri(ROW0 + r, c)]; };        // row 24 + r, col c
-    auto PF = [&](int fr, int c) -> double & { return Ps[tri(36 + fr, 24 + c)]; };   // feature row fr, col 24 + c
+    auto PR = [&](int r, int c) -> double & { return Ps[prec(N, ROW0 + r, c)]; };        // row 24 + r, col c
+    auto PF = [&](int fr, int c) -> double & { return Ps[prec(N, 36 + fr, 24 + c)]; };   // feature row fr, col 24 + c
     const int a_ = lane & 3, b_ = lane >> 2;
     double mu[13];
 #pragma unroll
@@ -711,13 +728,13 @@ SLB_DEV int usckf_predict_smem(double *Ps, double *mus, double *scr, const doubl
         }
     }
     __syncwarp();
+    // rows 24..35 x cols 0..23 are off-diagonal tiles of tile rows 3 and 4: one 16-byte store per lane and tile
 #pragma unroll
     for (int I = 0; I < 2; ++I)
 #pragma unroll
-        for (int J = 0; J < 3; ++J) {
-            const int r = 8 * I + b_, c = 8 * J + 2 * a_;
-            if (r < 12) { PR(r, c) = oc[I][J][0]; PR(r, c + 1) = oc[I][J][1]; }
-        }
+        for (int J = 0; J < 3; ++J)
+            if (8 * I + b_ < 12)
+                *reinterpret_cast<double2 *>(Ps + prec(N, ROW0 + 8 * I, 8 * J) + 2 * lane) = make_double2(oc[I][J][0], oc[I][J][1]);
 #pragma unroll
     for (int I = 0; I < NFT; ++I) {
 #pragma unroll
