@@ -11,15 +11,16 @@
 //   (8I + b, 8J + 2a) and (8I + b, 8J + 2a + 1) of tile (I, J)), so one panel's rank-4 update is ONE DMMA per tile fed
 //   by one shared-memory word per lane and tile row -- the scalar version needed 4 x (rows + cols) words and 4 FMAs
 //   per entry.  Per panel: the 16 lanes holding its columns park them in shared memory, every lane redoes the 4 x 4
-//   diagonal block's elimination (4 reciprocals, ~20 FMAs -- the same issue slots as one lane doing it), lane i
-//   finishes row i of the panel (6 FMAs), and the finished rows are both the A and (scaled by -1/d_k) the B fragments.
+//   diagonal block's elimination (4 reciprocals, ~20 FMAs -- the same issue slots as one lane doing it), lane t
+//   finishes row 8 J0 + t of the panel (6 FMAs; rows above tile row J0 = K >> 3 are zero and are skipped), and the
+//   finished rows are both the A and (scaled by -1/d_k) the B fragments.
 //   Only the columns that can move h are factored (j < 36 + nk, rounded up to a panel): rows below come out of the same
 //   panels (the TRSM is implicit), the trailing block of featuresk_l is never touched.
 //   The factor is NOT kept: sigma point j = mu [+] +-L(:,j) needs column j only, so after every 4 panels the 32 sigma
 //   points of those 16 columns go through h (one per lane), their contribution to the mean / innovation covariance is
 //   accumulated as deviations from Z0 = h(mu) (columns that cannot move h contribute nothing), and
 //   covXZ += U(:, 16 cols) W'(16 cols, :) with W'_j = (Z+_j - Z-_j) / (2 sqrt d_j)  (:714-737 without the
-//   exp/log round trip, quirk Q10).
+//   exp/log round trip, quirk Q10), one DMMA per panel and tile row into covXZ accumulator tiles.
 //   K = covXZ S^-1 (:286-288), K S K^T = covXZ K^T; Pk -= covXZ K^T is again one DMMA per tile, on the record in
 //   shared memory.
 // predict: slb_predict12.cuh's scheme on rows 24..35 of the resident record.
@@ -62,11 +63,14 @@ struct StepCfg {
     static constexpr int PL = 2 * NPAD + 8;
     static constexpr int PS4 = 2 * PL + 2;             // stride between the 4 panels of a group
     static constexpr int KP = (NK_ + 3) / 4 * 4;       // padded row length of K / covXZ (DMMA k-dimension)
+    static constexpr int NTN = (NK_ + 7) / 8;          // 8-column accumulator tiles of covXZ
     static constexpr int LF = 4 * PS4;                 // finished panel rows U of the current group
     static constexpr int LRAW = 2 * PL;                // the current panel as extracted from the accumulators (same planes)
     static constexpr int KK = 2 * NPAD * KP + NPAD;    // K | covXZ rows | K nu, overlay LF | LRAW once the factorisation is over
     static constexpr int SCR0 = (LF + LRAW > KK ? LF + LRAW : KK);
-    static constexpr int WGS = 16 * NK_;               // W' of the current group, [c][16]: column pairs are one double2
+    // W' of the current group, [c][WS]: the DMMA B fragment W'(K + a, c = b) is then conflict-free (4 c + a covers 0..15)
+    static constexpr int WS = 20;
+    static constexpr int WGS = WS * NK_;
     static constexpr int UPD_SCR = SCR0 + WGS + NPAD;       // + d_k
     static constexpr int PRED_SCR = PRED_LS + 28 * PRED_DS + 144 + 12 * PRED_DS + 16 + 16;   // ... + rsd + reduction slots
     static constexpr int SCR = (UPD_SCR > PRED_SCR ? UPD_SCR : PRED_SCR);
@@ -195,7 +199,7 @@ SLB_DEV void warp_sum12(const double *v, double *out, double *slots, int lane) {
 template <class C>
 struct UpdState {
     double c0[C::NT][C::JLAST + 1], c1[C::NT][C::JLAST + 1];   // accumulator tiles (I >= J)
-    double px0[C::NK], px1[C::NK];                             // covXZ rows lane, lane + 32 (unscaled sum)
+    double x0[C::NT][C::NTN], x1[C::NT][C::NTN];               // covXZ accumulator tiles (unscaled sum)
     double esum[C::NK], eep[C::NK * (C::NK + 1) / 2];          // sum e, sum e e^T over this lane's sigma points, e = Z - Z0
     double z0[C::NK];
     bool ok;
@@ -222,9 +226,11 @@ SLB_DEV void sigma_group(UpdState<C> &s, const double *mus_, const double *Lf, d
     const int jl = act ? lane >> 1 : 0;                    // idle lanes (last group) shadow column 0 with a zero scale
     const double rs = rsqrt_fast(dv[col0 + jl]);           // L(:,j) = U(:,j) / sqrt(d_j): the scale rides on the sign
     const double sgn = act ? (neg ? -rs : rs) : 0.0;
-    // U(r, j) = col[2 r]; rows above the diagonal hold zeros
+    // U(r, j) = col[2 r] for r >= 8 (j >> 3); the rows of tile row j >> 3 above the diagonal hold zeros, the rows above
+    // it are not written (finish) and read as zero here.  Rows >= RW are written for every column of the group.
+    constexpr int RW = 8 * ((col0 + ncols - 1) >> 3);
     const double *col = Lf + (jl >> 2) * PS4 + ((jl & 3) >> 1) * C::PL + (jl & 1);
-    auto Lc = [&](int r) -> double { return sgn * col[2 * r]; };
+    auto Lc = [&](int r) -> double { return sgn * (r >= RW || r >= col0 + jl ? col[2 * r] : 0.0); };
     double xpk[3], xqk[4], xpi[3], xqi[4], xf[NK];
     if (col0 <= 5) {   // column j perturbs rows >= j only: statek is untouched from the second group on
 #pragma unroll
@@ -264,27 +270,28 @@ SLB_DEV void sigma_group(UpdState<C> &s, const double *mus_, const double *Lf, d
         e[c] = act ? z[c] - s.z0[c] : 0.0;
         s.esum[c] += e[c];
         const double zp = __shfl_xor_sync(FULL, z[c], 1);
-        if (act && !neg) Wg[c * 16 + jl] = (0.5 * rs) * (z[c] - zp);   // W'_j = (Z+ - Z-) / (2 sqrt d_j)
+        if (act && !neg) Wg[c * C::WS + jl] = (0.5 * rs) * (z[c] - zp);   // W'_j = (Z+ - Z-) / (2 sqrt d_j)
     }
 #pragma unroll
     for (int r = 0; r < NK; ++r)
 #pragma unroll
         for (int c = 0; c <= r; ++c) s.eep[tri(r, c)] = fma(e[r], e[c], s.eep[tri(r, c)]);
     __syncwarp();
-    // covXZ rows `lane` and `lane + 32` += U(row, 16 cols) W'(16 cols, :)
-    const bool has1 = lane + 32 < C::NPAD;
+    // covXZ += U(:, K..K+3) W'(K..K+3, :) for each panel of the group: one DMMA per tile row I >= K >> 3 (the rows above
+    // are zero) and covXZ column tile, A = U(8I + b, K + a) as in the rank-4 update, B = W'(K + a, 8T + b), zero beyond nk
+    const int a_ = lane & 3, b_ = lane >> 2;
 #pragma unroll
     for (int qq = 0; qq < ncols / 4; ++qq) {
-        const double *pa = Lf + qq * PS4 + 2 * lane, *pb = pa + C::PL;
-        const double2 x01 = *reinterpret_cast<const double2 *>(pa), x23 = *reinterpret_cast<const double2 *>(pb);
-        double2 y01 = make_double2(0.0, 0.0), y23 = y01;
-        if (has1) { y01 = *reinterpret_cast<const double2 *>(pa + 64); y23 = *reinterpret_cast<const double2 *>(pb + 64); }
+        const int J0 = (col0 + 4 * qq) >> 3;
+        const double *fp = Lf + qq * PS4 + (a_ >> 1) * C::PL + (a_ & 1) + 2 * b_;
+        double w[C::NTN];
 #pragma unroll
-        for (int c = 0; c < NK; ++c) {
-            const double2 w01 = *reinterpret_cast<const double2 *>(Wg + c * 16 + 4 * qq);
-            const double2 w23 = *reinterpret_cast<const double2 *>(Wg + c * 16 + 4 * qq + 2);
-            s.px0[c] = fma(x23.y, w23.y, fma(x23.x, w23.x, fma(x01.y, w01.y, fma(x01.x, w01.x, s.px0[c]))));
-            s.px1[c] = fma(y23.y, w23.y, fma(y23.x, w23.x, fma(y01.y, w01.y, fma(y01.x, w01.x, s.px1[c]))));
+        for (int T = 0; T < C::NTN; ++T) w[T] = 8 * T + b_ < NK ? Wg[(8 * T + b_) * C::WS + 4 * qq + a_] : 0.0;
+#pragma unroll
+        for (int I = J0; I < C::NT; ++I) {
+            const double f = fp[16 * I];
+#pragma unroll
+            for (int T = 0; T < C::NTN; ++T) dmma884(s.x0[I][T], s.x1[I][T], f, w[T]);
         }
     }
 }
@@ -334,9 +341,11 @@ struct PanelStep {
             *reinterpret_cast<double2 *>(dv + K) = make_double2(d0, d1);
             *reinterpret_cast<double2 *>(dv + K + 2) = make_double2(d2, d3);
         }
-        // (3) lane i finishes rows i and i + 32 of the panel: U(i, K + c); zeros above the diagonal / above the panel.
-        //     Branch-free: rows above the panel read whatever the planes hold and select zeros.
-        auto finish = [&](int i, bool have) {
+        // (3) lane t finishes rows 8 J0 + t and 8 J0 + 32 + t of the panel: U(i, K + c), zeros above the diagonal.  The
+        //     rows above tile row J0 are zero and are neither written nor read: the fragments below start at I1 >= J0, the
+        //     covXZ DMMAs at J0, and the sigma points select zeros there.
+        constexpr int R0 = 8 * J0, NLIVE = C::NPAD - R0;
+        auto finish = [&](int i) {
             const double2 x01 = *reinterpret_cast<const double2 *>(Lraw + 2 * i);
             const double2 x23 = *reinterpret_cast<const double2 *>(Lraw + PL + 2 * i);
             const double u0 = x01.x;
@@ -348,18 +357,11 @@ struct PanelStep {
             u01.y = i >= K + 1 ? u1 : 0.0;
             u23.x = i >= K + 2 ? u2 : 0.0;
             u23.y = i >= K + 3 ? u3 : 0.0;
-            if (have) {
-                *reinterpret_cast<double2 *>(Lq + 2 * i) = u01;
-                *reinterpret_cast<double2 *>(Lq + PL + 2 * i) = u23;
-            }
+            *reinterpret_cast<double2 *>(Lq + 2 * i) = u01;
+            *reinterpret_cast<double2 *>(Lq + PL + 2 * i) = u23;
         };
-        if (K < 32) {
-            finish(lane, true);
-        } else {   // rows 0..31 lie above the panel
-            *reinterpret_cast<double2 *>(Lq + 2 * lane) = make_double2(0.0, 0.0);
-            *reinterpret_cast<double2 *>(Lq + PL + 2 * lane) = make_double2(0.0, 0.0);
-        }
-        if (C::NPAD > 32) finish(lane + 32 < C::NPAD ? lane + 32 : lane, lane + 32 < C::NPAD);
+        if (NLIVE >= 32 || lane < NLIVE) finish(R0 + lane);
+        if (NLIVE > 32 && lane < NLIVE - 32) finish(R0 + 32 + lane);
         __syncwarp();
         // (4) rank-4 update of the live tiles: A fragment = U(8I + b, K + a), B fragment = -U(8J + b, K + a) / d_{K+a}
         if (I1 <= JLAST) {
@@ -421,7 +423,11 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
                 s.c1[I][J] = elem(i, j + 1);
             }
 #pragma unroll
-    for (int c = 0; c < NK; ++c) s.px0[c] = s.px1[c] = s.esum[c] = 0.0;
+    for (int I = 0; I < NT; ++I)
+#pragma unroll
+        for (int T = 0; T < C::NTN; ++T) s.x0[I][T] = s.x1[I][T] = 0.0;
+#pragma unroll
+    for (int c = 0; c < NK; ++c) s.esum[c] = 0.0;
 #pragma unroll
     for (int e = 0; e < NK * (NK + 1) / 2; ++e) s.eep[e] = 0.0;
     {   // Z0 = h(mu)
@@ -484,7 +490,18 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
     }
     if (!sok) return SLB_ST_CHOL_FAIL;
     if (!chi2_accept(m2, a.gate)) return SLB_ST_GATE_REJECT;
-    auto finish_row = [&](const double *px, int i) {
+    // covXZ from the accumulator tiles into the rows of Cs, then lane i turns row i into K, -covXZ and K nu
+#pragma unroll
+    for (int I = 0; I < NT; ++I)
+#pragma unroll
+        for (int T = 0; T < C::NTN; ++T)
+            if (8 * T + 2 * a_ < KP)
+                *reinterpret_cast<double2 *>(Cs + (8 * I + b_) * KP + 8 * T + 2 * a_) = make_double2(s.x0[I][T], s.x1[I][T]);
+    __syncwarp();
+    auto finish_row = [&](int i) {
+        double px[NK];
+#pragma unroll
+        for (int c = 0; c < NK; ++c) px[c] = Cs[i * KP + c];
         double dsum = 0.0;
 #pragma unroll
         for (int c = 0; c < KP; ++c) {
@@ -499,8 +516,8 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
         }
         dl[i] = dsum;   // (K nu)_i
     };
-    finish_row(s.px0, lane);
-    if (lane + 32 < NPAD) finish_row(s.px1, lane + 32);
+    finish_row(lane);
+    if (lane + 32 < NPAD) finish_row(lane + 32);
     __syncwarp();
     dirty = true;
     // ---- mu = mu [+] K nu (:299-301): lane b < 12 owns block b of the three States, then the feature scalars ------
