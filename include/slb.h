@@ -137,11 +137,13 @@ int slb_device_ptr(slb_handle h, int field, void **dev);
 
 /* ---- ukfom::ukf<state> ----------------------------------------------------------------- */
 /* predict(g, R): sigma points -> g -> manifold mean -> cov + Q. u_dev: batch x nu (instance-
- * major), Q_dev: n x n row-major shared by the batch. */
+ * major), Q_dev: n x n row-major shared by the batch (batch x n x n with SLB_NOISE_Q_PER_INSTANCE, see
+ * slb_set_noise_layout). */
 int slb_ukf_predict(slb_handle h, int pm, const double *u_dev, double dt, const double *Q_dev,
                     void *stream);
 /* update(z, h, R[, mt]): gate_dof = 0 accepts any Mahalanobis distance, 1..9 applies the 5%
- * chi-square table (Usckf.hpp:794-855). z_dev: batch x m, R_dev: m x m shared. */
+ * chi-square table (Usckf.hpp:794-855). z_dev: batch x m, R_dev: m x m shared (batch x m x m
+ * with SLB_NOISE_R_PER_INSTANCE, see slb_set_noise_layout). */
 int slb_ukf_update(slb_handle h, int mm, const double *z_dev, const double *R_dev, int gate_dof,
                    void *stream);
 /* predict immediately followed by update in one launch (one HBM round trip). */
@@ -159,6 +161,17 @@ int slb_ukf_step_host(slb_handle h, int pm, int mm, const double *u_host, double
  * Usckf.hpp:518).  (26, 13) on a USCKF batch is statek_i, what Usckf::muSingleState() returns by default
  * (Usckf.hpp:457-478); (0, 13) on an MSCKF batch is Msckf::muSingleState() (Msckf.hpp:356). */
 int slb_set_output_slice(slb_handle h, int offset, int count);
+/* Layout of the noise covariances that later device entry points receive on this handle.  0 (the default) = one
+ * matrix shared by the batch, as before.  Q_PER_INSTANCE: Q_dev is batch x n x n row-major (instance i's matrix at
+ * Q_dev + i*n*n; lower triangle read, like the shared Q).  R_PER_INSTANCE: R_dev is batch x m x m row-major.
+ * Honoured by slb_ukf_predict/update/step (n = 6 or 9, m = 3), slb_usckf_predict/update/step (n = 12, m = nk),
+ * slb_usckf_set_measurement (R: len x len per instance) and slb_msckf_predict (n = 12).  Like the reference, which
+ * takes its noise per call and per object (Usckf::predict(f, Q), update(z, h, R), setMeasurement(mode, z, R)), a batch
+ * of B then stands for B objects handed different covariances.  SLB_ERR_INVALID for flags outside 0..3 and for
+ * R_PER_INSTANCE on an MSCKF handle (its update noise is shared).  While the flags are non-zero the *_step_host and
+ * *_step_host_async entry points refuse to run: per-instance noise is device-resident only. */
+enum { SLB_NOISE_Q_PER_INSTANCE = 1, SLB_NOISE_R_PER_INSTANCE = 2 };
+int slb_set_noise_layout(slb_handle h, int flags);
 /* Pipelined flavour: identical, but returns as soon as the step is enqueued on `stream` (no
  * synchronisation), so consecutive steps overlap their host<->device traffic with each other's
  * kernels.  The host buffers must stay valid (and mu_out_host unread) until slb_wait(h, stream);
@@ -174,7 +187,8 @@ int slb_wait(slb_handle h, void *stream);
 /* predict(f, Q) Usckf.hpp:107-244 */
 int slb_usckf_predict(slb_handle h, int pm, const double *u_dev, double dt, const double *Q_dev,
                       void *stream);
-/* update(z, h, R[, mt]) Usckf.hpp:246-308; z_dev: batch x m, R_dev: m x m shared */
+/* update(z, h, R[, mt]) Usckf.hpp:246-308; z_dev: batch x m, R_dev: m x m shared (batch x m x m with
+ * SLB_NOISE_R_PER_INSTANCE); predict's Q_dev: 12 x 12 (batch x 12 x 12 with SLB_NOISE_Q_PER_INSTANCE) */
 int slb_usckf_update(slb_handle h, int mm, const double *z_dev, const double *R_dev,
                      int gate_dof, void *stream);
 int slb_usckf_step(slb_handle h, int pm, int mm, const double *u_dev, double dt,
@@ -188,13 +202,14 @@ int slb_usckf_step_host_async(slb_handle h, int pm, int mm, const double *u_host
                               int gate_dof, double *mu_out_host, void *stream);
 /* cloning(mode) Usckf.hpp:391-433 */
 int slb_usckf_clone(slb_handle h, int mode, void *stream);
-/* setMeasurement(mode, z, R) Usckf.hpp:322-389; z_dev: batch x len, R_dev: len x len shared.
+/* setMeasurement(mode, z, R) Usckf.hpp:322-389; z_dev: batch x len, R_dev: len x len shared
+ * (batch x len x len with SLB_NOISE_R_PER_INSTANCE).
  * len must equal the configured nk (mode STATEK) or nl (STATEK_L). */
 int slb_usckf_set_measurement(slb_handle h, int mode, const double *z_dev, const double *R_dev,
                               void *stream);
 
 /* ---- localization::Msckf --------------------------------------------------------------- */
-/* predict(f, Q) Msckf.hpp:89-189 */
+/* predict(f, Q) Msckf.hpp:89-189; Q_dev: 12 x 12 shared (batch x 12 x 12 with SLB_NOISE_Q_PER_INSTANCE) */
 int slb_msckf_predict(slb_handle h, int pm, const double *u_dev, double dt, const double *Q_dev,
                       void *stream);
 /* update(z, h, R[, mt]) Msckf.hpp:196-277 (UKF flavour, per-feature 2-dof gate when gate != 0).

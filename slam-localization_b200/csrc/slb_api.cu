@@ -339,6 +339,19 @@ int slb_set_output_slice(slb_handle h, int offset, int count) {
     h->out_len = count;
     return SLB_OK;
 }
+int slb_set_noise_layout(slb_handle h, int flags) {
+    if (!h) return set_error(SLB_ERR_INVALID, "slb_set_noise_layout: null handle");
+    if (flags < 0 || flags > (SLB_NOISE_Q_PER_INSTANCE | SLB_NOISE_R_PER_INSTANCE))
+        return set_error(SLB_ERR_INVALID, "slb_set_noise_layout: flags must be a combination of SLB_NOISE_Q_PER_INSTANCE and "
+                                          "SLB_NOISE_R_PER_INSTANCE");
+    if (h->cfg.kind == SLB_KIND_MSCKF && (flags & SLB_NOISE_R_PER_INSTANCE))
+        return set_error(SLB_ERR_INVALID, "slb_set_noise_layout: MSCKF update noise is shared by the batch (only Q may be per instance)");
+    h->noise = flags;
+    return SLB_OK;
+}
+// doubles between consecutive instances' Q / R for a handle's noise layout (0 = shared)
+static int q_stride(slb_handle h, int n) { return (h->noise & SLB_NOISE_Q_PER_INSTANCE) ? n * n : 0; }
+static int r_stride(slb_handle h, int m) { return (h->noise & SLB_NOISE_R_PER_INSTANCE) ? m * m : 0; }
 int slb_dof(slb_handle h) { return h ? h->N : SLB_ERR_INVALID; }
 int slb_qdim(slb_handle h) { return h ? h->QD : SLB_ERR_INVALID; }
 
@@ -447,6 +460,7 @@ static int ukf_call(slb_handle h, int pm, int mm, bool pred, bool upd, const dou
     DeviceGuard guard(h->cfg.device);
     FilterArgs a = make_args(h);
     a.u = u; a.dt = dt; a.Q = Q; a.z = z; a.R = R; a.gate = gate; a.m = 3;
+    a.qs = q_stride(h, h->N); a.rs = r_stride(h, 3);
     return launch_ukf(h->cfg.layout, pm, mm, pred, upd, a, S(stream));
 }
 int slb_ukf_predict(slb_handle h, int pm, const double *u, double dt, const double *Q, void *stream) {
@@ -652,6 +666,7 @@ static int step_host(slb_handle h, const HostStep &hs, void *stream, bool wait =
 static int ukf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
                          const double *z_host, const double *R_host, int gate_dof, double *mu_out_host, void *stream, bool wait) {
     if (!h || h->cfg.kind != SLB_KIND_UKF) return set_error(SLB_ERR_INVALID, "slb_ukf_step_host: handle is not a UKF batch");
+    if (h->noise) return set_error(SLB_ERR_INVALID, "slb_ukf_step_host: per-instance noise (slb_set_noise_layout) is device-resident only");
     if (mm != SLB_MM_GPS_POS) return set_error(SLB_ERR_INVALID, "ukf: unsupported measurement model");
     const HostStep hs = {pm, mm, pm_nu(pm), 3, h->N, 0, gate_dof, dt, u_host, Q_host, nullptr, z_host, R_host, mu_out_host};
     return step_host(h, hs, stream, wait);
@@ -682,6 +697,7 @@ static int usckf_call(slb_handle h, int pm, int mm, bool pred, bool upd, const d
     DeviceGuard guard(h->cfg.device);
     FilterArgs a = make_args(h);
     a.u = u; a.dt = dt; a.Q = Q; a.z = z; a.R = R; a.gate = gate; a.m = h->cfg.nk;
+    a.qs = q_stride(h, 12); a.rs = r_stride(h, h->cfg.nk);
     return launch_usckf(pm, mm, pred, upd, a, S(stream));
 }
 int slb_usckf_predict(slb_handle h, int pm, const double *u, double dt, const double *Q, void *stream) {
@@ -697,6 +713,7 @@ int slb_usckf_step(slb_handle h, int pm, int mm, const double *u, double dt, con
 static int usckf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
                            const double *z_host, const double *R_host, int gate_dof, double *mu_out_host, void *stream, bool wait) {
     if (!h || h->cfg.kind != SLB_KIND_USCKF) return set_error(SLB_ERR_INVALID, "slb_usckf_step_host: handle is not a USCKF batch");
+    if (h->noise) return set_error(SLB_ERR_INVALID, "slb_usckf_step_host: per-instance noise (slb_set_noise_layout) is device-resident only");
     const HostStep hs = {pm, mm, pm_nu(pm), h->cfg.nk, 12, 0, gate_dof, dt, u_host, Q_host, nullptr, z_host, R_host, mu_out_host};
     return step_host(h, hs, stream, wait);
 }
@@ -720,6 +737,7 @@ int slb_usckf_set_measurement(slb_handle h, int mode, const double *z, const dou
     DeviceGuard guard(h->cfg.device);
     FilterArgs a = make_args(h);
     a.z = z; a.R = R;
+    a.rs = r_stride(h, mode == SLB_STATEK ? h->cfg.nk : h->cfg.nl);
     return launch_usckf_set_measurement(mode, a, S(stream));
 }
 
@@ -730,6 +748,7 @@ int slb_msckf_predict(slb_handle h, int pm, const double *u, double dt, const do
     DeviceGuard guard(h->cfg.device);
     FilterArgs a = make_args(h);
     a.u = u; a.dt = dt; a.Q = Q;
+    a.qs = q_stride(h, 12);
     return launch_msckf_predict(pm, a, S(stream));
 }
 int slb_msckf_update(slb_handle h, int mm, const double *params, int m, const double *z, const double *R, int gate,
@@ -771,6 +790,7 @@ static int msckf_step_host(slb_handle h, int pm, int mm, const double *u_host, d
                            const double *params_host, int nparams, int m, const double *z_host, const double *R_host,
                            int gate, double *mu_out_host, void *stream, bool wait) {
     if (!h || h->cfg.kind != SLB_KIND_MSCKF) return set_error(SLB_ERR_INVALID, "slb_msckf_step_host: handle is not an MSCKF batch");
+    if (h->noise) return set_error(SLB_ERR_INVALID, "slb_msckf_step_host: per-instance noise (slb_set_noise_layout) is device-resident only");
     if (!u_host || !Q_host || !params_host || !z_host || !R_host || m <= 0 || nparams <= 0)
         return set_error(SLB_ERR_INVALID, "slb_msckf_step_host: null argument");
     const HostStep hs = {pm, mm, pm_nu(pm), m, 12, nparams, gate, dt, u_host, Q_host, params_host, z_host, R_host, mu_out_host};

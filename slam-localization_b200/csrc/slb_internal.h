@@ -38,6 +38,7 @@ struct slb_batch_s {
     const void *step_key_p[6];
     cudaEvent_t ev_start, ev_done[SLB_NXS];
     int out_off, out_len;      // slb_set_output_slice: part of the q-vector the *_step_host entry points copy back
+    int noise;                 // slb_set_noise_layout: SLB_NOISE_* flags (0 = Q and R shared by the batch)
     // zero-copy *_step_host: host copy of the Q | R last uploaded to shared_small (the upload is skipped while the caller
     // keeps passing the same values: two tiny DMA operations per step are 10 % of a UKFoM step)
     double qr_cache[144 + 81];
@@ -86,11 +87,17 @@ struct FilterArgs {
     int m;
     int gate;
     int nk, nl, k;
+    // per-instance noise (slb_set_noise_layout): qs / rs = doubles between consecutive instances' Q / R, 0 = one matrix
+    // shared by the batch; the launchers select the kernels' per-instance instantiations when one of them is set.  The
+    // two fill alignment holes: the kernels' parameter layout (size, every other member's offset) is as without them.
+    int qs;
     int32_t *misc;
     int prefetch;     // USCKF step: L2-prefetch the record of instance (i + prefetch); 0 = off
+    int rs;
     double *mu_out;   // optional instance-major copy of the posterior means (may be mapped host memory), B x out_len
     int out_off, out_len;  // the slice [out_off, out_off + out_len) of the q-vector that goes to mu_out
 };
+static_assert(sizeof(FilterArgs) == 152, "FilterArgs layout");
 
 // slb_ukf.cu
 int launch_ukf(int layout, int pm, int mm, bool predict, bool update, const FilterArgs &a, cudaStream_t s);

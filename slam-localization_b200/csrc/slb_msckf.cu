@@ -1523,11 +1523,11 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_ekf_update_kernel(slb::FilterAr
 
 namespace slb {
 
-template <int PM>
+template <int PM, bool PIN>
 static int launch_ms_predict_t(const FilterArgs &a, cudaStream_t s) {
     constexpr int WPB = 8;
     constexpr size_t smem = (size_t)WPB * slbd::PRED_SM * sizeof(double);
-    auto kern = slbd::predict12_kernel<PM, WPB, 0, 0, false>;
+    auto kern = slbd::predict12_kernel<PM, WPB, 0, 0, false, PIN>;
     SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<(a.B + WPB - 1) / WPB, WPB * 32, smem, s>>>(a);
     count_launch();
@@ -1536,8 +1536,11 @@ static int launch_ms_predict_t(const FilterArgs &a, cudaStream_t s) {
 }
 
 int launch_msckf_predict(int pm, const FilterArgs &a, cudaStream_t s) {
-    if (pm == SLB_PM_MSCKF_DELTAPOSE) return launch_ms_predict_t<SLB_PM_MSCKF_DELTAPOSE>(a, s);
-    if (pm == SLB_PM_USCKF_TEST) return launch_ms_predict_t<SLB_PM_USCKF_TEST>(a, s);
+    // a.qs != 0: per-instance Q (slb_set_noise_layout)
+    if (pm == SLB_PM_MSCKF_DELTAPOSE)
+        return a.qs ? launch_ms_predict_t<SLB_PM_MSCKF_DELTAPOSE, true>(a, s) : launch_ms_predict_t<SLB_PM_MSCKF_DELTAPOSE, false>(a, s);
+    if (pm == SLB_PM_USCKF_TEST)
+        return a.qs ? launch_ms_predict_t<SLB_PM_USCKF_TEST, true>(a, s) : launch_ms_predict_t<SLB_PM_USCKF_TEST, false>(a, s);
     return set_error(SLB_ERR_INVALID, "msckf: unsupported process model");
 }
 

@@ -149,6 +149,15 @@ SLB_DEV void pred_cp_async8(double *smem_dst, const double *gsrc) {
 }
 SLB_DEV void pred_cp_async_wait_all() { asm volatile("cp.async.commit_group;\n cp.async.wait_group 0;\n" ::: "memory"); }
 
+// The 6 entries of a 12 x 12 process noise Q (row-major, lower triangle read) that lane (a_, b_) adds to the predicted
+// covariance's DMMA accumulator pairs: rows b_ / 8 + b_, columns 2 a_ (+1) / 8 + 2 a_ (+1); upper-triangle slots are 0.
+SLB_DEV void load_q_entries(const double *Qi, int a_, int b_, double *qv) {
+    const int rr[6] = {b_, b_, 8 + b_, 8 + b_, 8 + b_, 8 + b_};
+    const int cc[6] = {2 * a_, 2 * a_ + 1, 2 * a_, 2 * a_ + 1, 8 + 2 * a_, 9 + 2 * a_};
+#pragma unroll
+    for (int k = 0; k < 6; ++k) qv[k] = (rr[k] < 12 && cc[k] <= rr[k]) ? __ldg(Qi + rr[k] * 12 + cc[k]) : 0.0;
+}
+
 // ROW0: first row of the 12x12 block; MU0: q-vector offset of the block's mean; CROSS: propagate the
 // cross-covariances of the block's rows/columns with the rest of the state (USCKF) or not (MSCKF).
 //
@@ -157,7 +166,11 @@ SLB_DEV void pred_cp_async_wait_all() { asm volatile("cp.async.commit_group;\n c
 // rank-k contraction -- the propagated covariance 0.5 D^T D, Fk * P_i,(k|l), P_feat,i * Fk^T -- is 8x8x4 DMMA tiles
 // fed straight from shared memory (51 DMMAs replace ~1 100 LDS + DFMA issue slots; rows / columns beyond the block
 // only feed accumulator entries that are never stored).
-template <int PM, int WPB, int ROW0, int MU0, bool CROSS>
+//
+// PIN: per-instance Q (slb_set_noise_layout), instance i's 12 x 12 matrix at a.Q + i * a.qs.  Each lane adds at most 6
+// entries of Q (put below); it loads exactly those into registers together with the record, so the HBM latency of a
+// matrix that no longer sits in L1 overlaps the record's instead of the end of the step.
+template <int PM, int WPB, int ROW0, int MU0, bool CROSS, bool PIN = false>
 __global__ void __launch_bounds__(WPB * 32, 2) predict12_kernel(slb::FilterArgs a) {
     typedef LayState12 L;
     typedef CycCfg<12> C;
@@ -203,6 +216,8 @@ __global__ void __launch_bounds__(WPB * 32, 2) predict12_kernel(slb::FilterArgs 
         const int r = e / 12, c = e - r * 12;
         pred_cp_async8(Pf + e, Pg + prec(N, RS + r, 24 + c));
     }
+    double qv[PIN ? 6 : 1];
+    if (PIN) load_q_entries(a.Q + (size_t)inst * a.qs, a_, b_, qv);
     double mu[13];
 #pragma unroll
     for (int c = 0; c < 13; ++c) mu[c] = mug[MU0 + c];
@@ -305,13 +320,13 @@ __global__ void __launch_bounds__(WPB * 32, 2) predict12_kernel(slb::FilterArgs 
                 W[e] = 0.5 * (D[(1 + 2 * jj) * PRED_DS + c] - D[(2 + 2 * jj) * PRED_DS + c]);
             }
         }
-        auto put = [&](int r, int c, double v) {
-            if (r < 12 && c <= r) PR(r, ROW0 + c) = 0.5 * v + __ldg(a.Q + r * 12 + c);
+        auto put = [&](int r, int c, double v, int k) {
+            if (r < 12 && c <= r) PR(r, ROW0 + c) = 0.5 * v + (PIN ? qv[k] : __ldg(a.Q + r * 12 + c));
         };
         const int r = b_, c = 2 * a_;
-        put(r, c, c00[0]); put(r, c + 1, c00[1]);
-        put(8 + r, c, c10[0]); put(8 + r, c + 1, c10[1]);
-        put(8 + r, 8 + c, c11[0]); put(8 + r, 8 + c + 1, c11[1]);
+        put(r, c, c00[0], 0); put(r, c + 1, c00[1], 1);
+        put(8 + r, c, c10[0], 2); put(8 + r, c + 1, c10[1], 3);
+        put(8 + r, 8 + c, c11[0], 4); put(8 + r, 8 + c + 1, c11[1], 5);
     }
     if (CROSS) {
         __syncwarp();

@@ -163,9 +163,10 @@ SLB_DEV bool group_mean(const double *sig, int sub, bool go, double *ref) {
     return it < 10000;
 }
 
-// Msckf.hpp:554-570: P = 0.5 * sum (Yi [-] mean)(Yi [-] mean)^T (+ Qp), packed lower, written to `ps`.
-// `sig` is consumed: it becomes the reduction scratch.
-template <class L, int G, bool ADDQ>
+// Msckf.hpp:554-570: P = 0.5 * sum (Yi [-] mean)(Yi [-] mean)^T (+ Q), packed lower, written to `ps`.
+// `sig` is consumed: it becomes the reduction scratch.  Q is the warp's packed shared Qp, or (QREG, per-instance noise)
+// the entries e = sub + G k of this instance's packed Q, held in registers as Qp[k].
+template <class L, int G, bool ADDQ, bool QREG = false>
 SLB_DEV void group_cov(double *sig, double *ps, const double *Qp, int sub, const double *mean) {
     constexpr int N = L::N, QD = L::QD, NP = L::NP, NS = 2 * N + 1, ROUNDS = (NS + G - 1) / G;
     double acc[NP];
@@ -189,18 +190,39 @@ SLB_DEV void group_cov(double *sig, double *ps, const double *Qp, int sub, const
 #pragma unroll
     for (int e = 0; e < NP; ++e) sig[sub * NP + e] = acc[e];
     __syncwarp();
-    for (int e = sub; e < NP; e += G) {
-        double v = sig[e];
+    if constexpr (QREG) {
 #pragma unroll
-        for (int l = 1; l < G; ++l) v += sig[l * NP + e];
-        v *= 0.5;
-        if (ADDQ) v += Qp[e];
-        ps[e] = v;
+        for (int k = 0; k < (NP + G - 1) / G; ++k) {
+            const int e = sub + G * k;
+            if (e < NP) {
+                double v = sig[e];
+#pragma unroll
+                for (int l = 1; l < G; ++l) v += sig[l * NP + e];
+                v *= 0.5;
+                if (ADDQ) v += Qp[k];
+                ps[e] = v;
+            }
+        }
+    } else {
+        for (int e = sub; e < NP; e += G) {
+            double v = sig[e];
+#pragma unroll
+            for (int l = 1; l < G; ++l) v += sig[l * NP + e];
+            v *= 0.5;
+            if (ADDQ) v += Qp[e];
+            ps[e] = v;
+        }
     }
     __syncwarp();
 }
 
-template <class L, int PM, class MM, int G, int TPB, int MINB, bool PRED, bool UPD>
+// PIN: per-instance noise (slb_set_noise_layout).  Q and R are read at a.Q + inst * a.qs and a.R + inst * a.rs (a stride
+// of 0 = shared).  Each 4-lane group fetches the entries of its own instance that it adds into registers -- lane sub the
+// packed Q entries sub + 4k once the sigma points are drawn (the manifold-mean iterations cover their latency), every
+// lane the 6 lower entries of R as the update starts; the warp's shared Qp is not used (8 per-instance copies per warp
+// would cost a CTA).  Issued together with the record's copies they kept 18 more registers live through the predict and
+// the fused MTK9 step spilled 264 / 308 B instead of 216 / 260 B.
+template <class L, int PM, class MM, int G, int TPB, int MINB, bool PRED, bool UPD, bool PIN = false>
 __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
     typedef Rec<L, MM::M, G> R;
     constexpr int N = L::N, QD = L::QD, NP = L::NP, NS = 2 * N + 1, M = MM::M, MP = M * (M + 1) / 2;
@@ -218,6 +240,9 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
     if (wbase >= a.B) return;
     const int inst = wbase + grp;
     const bool valid = inst < a.B;
+    constexpr int QK = (NP + G - 1) / G;
+    double qreg[PIN ? QK : 1], rreg[PIN ? MP : 1];   // PIN: this instance's noise (see above)
+    const size_t ni = valid ? (size_t)inst : (size_t)(a.B - 1);   // idle tail groups borrow a real instance's noise
 
     // ---- stage the 8 records of this warp: lane -> (instance lane % IPW, fields lane / IPW + G k) ----
     // 8-byte LDGSTS: all ~14 loads of a lane are in flight before the first one lands (the staging loop used to
@@ -266,7 +291,7 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
                 }
             }
         }
-        if (PRED) {
+        if (PRED && !PIN) {
             for (int e = lane; e < NP; e += 32) {
                 int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);  // packed index -> (r, c), exact for e < 2^20
                 r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
@@ -320,9 +345,20 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
                 for (int c = 0; c < QD; ++c) sig[c * NS + s] = y[c];
             }
         }
+        if (PIN) {
+            const double *Qi = a.Q + ni * a.qs;
+#pragma unroll
+            for (int k = 0; k < QK; ++k) {
+                const int e = sub + G * k;
+                int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
+                r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
+                qreg[k] = e < NP ? __ldg(Qi + r * N + (e - tri(r, 0))) : 0.0;
+            }
+        }
         __syncwarp();
         if (!group_mean<L, G>(sig, sub, alive, mu) && alive) st |= SLB_ST_MEAN_NOCONV;
-        group_cov<L, G, true>(sig, ps, Qp, sub, mu);
+        if constexpr (PIN) group_cov<L, G, true, true>(sig, ps, qreg, sub, mu);
+        else group_cov<L, G, true>(sig, ps, Qp, sub, mu);
     }
 
     if (UPD) {
@@ -330,6 +366,13 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
         // `alive` = the record holds something to publish (in the fused step: the predicted state); a failing update
         // leaves that state as it is, exactly like calling predict and update separately
         bool upd = alive;
+        if (PIN) {
+            const double *Ri = a.R + ni * a.rs;
+#pragma unroll
+            for (int r = 0; r < M; ++r)
+#pragma unroll
+                for (int c = 0; c <= r; ++c) rreg[tri(r, c)] = __ldg(Ri + r * M + c);
+        }
         if (!group_chol<N>(ps, lf, sub) && alive) { st |= SLB_ST_CHOL_FAIL; upd = false; }
         double *Z = sig + R::ZO, *DZ = sig + R::DZO, *Ks = sig + R::KO, *KSs = sig + R::KSO, *DL = sig + R::DLO;
         double zsum[M];
@@ -371,7 +414,7 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
 #pragma unroll
         for (int r = 0; r < M; ++r)
 #pragma unroll
-            for (int c = 0; c <= r; ++c) S[tri(r, c)] = 0.5 * gsum<G>(S[tri(r, c)]) + __ldg(a.R + r * M + c);
+            for (int c = 0; c <= r; ++c) S[tri(r, c)] = 0.5 * gsum<G>(S[tri(r, c)]) + (PIN ? rreg[tri(r, c)] : __ldg(a.R + r * M + c));
         // Pxz = 0.5 sum (Xi [-] mu)(Zi - zbar)^T.  Xi [-] mu is +-L e_j by construction (the reference
         // recovers it through log(exp(.)), identical below |.| < pi), and the zbar terms of a +- pair
         // cancel: Pxz = 0.5 L DZ with DZ_j = Z+_j - Z-_j.
@@ -533,6 +576,8 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
 
 namespace slb {
 
+// Per-instance noise (a.qs / a.rs set by slb_set_noise_layout) selects the PIN instantiations; the shared-noise
+// kernels are unchanged.
 template <class L, int PM, class MM>
 static int launch_ukf_t(bool predict, bool update, const FilterArgs &a, cudaStream_t s) {
     constexpr int G = 4, TPB = 128, MINB = 3;
@@ -548,6 +593,12 @@ static int launch_ukf_t(bool predict, bool update, const FilterArgs &a, cudaStre
         SLB_CUDA(cudaGetLastError());
         return SLB_OK;
     };
+    const bool pin = (predict && a.qs) || (update && a.rs);
+    if (pin) {
+        if (predict && update) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true, true>);
+        if (predict) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, false, true>);
+        if (update) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true, true>);
+    }
     if (predict && update) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true>);
     if (predict) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, false>);
     if (update) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true>);

@@ -80,7 +80,7 @@ __global__ void usckf_set_measurement_kernel(slb::FilterArgs a, int mode) {
     double v = 0.0;  // Pk.setZero() (:348,:376): every state<->feature and k<->k+l cross term
     if (c >= 36) {
         const bool rin = fr >= f0 && fr < f0 + len, cin = fc >= f0 && fc < f0 + len;
-        if (rin && cin) v = a.R[(fr - f0) * len + (fc - f0)];      // new block = R (:353,:381)
+        if (rin && cin) v = a.R[(size_t)inst * a.rs + (fr - f0) * len + (fc - f0)];   // new block = R (:353,:381)
         else if (!rin && !cin) v = P[prec(N, r, c)];                // the block that stays (:355,:383)
     }
     P[prec(N, r, c)] = v;
@@ -90,11 +90,11 @@ __global__ void usckf_set_measurement_kernel(slb::FilterArgs a, int mode) {
 
 namespace slb {
 
-template <int PM>
+template <int PM, bool PIN>
 static int launch_predict_t(const FilterArgs &a, cudaStream_t s) {
     constexpr int WPB = 8;
     constexpr size_t smem = (size_t)WPB * slbd::PRED_SM * sizeof(double);
-    auto kern = slbd::predict12_kernel<PM, WPB, 24, 26, true>;
+    auto kern = slbd::predict12_kernel<PM, WPB, 24, 26, true, PIN>;
     SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     kern<<<(a.B + WPB - 1) / WPB, WPB * 32, smem, s>>>(a);
     count_launch();
@@ -131,8 +131,8 @@ bool usckf_shape_supported(int nk, int nl) {
     return false;
 }
 
-// record-resident kernel (slb_usckf_step.cuh): PRED && UPD = the fused step, UPD alone = update
-template <int NK, int NL, bool PRED, bool UPD>
+// record-resident kernel (slb_usckf_step.cuh): PRED && UPD = the fused step, UPD alone = update; PIN = per-instance noise
+template <int NK, int NL, bool PRED, bool UPD, bool PIN>
 static int launch_step_t(const FilterArgs &a, cudaStream_t s) {
     typedef slbd::StepCfg<NK, NL> C;
     // CTA shape: the register file (168 registers) holds 12 warps per SM.  Measured on the (3,9) fleet, 524 288 instances
@@ -140,7 +140,9 @@ static int launch_step_t(const FilterArgs &a, cudaStream_t s) {
     // step.  Two CTAs of six warps win: warps that start together walk the 104 KB unrolled instruction stream together
     // (the L1.5 instruction cache is 32 KB), while a single 12-warp CTA leaves the SM idle between its tail and the next
     // CTA's record loads.  Explicit CTA barriers to keep the warps aligned did not help (6.21 ms).
-    constexpr size_t pw = (size_t)C::SM * sizeof(double);
+    // The PIN instantiation's RP extra doubles per warp (R staged next to z) fit in the slack of the same CTA shape for
+    // every built shape: see the static_assert below.
+    constexpr size_t pw = (size_t)(PIN ? C::SMP : C::SM) * sizeof(double);
     constexpr size_t SM_BYTES = 228 * 1024, CTA_MAX = 227 * 1024, RSV = 1024;
 #ifdef SLB_USCKF_WPB
     constexpr int WPB = SLB_USCKF_WPB;   // experiment knob (compile time)
@@ -151,7 +153,15 @@ static int launch_step_t(const FilterArgs &a, cudaStream_t s) {
     constexpr int fit = (int)(SM_BYTES / (smem + RSV));
     constexpr int cap = 12 / WPB < 1 ? 1 : 12 / WPB;
     constexpr int MINB = fit > cap ? cap : fit < 1 ? 1 : fit;
-    auto kern = slbd::usckf_step_kernel<SLB_PM_USCKF_TEST, NK, NL, PRED, UPD, WPB, MINB>;
+#ifndef SLB_USCKF_WPB
+    {   // per-instance noise must not cost the fused step a CTA
+        constexpr size_t pw0 = (size_t)C::SM * sizeof(double);
+        constexpr int WPB0 = 2 * (6 * pw0 + RSV) <= SM_BYTES ? 6 : 4;
+        constexpr int fit0 = (int)(SM_BYTES / ((size_t)WPB0 * pw0 + RSV));
+        static_assert(!PIN || (WPB == WPB0 && fit >= (fit0 < 12 / WPB0 ? fit0 : 12 / WPB0)), "PIN costs occupancy");
+    }
+#endif
+    auto kern = slbd::usckf_step_kernel<SLB_PM_USCKF_TEST, NK, NL, PRED, UPD, WPB, MINB, PIN>;
     SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     // L2 prefetch distance in instances: SLB_USCKF_PREFETCH waves of (SMs x resident warps); default off (measured: no
     // gain at 0 / 1 / 2 / 4 waves, and 16 % more DRAM reads at the full fleet size)
@@ -179,14 +189,17 @@ static int launch_step_t(const FilterArgs &a, cudaStream_t s) {
 
 template <int NK, int NL>
 static int launch_step_nknl(bool predict, const FilterArgs &a, cudaStream_t s) {
-    return predict ? launch_step_t<NK, NL, true, true>(a, s) : launch_step_t<NK, NL, false, true>(a, s);
+    if ((predict && a.qs) || a.rs)
+        return predict ? launch_step_t<NK, NL, true, true, true>(a, s) : launch_step_t<NK, NL, false, true, true>(a, s);
+    return predict ? launch_step_t<NK, NL, true, true, false>(a, s) : launch_step_t<NK, NL, false, true, false>(a, s);
 }
 
 int launch_usckf(int pm, int mm, bool predict, bool update, const FilterArgs &a, cudaStream_t s) {
     if (predict && pm != SLB_PM_USCKF_TEST) return set_error(SLB_ERR_INVALID, "usckf: unsupported process model");
     if (update && mm != SLB_MM_USCKF_VO) return set_error(SLB_ERR_INVALID, "usckf: unsupported measurement model");
     // predict alone touches rows 24..35 of the record only: the partial-record kernel of slb_predict12.cuh
-    if (predict && !update) return launch_predict_t<SLB_PM_USCKF_TEST>(a, s);
+    if (predict && !update)
+        return a.qs ? launch_predict_t<SLB_PM_USCKF_TEST, true>(a, s) : launch_predict_t<SLB_PM_USCKF_TEST, false>(a, s);
     if (update) {
 #define SLB_USCKF_SHAPE(NK_, NL_) \
     if (a.nk == NK_ && a.nl == NL_) return launch_step_nknl<NK_, NL_>(predict, a, s);

@@ -76,6 +76,10 @@ struct StepCfg {
     static constexpr int SCR = (UPD_SCR > PRED_SCR ? UPD_SCR : PRED_SCR);
     static constexpr int ZS = (NK_ + 1) / 2 * 2;
     static constexpr int SM = PSTR + QS + SCR + ZS + 2;    // doubles per warp (even); last slot = mbarrier
+    // per-instance noise (the PIN instantiation): the lower triangle of this instance's R, packed, between z and the
+    // mbarrier.  (Its Q entries travel in registers: 6 per lane, see load_q_entries.)
+    static constexpr int RP = (NK_ * (NK_ + 1) / 2 + 1) / 2 * 2;
+    static constexpr int SMP = SM + RP;
     static_assert(NK_ % 3 == 0 && NK_ >= 3, "the VO model moves 3-D features");
     static_assert(N <= 64, "two rows per lane");
     static_assert(SM % 2 == 0 && PSTR % 2 == 0 && QS % 2 == 0, "16-byte alignment of the bulk copies");
@@ -391,9 +395,10 @@ struct PanelStep<C, C::NPAN> {
 };
 
 // update of the resident record.  Returns status bits; `dirty` is set when Ps / mus changed.
-template <int NK, int NL>
-SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double *zs, const slb::FilterArgs &a, int lane,
-                              bool &dirty) {
+// PIN: R comes from `Rs`, this instance's packed lower triangle staged in shared memory (cp.async, issued with z).
+template <int NK, int NL, bool PIN = false>
+SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double *zs, const double *Rs,
+                              const slb::FilterArgs &a, int lane, bool &dirty) {
     typedef StepCfg<NK, NL> C;
     constexpr int N = C::N, NT = C::NT, NPAD = C::NPAD, JLAST = C::JLAST, KP = C::KP;
     const int a_ = lane & 3, b_ = lane >> 2;
@@ -447,6 +452,11 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
     // ---- mean / innovation covariance (:280-282) from the deviations e = Z - Z0 -----------------------------------
     constexpr double NS = (double)(2 * N + 1);
     double ebar[NK], S[NK * (NK + 1) / 2];
+    if (PIN) {   // the staged R (and z) must have landed, and be visible to the whole warp
+        asm volatile("cp.async.wait_group 0;\n" ::: "memory");
+        __syncwarp();
+    }
+    auto Rv = [&](int r, int c) { return PIN ? Rs[tri(r, c)] : __ldg(a.R + r * NK + c); };
     if (NK == 3) {   // 3 + 6 sums in one reduce-scatter pass (the d_k slots are dead: every sigma point has been drawn)
         double v[12], o[12];
 #pragma unroll
@@ -461,7 +471,7 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
         for (int r = 0; r < NK; ++r)
 #pragma unroll
             for (int c = 0; c <= r; ++c)
-                S[tri(r, c)] = 0.5 * fma(-NS * ebar[r], ebar[c], o[3 + tri(r, c)]) + __ldg(a.R + r * NK + c);
+                S[tri(r, c)] = 0.5 * fma(-NS * ebar[r], ebar[c], o[3 + tri(r, c)]) + Rv(r, c);
     } else {
 #pragma unroll
         for (int c = 0; c < NK; ++c) ebar[c] = warp_sum(s.esum[c]) * (1.0 / NS);
@@ -469,7 +479,7 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
         for (int r = 0; r < NK; ++r)
 #pragma unroll
             for (int c = 0; c <= r; ++c)
-                S[tri(r, c)] = 0.5 * fma(-NS * ebar[r], ebar[c], warp_sum(s.eep[tri(r, c)])) + __ldg(a.R + r * NK + c);
+                S[tri(r, c)] = 0.5 * fma(-NS * ebar[r], ebar[c], warp_sum(s.eep[tri(r, c)])) + Rv(r, c);
     }
     // ---- K = covXZ S^-1 (:286-288), innovation, Mahalanobis gate (:290-294) --------------------------------------
     double Si[NK * (NK + 1) / 2];
@@ -584,9 +594,10 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
 
 // predict of the resident record (statek_i: rows 24..35, mean at q-offset 26); see predict12_kernel for the scheme.
 // Returns status bits; `dirty` is set when Ps / mus changed.
-template <int PM, int NF>
-SLB_DEV int usckf_predict_smem(double *Ps, double *mus, double *scr, const double *u, double dt, const double *Qg, int lane,
-                               bool &dirty) {
+// PIN: Q comes from `qv`, the 6 entries this lane adds (load_q_entries), instead of the shared matrix at Qg.
+template <int PM, int NF, bool PIN = false>
+SLB_DEV int usckf_predict_smem(double *Ps, double *mus, double *scr, const double *u, double dt, const double *Qg,
+                               const double *qv, int lane, bool &dirty) {
     typedef LayState12 L;
     typedef CycCfg<12> C;
     constexpr int ROW0 = 24, MU0 = 26, N = 36 + NF;
@@ -685,13 +696,13 @@ SLB_DEV int usckf_predict_smem(double *Ps, double *mus, double *scr, const doubl
             W[e] = 0.5 * (D[(1 + 2 * jj) * PRED_DS + c] - D[(2 + 2 * jj) * PRED_DS + c]);
         }
         __syncwarp();   // the old block (rows 24..35, cols 24..35) was consumed by the factorisation: overwrite it
-        auto put = [&](int r, int c, double v) {
-            if (r < 12 && c <= r) PR(r, ROW0 + c) = 0.5 * v + __ldg(Qg + r * 12 + c);
+        auto put = [&](int r, int c, double v, int k) {
+            if (r < 12 && c <= r) PR(r, ROW0 + c) = 0.5 * v + (PIN ? qv[k] : __ldg(Qg + r * 12 + c));
         };
         const int r = b_, c = 2 * a_;
-        put(r, c, c00[0]); put(r, c + 1, c00[1]);
-        put(8 + r, c, c10[0]); put(8 + r, c + 1, c10[1]);
-        put(8 + r, 8 + c, c11[0]); put(8 + r, 8 + c + 1, c11[1]);
+        put(r, c, c00[0], 0); put(r, c + 1, c00[1], 1);
+        put(8 + r, c, c10[0], 2); put(8 + r, c + 1, c10[1], 3);
+        put(8 + r, 8 + c, c11[0], 4); put(8 + r, 8 + c + 1, c11[1], 5);
     }
     // ---- Fk = W^T L^-1  <=>  L^T Fk^T = W: lane c back-substitutes column c (:154); L(p,r) = U(p,r) / sqrt(d_r) --
     if (lane < 12) {
@@ -773,15 +784,20 @@ SLB_DEV int usckf_predict_smem(double *Ps, double *mus, double *scr, const doubl
 
 // One instance per warp: record in (TMA bulk load), predict and / or update in shared memory, record out (TMA bulk
 // store).  PRED && UPD is the fused step (slb_usckf_step, the *_step_host paths); UPD alone is slb_usckf_update.
-template <int PM, int NK, int NL, bool PRED, bool UPD, int WPB, int MINB>
+// PIN: per-instance noise (slb_set_noise_layout), Q at a.Q + inst * a.qs and R at a.R + inst * a.rs (stride 0 = shared).
+// Both are fetched with the record: R's lower triangle by cp.async into RP extra doubles of the warp's area, the 6 Q
+// entries a lane adds into registers.
+template <int PM, int NK, int NL, bool PRED, bool UPD, int WPB, int MINB, bool PIN = false>
 __global__ void __launch_bounds__(WPB * 32, MINB) usckf_step_kernel(slb::FilterArgs a) {
     typedef StepCfg<NK, NL> C;
+    constexpr int SMW = PIN ? C::SMP : C::SM;
     extern __shared__ __align__(128) double smem[];
     const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
     const int inst = blockIdx.x * WPB + w;
     if (inst >= a.B) return;
-    double *Ps = smem + (size_t)w * C::SM, *mus = Ps + C::PSTR, *scr = mus + C::QS, *zs = scr + C::SCR;
-    uint64_t *bar = reinterpret_cast<uint64_t *>(zs + C::ZS);
+    double *Ps = smem + (size_t)w * SMW, *mus = Ps + C::PSTR, *scr = mus + C::QS, *zs = scr + C::SCR;
+    double *Rs = zs + C::ZS;   // PIN only
+    uint64_t *bar = reinterpret_cast<uint64_t *>(zs + C::ZS + (PIN ? C::RP : 0));
     double *Pg = a.P + (size_t)inst * a.pstride;
     double *mug = a.mu + (size_t)inst * a.qstride;
     if (lane == 0) {
@@ -799,6 +815,18 @@ __global__ void __launch_bounds__(WPB * 32, MINB) usckf_step_kernel(slb::FilterA
                      "l"(a.z + (size_t)inst * NK + lane)
                      : "memory");
     }
+    if (PIN && UPD) {   // lower triangle of this instance's R, packed (Rs[tri(r, c)])
+        const double *Ri = a.R + (size_t)inst * a.rs;
+        for (int e = lane; e < NK * (NK + 1) / 2; e += 32) {
+            int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
+            r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
+            asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(saddr(Rs + e)), "l"(Ri + r * NK + (e - tri(r, 0)))
+                         : "memory");
+        }
+        asm volatile("cp.async.commit_group;\n" ::: "memory");
+    }
+    double qv[PIN && PRED ? 6 : 1];
+    if (PIN && PRED) load_q_entries(a.Q + (size_t)inst * a.qs, lane & 3, lane >> 2, qv);
     double u[ProcessModel<PM>::NU];
     if (PRED) {
 #pragma unroll
@@ -809,9 +837,9 @@ __global__ void __launch_bounds__(WPB * 32, MINB) usckf_step_kernel(slb::FilterA
     SLB_CTA_SYNC();
     int st = 0;
     bool dirty = false;
-    if (PRED) st |= usckf_predict_smem<PM, NK + NL>(Ps, mus, scr, u, a.dt, a.Q, lane, dirty);
+    if (PRED) st |= usckf_predict_smem<PM, NK + NL, PIN>(Ps, mus, scr, u, a.dt, a.Q, qv, lane, dirty);
     if (PRED) SLB_CTA_SYNC();
-    if (UPD) st |= usckf_update_smem<NK, NL>(Ps, mus, scr, zs, a, lane, dirty);
+    if (UPD) st |= usckf_update_smem<NK, NL, PIN>(Ps, mus, scr, zs, Rs, a, lane, dirty);
     asm volatile("cp.async.wait_group 0;\n" ::: "memory");   // (an update that bailed out early has not waited for z)
     // ---- record out ----------------------------------------------------------------------------------------------
     if (dirty) {

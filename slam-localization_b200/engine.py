@@ -21,6 +21,7 @@ STATEK, STATEK_L, STATEK_I = 1, 2, 3
 FIELD_MU, FIELD_P, FIELD_STATUS, FIELD_OUTLIERS = 1, 2, 3, 4
 ST_CHOL_FAIL, ST_MEAN_NOCONV, ST_GATE_REJECT, ST_NONFINITE, ST_QR_ROWS = 1, 2, 4, 8, 16
 NSTATUS = 5
+NOISE_Q_PER_INSTANCE, NOISE_R_PER_INSTANCE = 1, 2
 
 EXPORTS = [
     "slb_version", "slb_last_error", "slb_create", "slb_destroy", "slb_dof", "slb_qdim", "slb_upload",
@@ -32,7 +33,7 @@ EXPORTS = [
     "slb_msckf_step_host", "slb_ekf_predict", "slb_ekf_update", "slb_ekf_single_update", "slb_ekf_clone",
     "slb_datamodel_safe_fuse", "slb_msckf_update_ekf", "slb_transform_compose", "slb_deadreckon_update_pose",
     "slb_ukf_step_host_async", "slb_usckf_step_host_async", "slb_msckf_step_host_async", "slb_wait",
-    "slb_set_output_slice", "slb_check_sigma_points", "slb_gather_stats", "slb_nccl_unique_id", "slb_nccl_comm_init", "slb_nccl_comm_destroy",
+    "slb_set_output_slice", "slb_set_noise_layout", "slb_check_sigma_points", "slb_gather_stats", "slb_nccl_unique_id", "slb_nccl_comm_init", "slb_nccl_comm_destroy",
 ]
 
 
@@ -78,6 +79,7 @@ def lib():
         L.slb_usckf_step_host_async.argtypes = L.slb_usckf_step_host.argtypes
         L.slb_wait.argtypes = [vp, vp]
         L.slb_set_output_slice.argtypes = [vp, i32, i32]
+        L.slb_set_noise_layout.argtypes = [vp, i32]
         L.slb_check_sigma_points.argtypes = [vp, vp, vp, vp]
         L.slb_gather_stats.argtypes = [vp, vp, dp, vp]
         L.slb_nccl_unique_id.argtypes = [vp]
@@ -191,6 +193,7 @@ class Batch:
         self.N = lib().slb_dof(self.h)
         self.QD = lib().slb_qdim(self.h)
         self.kind, self.nk, self.nl, self.k = kind, nk, nl, nclones
+        self.noise = 0   # slb_set_noise_layout flags of the handle
 
     def close(self):
         if self.h:
@@ -248,6 +251,42 @@ class Batch:
         """Part of the posterior q-vector step_host copies back (default: all); e.g. (26, 13) = statek_i of a USCKF."""
         check(lib().slb_set_output_slice(self.h, offset, count))
 
+    def set_noise_layout(self, flags):
+        """slb_set_noise_layout: NOISE_Q_PER_INSTANCE / NOISE_R_PER_INSTANCE make the device entry points read Q / R as
+        batch x n x n arrays (one matrix per instance); 0 = one matrix shared by the batch.  The filter methods call it
+        themselves from the shapes of the Q / R they are given."""
+        check(lib().slb_set_noise_layout(self.h, flags))
+        self.noise = flags
+
+    def _noise_bit(self, name, a, n, bit):
+        """The layout bit a noise matrix asks for: (n, n) is shared by the batch, (B, n, n) one matrix per instance."""
+        shape = tuple(a.t.shape) if isinstance(a, DeviceArray) else tuple(a.shape) if hasattr(a, "shape") else np.shape(a)
+        if shape == (n, n):
+            return 0
+        if shape == (self.B, n, n):
+            return bit
+        raise ValueError("%s must have shape (%d, %d) (shared by the batch) or (%d, %d, %d) (one per instance), got %s"
+                         % (name, n, n, self.B, n, n, shape))
+
+    def _use_noise(self, Q=None, n=0, R=None, m=0):
+        """Checks the shapes of Q (n x n) / R (m x m) and sets the handle's noise layout to what they ask for (the bit of
+        a matrix that is not passed is left as it is)."""
+        flags = self.noise
+        if Q is not None:
+            flags = (flags & ~NOISE_Q_PER_INSTANCE) | self._noise_bit("Q", Q, n, NOISE_Q_PER_INSTANCE)
+        if R is not None:
+            flags = (flags & ~NOISE_R_PER_INSTANCE) | self._noise_bit("R", R, m, NOISE_R_PER_INSTANCE)
+        if flags != self.noise:
+            self.set_noise_layout(flags)
+
+    def _host_noise(self, Q, n, R, m):
+        """The host-buffer steps take shared noise only (per-instance noise is device-resident, slb_set_noise_layout): an
+        array holding batch x n x n values is refused, anything else is passed through as before (n x n read)."""
+        if self.B > 1 and (np.size(Q) == self.B * n * n or np.size(R) == self.B * m * m):
+            raise ValueError("step_host takes Q and R shared by the batch; per-instance noise needs the device entry points")
+        if self.noise:
+            self.set_noise_layout(0)
+
     def wait(self):
         """Completes the steps enqueued with step_host(..., wait=False) on the current stream."""
         check(lib().slb_wait(self.h, _stream()))
@@ -303,20 +342,26 @@ class Ukf(Batch):
         super().__init__(KIND_UKF, batch, layout=layout, device=device)
 
     def predict(self, pm, u, dt, Q):
+        """Q: (n, n) shared by the batch or (batch, n, n) one per instance."""
+        self._use_noise(Q=Q, n=self.N)
         u, Q = dev(u), dev(Q)
         check(lib().slb_ukf_predict(self.h, pm, u.ptr, dt, Q.ptr, _stream()))
 
     def update(self, mm, z, R, gate_dof=0):
+        """R: (3, 3) shared by the batch or (batch, 3, 3) one per instance."""
+        self._use_noise(R=R, m=3)
         z, R = dev(z), dev(R)
         check(lib().slb_ukf_update(self.h, mm, z.ptr, R.ptr, gate_dof, _stream()))
 
     def step(self, pm, mm, u, dt, Q, z, R, gate_dof=0):
+        self._use_noise(Q=Q, n=self.N, R=R, m=3)
         u, Q, z, R = dev(u), dev(Q), dev(z), dev(R)
         check(lib().slb_ukf_step(self.h, pm, mm, u.ptr, dt, Q.ptr, z.ptr, R.ptr, gate_dof, _stream()))
 
     def step_host(self, pm, mm, u, dt, Q, z, R, gate_dof=0, mu_out=None, wait=True):
         """u, z, Q, R are HOST arrays (numpy or pinned torch); returns/fills the posterior means.  wait=False is the
         pipelined flavour (slb_ukf_step_host_async): call .wait() before touching the buffers again."""
+        self._host_noise(Q, self.N, R, 3)
         fn = lib().slb_ukf_step_host if wait else lib().slb_ukf_step_host_async
         check(fn(self.h, pm, mm, _ptr_of(u), dt, _ptr_of(Q), _ptr_of(z), _ptr_of(R), gate_dof,
                  _ptr_of(mu_out) if mu_out is not None else None, _stream()))
@@ -329,18 +374,24 @@ class Usckf(Batch):
         super().__init__(KIND_USCKF, batch, nk=nk, nl=nl, device=device)
 
     def predict(self, pm, u, dt, Q):
+        """Q: (12, 12) shared by the batch or (batch, 12, 12) one per instance."""
+        self._use_noise(Q=Q, n=12)
         u, Q = dev(u), dev(Q)
         check(lib().slb_usckf_predict(self.h, pm, u.ptr, dt, Q.ptr, _stream()))
 
     def update(self, mm, z, R, gate_dof=0):
+        """R: (nk, nk) shared by the batch or (batch, nk, nk) one per instance."""
+        self._use_noise(R=R, m=self.nk)
         z, R = dev(z), dev(R)
         check(lib().slb_usckf_update(self.h, mm, z.ptr, R.ptr, gate_dof, _stream()))
 
     def step(self, pm, mm, u, dt, Q, z, R, gate_dof=0):
+        self._use_noise(Q=Q, n=12, R=R, m=self.nk)
         u, Q, z, R = dev(u), dev(Q), dev(z), dev(R)
         check(lib().slb_usckf_step(self.h, pm, mm, u.ptr, dt, Q.ptr, z.ptr, R.ptr, gate_dof, _stream()))
 
     def step_host(self, pm, mm, u, dt, Q, z, R, gate_dof=0, mu_out=None, wait=True):
+        self._host_noise(Q, 12, R, self.nk)
         fn = lib().slb_usckf_step_host if wait else lib().slb_usckf_step_host_async
         check(fn(self.h, pm, mm, _ptr_of(u), dt, _ptr_of(Q), _ptr_of(z), _ptr_of(R), gate_dof,
                  _ptr_of(mu_out) if mu_out is not None else None, _stream()))
@@ -349,6 +400,8 @@ class Usckf(Batch):
         check(lib().slb_usckf_clone(self.h, mode, _stream()))
 
     def set_measurement(self, mode, z, R):
+        """R: (len, len) shared by the batch or (batch, len, len) one per instance, len = nk (STATEK) or nl (STATEK_L)."""
+        self._use_noise(R=R, m=self.nk if mode == STATEK else self.nl)
         z, R = dev(z), dev(R)
         check(lib().slb_usckf_set_measurement(self.h, mode, z.ptr, R.ptr, _stream()))
 
@@ -360,6 +413,8 @@ class Msckf(Batch):
         super().__init__(KIND_MSCKF, batch, nclones=nclones, device=device)
 
     def predict(self, pm, u, dt, Q):
+        """Q: (12, 12) shared by the batch or (batch, 12, 12) one per instance."""
+        self._use_noise(Q=Q, n=12)
         u, Q = dev(u), dev(Q)
         check(lib().slb_msckf_predict(self.h, pm, u.ptr, dt, Q.ptr, _stream()))
 
@@ -377,6 +432,7 @@ class Msckf(Batch):
     def step_host(self, pm, mm, u, dt, Q, params, z, R, gate=True, mu_out=None, wait=True):
         """predict + update with HOST arrays (numpy or pinned torch); fills the posterior means."""
         m = z.shape[1]
+        self._host_noise(Q, 12, R, m)
         nparams = int(np.prod(params.shape))
         fn = lib().slb_msckf_step_host if wait else lib().slb_msckf_step_host_async
         check(fn(self.h, pm, mm, _ptr_of(u), dt, _ptr_of(Q), _ptr_of(params), nparams, m, _ptr_of(z), _ptr_of(R), int(gate),

@@ -76,6 +76,21 @@ class Batch {
   protected:
     slb_handle h_ = nullptr;
     int B_ = 0, N_ = 0, QD_ = 0;
+    int noise_ = 0;   // slb_set_noise_layout flags of the handle
+    // Noise matrices are n x n row-major: n*n doubles are shared by the batch, batch*n*n doubles are one matrix per
+    // instance (with batch == 1 the two are the same thing, as in the reference).  Sets the handle's layout bit `bit`
+    // from the length of `v`; any other length throws.
+    void useNoise(const Vec &v, size_t n, int bit, const char *what) {
+        int flag;
+        if (v.size() == n * n) flag = 0;
+        else if (v.size() == (size_t)B_ * n * n) flag = bit;
+        else throw Error(SLB_ERR_INVALID, (std::string(what) + ": noise must hold n*n or batch*n*n doubles").c_str());
+        const int flags = (noise_ & ~bit) | flag;
+        if (flags != noise_) {
+            check(slb_set_noise_layout(h_, flags), "slb_set_noise_layout");
+            noise_ = flags;
+        }
+    }
     void create(int kind, int batch, int layout, int nk, int nl, int nclones, int device) {
         slb_config cfg = {};
         cfg.kind = kind; cfg.layout = layout; cfg.batch = batch; cfg.nk = nk; cfg.nl = nl; cfg.nclones = nclones;
@@ -143,13 +158,15 @@ class Ukf : public Batch {
         setMu(mu0);
         setPk(sigma0);
     }
-    // u: batch x nu control inputs of process model `g`; Q: n x n
+    // u: batch x nu control inputs of process model `g`; Q: n x n, or batch x n x n (one per instance)
     void predict(int g, const Vec &u, double dt, const Vec &Q) {
+        useNoise(Q, N_, SLB_NOISE_Q_PER_INSTANCE, "Ukf::predict");
         DevBuf du(u), dQ(Q);
         check(slb_ukf_predict(h_, g, du.get(), dt, dQ.get(), nullptr), "slb_ukf_predict");
     }
-    // gate_dof = 0 is ukfom::accept_any_mahalanobis_distance
+    // gate_dof = 0 is ukfom::accept_any_mahalanobis_distance; R: 3 x 3, or batch x 3 x 3
     void update(const Vec &z, int h, const Vec &R, int gate_dof = 0) {
+        useNoise(R, 3, SLB_NOISE_R_PER_INSTANCE, "Ukf::update");
         DevBuf dz(z), dR(R);
         check(slb_ukf_update(h_, h, dz.get(), dR.get(), gate_dof, nullptr), "slb_ukf_update");
     }
@@ -186,18 +203,22 @@ class Usckf : public Batch {
         cloning(STATEK_I);
         cloning(STATEK_L);
     }
+    // Q: 12 x 12, or batch x 12 x 12 (one per instance); R: nk x nk, or batch x nk x nk
     void predict(int f, const Vec &u, double dt, const Vec &Q) {                       // Usckf.hpp:107-244
+        useNoise(Q, 12, SLB_NOISE_Q_PER_INSTANCE, "Usckf::predict");
         DevBuf du(u), dQ(Q);
         check(slb_usckf_predict(h_, f, du.get(), dt, dQ.get(), nullptr), "slb_usckf_predict");
     }
     void update(const Vec &z, int h, const Vec &R, int gate_dof = 0) {                // Usckf.hpp:246-308
+        useNoise(R, (size_t)nk_, SLB_NOISE_R_PER_INSTANCE, "Usckf::update");
         DevBuf dz(z), dR(R);
         check(slb_usckf_update(h_, h, dz.get(), dR.get(), gate_dof, nullptr), "slb_usckf_update");
     }
     void setMeasurement(CloningMode mode, const Vec &z, const Vec &R) {               // Usckf.hpp:322-389
         const size_t len = mode == STATEK ? nk_ : nl_;
-        if (z.size() != len * B_ || R.size() != len * len)                            // the asserts at :325-327
+        if (z.size() != len * B_ || (R.size() != len * len && R.size() != B_ * len * len))   // the asserts at :325-327
             throw Error(SLB_ERR_INVALID, "setMeasurement: z.size() must equal R.rows() == R.cols()");
+        useNoise(R, len, SLB_NOISE_R_PER_INSTANCE, "Usckf::setMeasurement");   // R: len x len, or batch x len x len
         DevBuf dz(z), dR(R);
         check(slb_usckf_set_measurement(h_, mode, dz.get(), dR.get(), nullptr), "slb_usckf_set_measurement");
     }
@@ -251,7 +272,9 @@ class Msckf : public Batch {
         setMu(state);
         setPk(P0);
     }
+    // Q: 12 x 12, or batch x 12 x 12 (one per instance)
     void predict(int f, const Vec &u, double dt, const Vec &Q) {                        // Msckf.hpp:89-189
+        useNoise(Q, 12, SLB_NOISE_Q_PER_INSTANCE, "Msckf::predict");
         DevBuf du(u), dQ(Q);
         check(slb_msckf_predict(h_, f, du.get(), dt, dQ.get(), nullptr), "slb_msckf_predict");
     }
