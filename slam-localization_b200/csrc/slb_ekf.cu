@@ -17,18 +17,11 @@
 // (O(N^2 m) instead of two N^3 products) and symmetrised as 0.5 (P + P^T) like :359.
 #include "slb_internal.h"
 #include "slb_math.cuh"
+#include "slb_ptx.cuh"
 
 namespace slbd {
 
 constexpr int EKF_NS = 15, EKF_NA = 45, EKF_QS = 16, EKF_QA = 48;
-constexpr unsigned EKF_FULL = 0xffffffffu;
-
-// 8-byte LDGSTS: the loads of a record are all issued before the first one lands (instance records are only 8-byte
-// aligned -- 2025 doubles -- so the 16-byte form does not apply); one wait for the lot.
-SLB_DEV void ekf_cp8(double *smem_dst, const double *gsrc) {
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"((unsigned)__cvta_generic_to_shared(smem_dst)), "l"(gsrc) : "memory");
-}
-SLB_DEV void ekf_cp_wait() { asm volatile("cp.async.commit_group;\n cp.async.wait_group 0;\n" ::: "memory"); }
 
 // closed-form inverse of a general 3x3 (Eigen's fixed-size path: cofactors / determinant)
 SLB_DEV void inv3(const double *A, double *C) {
@@ -54,9 +47,6 @@ SLB_DEV void inv3(const double *A, double *C) {
 constexpr int EKP_FS = 20, EKP_RS = 52;   // row strides of F (16 x 16 padded) and of the block row (16 x 48 padded):
                                           // = 4 (mod 16) doubles, so a 4 x 8 fragment load touches 32 distinct banks
 constexpr int EKP_SM = 16 * EKP_FS + 16 * EKP_RS;
-SLB_DEV void ekf_dmma(double &d0, double &d1, double a, double b) {
-    asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0,%1}, {%2}, {%3}, {%0,%1};\n" : "+d"(d0), "+d"(d1) : "d"(a), "d"(b));
-}
 template <int WPB>
 __global__ void __launch_bounds__(WPB * 32) ekf_predict_kernel(int64_t n, double *err, double *P, const double *F, const double *Q) {
     extern __shared__ __align__(16) double sm[];
@@ -67,21 +57,23 @@ __global__ void __launch_bounds__(WPB * 32) ekf_predict_kernel(int64_t n, double
     double *Fs = sm + (size_t)w * EKP_SM, *Rs = Fs + 16 * EKP_FS;
     double *Pg = P + inst * (EKF_NA * EKF_NA);
     const double *Fg = F + inst * (EKF_NS * EKF_NS);
-    for (int e = lane; e < 225; e += 32) ekf_cp8(Fs + (e / 15) * EKP_FS + e % 15, Fg + e);
-    for (int e = lane; e < 675; e += 32) ekf_cp8(Rs + (e / 45) * EKP_RS + e % 45, Pg + 30 * 45 + e);
+    // 8-byte LDGSTS: the loads of a record are all issued before the first one lands (instance records are only 8-byte
+    // aligned -- 2025 doubles -- so the 16-byte form does not apply); one wait for the lot.
+    for (int e = lane; e < 225; e += 32) cp_async8(Fs + (e / 15) * EKP_FS + e % 15, Fg + e);
+    for (int e = lane; e < 675; e += 32) cp_async8(Rs + (e / 45) * EKP_RS + e % 45, Pg + 30 * 45 + e);
     // zero padding of the k-dimension (column 15 of F, row 15 of the block row) and of the unused columns 45..47
     if (lane < 16) { Fs[lane * EKP_FS + 15] = 0.0; Fs[15 * EKP_FS + lane] = 0.0; }
     for (int e = lane; e < 48; e += 32) Rs[15 * EKP_RS + e] = 0.0;
     for (int e = lane; e < 48; e += 32) Rs[(e / 3) * EKP_RS + 45 + e % 3] = 0.0;
     double ei = lane < 15 ? err[inst * EKF_NA + 30 + lane] : 0.0;
-    ekf_cp_wait();
+    cp_async_wait_all();
     __syncwarp();
     // mu_error.statek_i <- F mu_error.statek_i (:93)
     {
         double s = 0.0;
 #pragma unroll
         for (int k = 0; k < 15; ++k) {
-            const double ek = __shfl_sync(EKF_FULL, ei, k);
+            const double ek = __shfl_sync(FULL, ei, k);
             if (lane < 15) s += Fs[lane * EKP_FS + k] * ek;
         }
         if (lane < 15) err[inst * EKF_NA + 30 + lane] = s;
@@ -99,8 +91,8 @@ __global__ void __launch_bounds__(WPB * 32) ekf_predict_kernel(int64_t n, double
 #pragma unroll
         for (int kq = 0; kq < 4; ++kq) {
             const double bv = Rs[(4 * kq + fk) * EKP_RS + 8 * J + fr];   // B[k][n] = row k, column 8J + n
-            ekf_dmma(y0[0], y0[1], fa[0][kq], bv);
-            ekf_dmma(y1[0], y1[1], fa[1][kq], bv);
+            dmma884(y0[0], y0[1], fa[0][kq], bv);
+            dmma884(y1[0], y1[1], fa[1][kq], bv);
         }
         __syncwarp();
         Rs[fr * EKP_RS + 8 * J + 2 * fk] = y0[0];
@@ -119,10 +111,10 @@ __global__ void __launch_bounds__(WPB * 32) ekf_predict_kernel(int64_t n, double
 #pragma unroll
         for (int kq = 0; kq < 4; ++kq) {
             const double a0 = Rs[fr * EKP_RS + 30 + 4 * kq + fk], a1 = Rs[(8 + fr) * EKP_RS + 30 + 4 * kq + fk];
-            ekf_dmma(c[0][0][0], c[0][0][1], a0, fa[0][kq]);
-            ekf_dmma(c[0][1][0], c[0][1][1], a0, fa[1][kq]);
-            ekf_dmma(c[1][0][0], c[1][0][1], a1, fa[0][kq]);
-            ekf_dmma(c[1][1][0], c[1][1][1], a1, fa[1][kq]);
+            dmma884(c[0][0][0], c[0][0][1], a0, fa[0][kq]);
+            dmma884(c[0][1][0], c[0][1][1], a0, fa[1][kq]);
+            dmma884(c[1][0][0], c[1][0][1], a1, fa[0][kq]);
+            dmma884(c[1][1][0], c[1][1][1], a1, fa[1][kq]);
         }
         __syncwarp();
 #pragma unroll
@@ -181,7 +173,7 @@ SLB_DEV bool joseph_update(double *Pl, double *rows, const double *Hs, const dou
 #pragma unroll
             for (int kq = 0; kq < KQ; ++kq) {
                 const int jc = min(4 * kq + fk, N - 1);
-                ekf_dmma(d0, d1, Pl[ri >= jc ? tr0 + jc : tri(jc, ri)], hb[kq]);
+                dmma884(d0, d1, Pl[ri >= jc ? tr0 + jc : tri(jc, ri)], hb[kq]);
             }
             const int r = 8 * I + fr;
             if (r < N) {
@@ -205,13 +197,13 @@ SLB_DEV bool joseph_update(double *Pl, double *rows, const double *Hs, const dou
         const double h0 = i0 < N ? Hs[r * N + i0] : 0.0, h1 = i1 < N ? Hs[r * N + i1] : 0.0;
         double t = fma(h0, i0 < N ? xhat[i0] : 0.0, h1 * (i1 < N ? xhat[i1] : 0.0));
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(EKF_FULL, t, o);
+        for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(FULL, t, o);
         hx[r] = t;
 #pragma unroll
         for (int c = 0; c < M; ++c) {
             double v = fma(h0, A0[c], h1 * A1[c]);
 #pragma unroll
-            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(EKF_FULL, v, o);
+            for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
             S[r * M + c] = v + __ldg(Rg + r * M + c);
         }
     }
@@ -275,9 +267,9 @@ SLB_DEV bool joseph_update(double *Pl, double *rows, const double *Hs, const dou
             for (int J = 0; J <= I; ++J) {
                 const double *rj = rows + min(8 * J + fr, N - 1) * C::ROW;
                 double d0 = 0.0, d1 = 0.0;
-                ekf_dmma(d0, d1, xa0, rj[yo[0]]);
-                ekf_dmma(d0, d1, xa1, rj[yo[1]]);
-                ekf_dmma(d0, d1, xa2, rj[yo[2]]);
+                dmma884(d0, d1, xa0, rj[yo[0]]);
+                dmma884(d0, d1, xa1, rj[yo[1]]);
+                dmma884(d0, d1, xa2, rj[yo[2]]);
                 const int c = 8 * J + 2 * fk;
                 if (r < N) {
                     double *pr = Pl + tri(r, 0);
@@ -307,7 +299,7 @@ __global__ void __launch_bounds__(WPB * 32) ekf_update_kernel(int64_t n, const d
     for (int e = lane; e < C::NP; e += 32) {
         int i = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
         i += (tri(i + 1, 0) <= e) - (tri(i, 0) > e);
-        ekf_cp8(Pl + e, Pg + i * N + (e - tri(i, 0)));
+        cp_async8(Pl + e, Pg + i * N + (e - tri(i, 0)));
     }
     for (int e = lane; e < M * N; e += 32) Hs[e] = __ldg(H + e);
     // x_hat = mu_state vectorised with the error-quaternion convention (:331)
@@ -315,7 +307,7 @@ __global__ void __launch_bounds__(WPB * 32) ekf_update_kernel(int64_t n, const d
         const int s = e / EKF_NS, c = e - s * EKF_NS;
         xh[e] = mu[inst * EKF_QA + s * EKF_QS + (c < 6 ? c : c + 1)];
     }
-    ekf_cp_wait();
+    cp_async_wait_all();
     __syncwarp();
     double innov[M];
     const bool ok = joseph_update<N, M>(Pl, rows, Hs, xh, z + inst * M, R, gate, lane, innov);
@@ -349,11 +341,11 @@ __global__ void __launch_bounds__(WPB * 32) ekf_single_update_kernel(int64_t n, 
     double *Pg = P + inst * (EKF_NA * EKF_NA);
     for (int e = lane; e < N * N; e += 32) {
         const int i = e / N, j = e - i * N;
-        if (j <= i) ekf_cp8(Pl + tri(i, j), Pg + (30 + i) * EKF_NA + 30 + j);
+        if (j <= i) cp_async8(Pl + tri(i, j), Pg + (30 + i) * EKF_NA + 30 + j);
     }
     for (int e = lane; e < M * N; e += 32) Hs[e] = __ldg(H + e);
     if (lane < N) xk[lane] = err[inst * EKF_NA + 30 + lane];
-    ekf_cp_wait();
+    cp_async_wait_all();
     __syncwarp();
     double innov[M];
     const bool ok = joseph_update<N, M>(Pl, rows, Hs, xk, z + inst * M, R, gate, lane, innov);
@@ -374,7 +366,7 @@ __global__ void __launch_bounds__(WPB * 32) ekf_single_update_kernel(int64_t n, 
         }
     }
     double *s = mu + inst * EKF_QA + 2 * EKF_QS;
-    const double qx = __shfl_sync(EKF_FULL, x, 6), qy = __shfl_sync(EKF_FULL, x, 7), qz = __shfl_sync(EKF_FULL, x, 8);
+    const double qx = __shfl_sync(FULL, x, 6), qy = __shfl_sync(FULL, x, 7), qz = __shfl_sync(FULL, x, 8);
     if (lane < 6) s[lane] += x;                       // pos, vel
     else if (lane >= 9 && lane < N) s[lane + 1] += x;  // gbias, abias
     if (lane == 6) {

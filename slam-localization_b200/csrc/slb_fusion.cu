@@ -15,6 +15,7 @@
 // back through the same staging so stores are coalesced too.
 #include "slb_internal.h"
 #include "slb_math.cuh"
+#include "slb_ptx.cuh"
 
 namespace slbd {
 
@@ -148,14 +149,6 @@ SLB_DEV void inverse_fixed_cols(double *A, Sink sink) {
 }
 
 constexpr int FUSE_WARPS = 4;
-
-SLB_DEV void cp_async8(double *smem_dst, const double *gsrc) {
-    const unsigned sa = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(sa), "l"(gsrc) : "memory");
-}
-SLB_DEV void cp_async_wait_all() {
-    asm volatile("cp.async.commit_group;\n cp.async.wait_group 0;\n" ::: "memory");
-}
 
 template <int D>
 struct FuseCfg {

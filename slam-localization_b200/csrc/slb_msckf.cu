@@ -14,7 +14,7 @@
 //
 // FP64 tensor cores: every rank-k contraction here (S = Zc^T Zc, covXZ = L W, the trailing updates of the
 // blocked Cholesky / triangular solve, P - Y Y^T, the re-estimated covariance D^T D) runs as 8x8x4 DMMA
-// tiles (mma.sync.m8n8k4.f64).  profiles/r01_dmma_vs_dfma_peak.txt: on B200 the DMMA pipe delivers the same
+// tiles (m8n8k4, dmma884).  profiles/r01_dmma_vs_dfma_peak.txt: on B200 the DMMA pipe delivers the same
 // 37 TFLOP/s as the SIMT FP64 pipe, so it does not raise the roofline -- but one DMMA replaces 8 DFMA issue
 // slots per lane and needs 2 operand loads per 8 FMA instead of the 4x4 register tile's 8 per 16, and this
 // kernel was bound by instruction issue and shared-memory operand traffic (FP64 pipe 7.5 % busy before),
@@ -505,11 +505,11 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_update_kernel(slb::FilterArgs a
         if (have_l) {
             for (int e = tid; e < NP; e += MS_T) RA[e] = RC[MS_NXL + e];
         } else {
-            for (int e = tid; e < NP; e += MS_T) pred_cp_async8(RA + e, Pg + e);
+            for (int e = tid; e < NP; e += MS_T) cp_async8(RA + e, Pg + e);
         }
         for (int e = tid; e < QD; e += MS_T) mu[e] = mug[e];
         if (tid == 0) { flags[0] = have_l ? flags[5] : 1; flags[1] = M; flags[2] = 0; }
-        pred_cp_async_wait_all();
+        cp_async_wait_all();
         __syncthreads();
         MS_PH(1);
         // ---- L = chol(Pk) (:229 -> :412), unless the previous iteration already did it ------------------
@@ -737,7 +737,7 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_update_kernel(slb::FilterArgs a
         const bool more = inst + (int)gridDim.x < a.B;
         if (more) {
             const double *Pn = a.P + (size_t)(inst + gridDim.x) * a.pstride;
-            for (int e = tid; e < NP; e += MS_T) pred_cp_async8(RB + e, Pn + e);
+            for (int e = tid; e < NP; e += MS_T) cp_async8(RB + e, Pn + e);
             if (tid == 0) flags[5] = 1;
         }
         // ---- delta = Y w, w = the extra row of the solve ---------------------------------------------------------
@@ -774,7 +774,7 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_update_kernel(slb::FilterArgs a
                 }
             }
         }
-        pred_cp_async_wait_all();
+        cp_async_wait_all();
         __syncthreads();
         MS_PH(12);
         // ---- applyDelta(K nu) (:263 -> :659-666): L2 = chol(P_new), X = mu [+] (delta +- L2 e_j).  A factorisation without
@@ -1008,7 +1008,7 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_ekf_update_kernel(slb::FilterAr
         const double *zg = a.z + (size_t)inst * M;
         __syncthreads();
         if (fetched) {
-            pred_cp_async_wait_all();
+            cp_async_wait_all();
             __syncthreads();
             for (int e = tid; e < NP; e += MS_T) RA[e] = RQ[e];
         } else {
@@ -1198,7 +1198,7 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_ekf_update_kernel(slb::FilterAr
             if (a.gate && inst + (int)gridDim.x < a.B) {
                 // T is consumed: RQ is idle for the rest of this instance and receives the next instance's covariance record
                 const double *Pn = a.P + (size_t)(inst + gridDim.x) * a.pstride;
-                for (int e = tid; e < NP; e += MS_T) pred_cp_async8(RQ + e, Pn + e);
+                for (int e = tid; e < NP; e += MS_T) cp_async8(RQ + e, Pn + e);
                 fetched = true;
             }
             if (compact || !a.gate) {

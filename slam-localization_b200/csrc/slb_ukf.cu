@@ -23,16 +23,14 @@
 //   * predict+update fused in one launch moves each instance through HBM exactly once.
 #include "slb_internal.h"
 #include "slb_models.cuh"
-#include "slb_predict12.cuh"   // TMA bulk copy / mbarrier helpers
+#include "slb_ptx.cuh"
 
 namespace slbd {
-
-constexpr unsigned UKF_FULL = 0xffffffffu;
 
 template <int G>
 SLB_DEV double gsum(double v) {
 #pragma unroll
-    for (int o = G / 2; o > 0; o >>= 1) v += __shfl_xor_sync(UKF_FULL, v, o);
+    for (int o = G / 2; o > 0; o >>= 1) v += __shfl_xor_sync(FULL, v, o);
     return v;
 }
 
@@ -83,7 +81,7 @@ struct Rec {
     static constexpr int ZO = 0, DZO = NS * M, KO = DZO + N * M, KSO = KO + N * M, DLO = KSO + N * M;
 };
 
-// doubles of shared memory per warp: 32/G records, the packed Q, and (16-byte aligned) an mbarrier slot
+// doubles of shared memory per warp: 32/G records, the packed Q, and (16-byte aligned) a barrier slot (mbar_init)
 template <class L, int M, int G>
 struct UkfWarp {
     static constexpr int DOUBLES = ((32 / G) * Rec<L, M, G>::IS + L::NP + 1) / 2 * 2 + 2;
@@ -125,7 +123,7 @@ SLB_DEV bool group_mean(const double *sig, int sub, bool go, double *ref) {
 #pragma unroll
     for (int c = 0; c < QD; ++c) ref[c] = sig[c * NS];
     int it = 0;
-    while (__any_sync(UKF_FULL, go)) {
+    while (__any_sync(FULL, go)) {
         double md[N];
 #pragma unroll
         for (int r = 0; r < N; ++r) md[r] = 0.0;
@@ -227,7 +225,7 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
     typedef Rec<L, MM::M, G> R;
     constexpr int N = L::N, QD = L::QD, NP = L::NP, NS = 2 * N + 1, M = MM::M, MP = M * (M + 1) / 2;
     constexpr int IPW = 32 / G, WPB = TPB / 32, ROUNDS = (NS + G - 1) / G, RROWS = (N + G - 1) / G;
-    constexpr int WSZ = UkfWarp<L, MM::M, G>::DOUBLES;  // per-warp shared memory: IPW records + packed Q + mbarrier
+    constexpr int WSZ = UkfWarp<L, MM::M, G>::DOUBLES;  // per-warp shared memory: IPW records + packed Q + barrier
     static_assert(M == 3, "only 3-dof measurement models are wired to the UKF kernel");
     extern __shared__ double sm[];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -256,7 +254,7 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
             double *d = dst + (e < QD ? R::MU + e : R::PS + (e - QD));
             if (lv) {
                 const double *src = e < QD ? a.mu + (size_t)e * a.stride + wbase + li : a.P + (size_t)(e - QD) * a.stride + wbase + li;
-                asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"((unsigned)__cvta_generic_to_shared(d)), "l"(src) : "memory");
+                cp_async8(d, src);
             } else {
                 *d = 0.0;
             }
@@ -284,7 +282,7 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
                     const bool need = c < NU ? PRED : UPD;
                     if (need && wbase + li2 < a.B) {
                         const double *src = c < NU ? a.u + (size_t)(wbase + li2) * NU + c : a.z + (size_t)(wbase + li2) * M + (c - NU);
-                        asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"((unsigned)__cvta_generic_to_shared(d)), "l"(src) : "memory");
+                        cp_async8(d, src);
                     } else {
                         *d = 0.0;
                     }
@@ -298,7 +296,7 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
                 Qp[e] = __ldg(a.Q + r * N + (e - tri(r, 0)));
             }
         }
-        asm volatile("cp.async.commit_group;\n cp.async.wait_group 0;\n" ::: "memory");
+        cp_async_wait_all();
     }
     __syncwarp();
     if (wbase + IPW <= a.B) mbar_wait(ubar, 0);

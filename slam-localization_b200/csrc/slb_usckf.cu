@@ -7,10 +7,11 @@
 // A record is contiguous, so a warp streams it with one TMA bulk copy (cp.async.bulk -> UBLKCP).
 //
 // predict (Usckf.hpp:113-244) touches only statek_i: rows 24..35, i.e. tile rows 3 and 4 (rows 24..39, one
-//   contiguous span of 520 doubles at N >= 40), and the 12-wide segments of the feature rows below.  Lane s evaluates sigma
-//   point s (25 of 32 lanes); Fk = Pxy^T Pii^-1 is obtained as W^T L^-1 with W = 0.5 (dY+ - dY-) by a
-//   triangular solve, because X_i [-] mu_old is +-L e_j by construction (same algebra as :152-154,
-//   without the explicit inverse).
+//   contiguous span of 520 doubles at N >= 40), and the 12-wide segments of the feature rows below.  Called alone it is
+//   predict12_kernel (slb_predict12.cuh), which fetches just those rows and runs predict12_block on them, the body the
+//   fused step runs on its resident record.  Lane s evaluates sigma point s (25 of 32 lanes); Fk = Pxy^T Pii^-1 is
+//   obtained as W^T L^-1 with W = 0.5 (dY+ - dY-) by a triangular solve, because X_i [-] mu_old is +-L e_j by
+//   construction (same algebra as :152-154, without the explicit inverse).
 // update (Usckf.hpp:260-308) and the fused predict+update step: slb_usckf_step.cuh (record resident in shared
 //   memory, blocked square-root-free factorisation on DMMA accumulator tiles, sigma points streamed per 16 columns).
 #include <cstdlib>

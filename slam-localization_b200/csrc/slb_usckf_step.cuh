@@ -23,7 +23,7 @@
 //   exp/log round trip, quirk Q10), one DMMA per panel and tile row into covXZ accumulator tiles.
 //   K = covXZ S^-1 (:286-288), K S K^T = covXZ K^T; Pk -= covXZ K^T is again one DMMA per tile, on the record in
 //   shared memory.
-// predict: slb_predict12.cuh's scheme on rows 24..35 of the resident record.
+// predict: slb_predict12.cuh's predict12_block on rows 24..35 of the resident record.
 #pragma once
 #include "slb_predict12.cuh"
 
@@ -72,29 +72,17 @@ struct StepCfg {
     static constexpr int WS = 20;
     static constexpr int WGS = WS * NK_;
     static constexpr int UPD_SCR = SCR0 + WGS + NPAD;       // + d_k
-    static constexpr int PRED_SCR = PRED_LS + 28 * PRED_DS + 144 + 12 * PRED_DS + 16 + 16;   // ... + rsd + reduction slots
     static constexpr int SCR = (UPD_SCR > PRED_SCR ? UPD_SCR : PRED_SCR);
     static constexpr int ZS = (NK_ + 1) / 2 * 2;
-    static constexpr int SM = PSTR + QS + SCR + ZS + 2;    // doubles per warp (even); last slot = mbarrier
+    static constexpr int SM = PSTR + QS + SCR + ZS + 2;    // doubles per warp (even); last slot = barrier
     // per-instance noise (the PIN instantiation): the lower triangle of this instance's R, packed, between z and the
-    // mbarrier.  (Its Q entries travel in registers: 6 per lane, see load_q_entries.)
+    // barrier.  (Its Q entries travel in registers: 6 per lane, see load_q_entries.)
     static constexpr int RP = (NK_ * (NK_ + 1) / 2 + 1) / 2 * 2;
     static constexpr int SMP = SM + RP;
     static_assert(NK_ % 3 == 0 && NK_ >= 3, "the VO model moves 3-D features");
     static_assert(N <= 64, "two rows per lane");
     static_assert(SM % 2 == 0 && PSTR % 2 == 0 && QS % 2 == 0, "16-byte alignment of the bulk copies");
 };
-
-SLB_DEV void bulk_s2g(void *gdst, const void *ssrc, unsigned bytes) {
-    asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;\n cp.async.bulk.commit_group;\n" ::"l"(gdst),
-                 "r"(saddr(ssrc)), "r"(bytes)
-                 : "memory");
-}
-SLB_DEV void bulk_prefetch_l2(const void *gsrc, unsigned bytes) {
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;\n" ::"l"(gsrc), "r"(bytes) : "memory");
-}
-SLB_DEV void bulk_store_wait() { asm volatile("cp.async.bulk.wait_group.read 0;\n" ::: "memory"); }
-SLB_DEV void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory"); }
 
 // symmetric inverse of the M x M innovation covariance (packed lower in, packed lower out) through its LDL^T
 // factorisation, redundantly on every lane; false if a pivot is not positive
@@ -155,48 +143,6 @@ SLB_DEV void vo_model(const double *pk, const double *qk, const double *pi, cons
         z[c] = rz[0] + (pk[0] - pi[0]);
         z[c + 1] = rz[1] + (pk[1] - pi[1]);
         z[c + 2] = rz[2] + (pk[2] - pi[2]);
-    }
-}
-
-// Sums of 12 values over the 32 lanes, result on every lane.  A butterfly per value costs 5 shuffles each (120 SHFL.32 for
-// 12 doubles, and shuffles travel through the same data pipe as shared memory, the kernel's limiter); here the lanes halve
-// the VALUE set while they halve the lane set (8 + 4 + 2 + 1 + 1 exchanges), the 16 partial owners park their sums in
-// shared memory and everybody reads them back with broadcast loads: 32 SHFL.32 + 1 STS + 6 LDS.128.  Fixed order: bitwise
-// reproducible.
-SLB_DEV void warp_sum12(const double *v, double *out, double *slots, int lane) {
-    double a[8], b[4], c[2], d1;
-    const bool h16 = lane & 16, h8 = lane & 8, h4 = lane & 4, h2 = lane & 2;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) {   // values 12..15 are zero padding
-        const double lo = v[i], hi = i < 4 ? v[8 + i] : 0.0;
-        const double r = __shfl_xor_sync(FULL, h16 ? lo : hi, 16);
-        a[i] = (h16 ? hi : lo) + r;                     // lanes < 16 own values 0..7, lanes >= 16 own 8..15
-    }
-#pragma unroll
-    for (int i = 0; i < 4; ++i) {
-        const double r = __shfl_xor_sync(FULL, h8 ? a[i] : a[4 + i], 8);
-        b[i] = (h8 ? a[4 + i] : a[i]) + r;
-    }
-#pragma unroll
-    for (int i = 0; i < 2; ++i) {
-        const double r = __shfl_xor_sync(FULL, h4 ? b[i] : b[2 + i], 4);
-        c[i] = (h4 ? b[2 + i] : b[i]) + r;
-    }
-    {
-        const double r = __shfl_xor_sync(FULL, h2 ? c[0] : c[1], 2);
-        d1 = (h2 ? c[1] : c[0]) + r;
-    }
-    d1 += __shfl_xor_sync(FULL, d1, 1);
-    // value index owned by this lane: bit 3 = h16, bit 2 = h8, bit 1 = h4, bit 0 = h2
-    const int idx = (h16 ? 8 : 0) + (h8 ? 4 : 0) + (h4 ? 2 : 0) + (h2 ? 1 : 0);
-    __syncwarp();
-    if (!(lane & 1)) slots[idx] = d1;
-    __syncwarp();
-#pragma unroll
-    for (int i = 0; i < 6; ++i) {
-        const double2 t = *reinterpret_cast<const double2 *>(slots + 2 * i);
-        out[2 * i] = t.x;
-        out[2 * i + 1] = t.y;
     }
 }
 
@@ -453,7 +399,7 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
     constexpr double NS = (double)(2 * N + 1);
     double ebar[NK], S[NK * (NK + 1) / 2];
     if (PIN) {   // the staged R (and z) must have landed, and be visible to the whole warp
-        asm volatile("cp.async.wait_group 0;\n" ::: "memory");
+        cp_async_wait0();
         __syncwarp();
     }
     auto Rv = [&](int r, int c) { return PIN ? Rs[tri(r, c)] : __ldg(a.R + r * NK + c); };
@@ -485,7 +431,7 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
     double Si[NK * (NK + 1) / 2];
     const bool sok = sym_inverse<NK>(S, Si);
     auto SiAt = [&](int r, int c) { return r >= c ? Si[tri(r, c)] : Si[tri(c, r)]; };
-    asm volatile("cp.async.wait_group 0;\n" ::: "memory");
+    cp_async_wait0();
     __syncwarp();   // z has landed; every lane is done reading Lf / Wg: K | covXZ overlay them
     double nu[NK], sn[NK], m2 = 0.0;
 #pragma unroll
@@ -592,195 +538,15 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
     return __all_sync(FULL, finite) ? 0 : SLB_ST_NONFINITE;
 }
 
-// predict of the resident record (statek_i: rows 24..35, mean at q-offset 26); see predict12_kernel for the scheme.
-// Returns status bits; `dirty` is set when Ps / mus changed.
-// PIN: Q comes from `qv`, the 6 entries this lane adds (load_q_entries), instead of the shared matrix at Qg.
-template <int PM, int NF, bool PIN = false>
-SLB_DEV int usckf_predict_smem(double *Ps, double *mus, double *scr, const double *u, double dt, const double *Qg,
-                               const double *qv, int lane, bool &dirty) {
-    typedef LayState12 L;
-    typedef CycCfg<12> C;
-    constexpr int ROW0 = 24, MU0 = 26, N = 36 + NF;
-    double *Ls = scr, *D = Ls + PRED_LS, *W = D + 28 * PRED_DS, *Fk = W + 144, *rsd = Fk + 12 * PRED_DS, *slots = rsd + 16;
-    auto PR = [&](int r, int c) -> double & { return Ps[prec(N, ROW0 + r, c)]; };        // row 24 + r, col c
-    auto PF = [&](int fr, int c) -> double & { return Ps[prec(N, 36 + fr, 24 + c)]; };   // feature row fr, col 24 + c
-    const int a_ = lane & 3, b_ = lane >> 2;
-    double mu[13];
-#pragma unroll
-    for (int c = 0; c < 13; ++c) mu[c] = mus[MU0 + c];
-    ProcessModel<PM> f;
-    f.prepare(u, dt);
-    // ---- Pk_i = U D^-1 U^T (Eigen::LLT of :572-577 up to the per-column scale 1/sqrt(d_k)) ---------------------
-    double T[C::RT][C::CT];
-#pragma unroll
-    for (int r = 0; r < C::RT; ++r)
-#pragma unroll
-        for (int c = 0; c < C::CT; ++c)
-            if (C::exists(r, c)) {
-                const int i = a_ + 4 * r, j = b_ + 8 * c;
-                T[r][c] = (i < 12 && j <= i) ? PR(i, ROW0 + j) : 0.0;
-            }
-    bool ok = true;
-    {
-        const double x0 = __shfl_sync(FULL, T[0][0], 0);
-        CholStep<C, 0>::run(T, Ls, a_, b_, ok, x0, -rcp_fast(x0));
-    }
-    if (!ok) return SLB_ST_CHOL_FAIL;
-    __syncwarp();
-    if (lane < 12) {
-        double sq_, rs_;
-        sqrt_rsqrt(Ls[C::cb(lane)], sq_, rs_);
-        rsd[lane] = rs_;  // 1 / L_kk
-    }
-    __syncwarp();
-    // ---- sigma point `lane` (Usckf.hpp:572-598), process model (:141) ---------------------------------
-    const bool act = lane < 25;
-    const int j = lane >= 1 ? (lane - 1) >> 1 : 0, jc = j < 12 ? j : 11;
-    double Y[13];
-    {
-        const double sgn = (lane & 1) ? rsd[jc] : -rsd[jc];
-        const int cj = C::cb(jc) - jc;
-        double d[12], X[13];
-#pragma unroll
-        for (int r = 0; r < 12; ++r) d[r] = (act && lane >= 1 && r >= jc) ? sgn * Ls[cj + r] : 0.0;
-        boxplus<L>(mu, d, 1.0, X);
-        f.apply(X, Y);
-    }
-    // ---- manifold mean (:601-627) --------------------------------------------------------------------
-    double ref[13];
-#pragma unroll
-    for (int c = 0; c < 13; ++c) ref[c] = bcast(Y[c], 0);
-    int it = 0;
-    double nrm2;
-    do {
-        double dd[12], md[12], nr[13];
-        boxminus<L>(Y, ref, dd);
-#pragma unroll
-        for (int r = 0; r < 12; ++r) dd[r] = act ? dd[r] : 0.0;
-        warp_sum12(dd, md, slots, lane);
-        nrm2 = 0.0;
-#pragma unroll
-        for (int r = 0; r < 12; ++r) {
-            md[r] *= (1.0 / 25.0);
-            nrm2 += md[r] * md[r];
-        }
-        boxplus<L>(ref, md, 1.0, nr);
-#pragma unroll
-        for (int c = 0; c < 13; ++c) ref[c] = nr[c];
-    } while (sqrt(nrm2) > 1e-6 && ++it < 10000);
-    int st = (it >= 10000) ? SLB_ST_MEAN_NOCONV : 0;
-    {   // deviations, one row per sigma point; rows 25..27 are the zero padding of the DMMA k-dimension
-        double dY[12];
-        boxminus<L>(Y, ref, dY);
-        if (lane < 28) {
-#pragma unroll
-            for (int r = 0; r < 12; r += 2)   // (row stride 160 B: 16-byte stores, 2-way instead of 8-way bank conflicts)
-                *reinterpret_cast<double2 *>(D + lane * PRED_DS + r) = act ? make_double2(dY[r], dY[r + 1]) : make_double2(0.0, 0.0);
-        }
-    }
-    __syncwarp();
-    dirty = true;
-    // ---- Pk_i = 0.5 D^T D + Q (:178): three lower 8x8 tiles, k = 28 ---------------------------------------------
-    {
-        double c00[2] = {0.0, 0.0}, c10[2] = {0.0, 0.0}, c11[2] = {0.0, 0.0};
-        const double *p0 = D + a_ * PRED_DS + b_, *p1 = p0 + 8;  // A[m][k] = D[k][m]: lane (row b_, k a_)
-#pragma unroll
-        for (int k0 = 0; k0 < 28; k0 += 4) {
-            const double f0 = p0[k0 * PRED_DS], f1 = p1[k0 * PRED_DS];  // columns 12..15 of D only feed dropped outputs
-            dmma884(c00[0], c00[1], f0, f0);
-            dmma884(c10[0], c10[1], f1, f0);
-            dmma884(c11[0], c11[1], f1, f1);
-        }
-        for (int e = lane; e < 144; e += 32) {
-            const int jj = e / 12, c = e - jj * 12;
-            W[e] = 0.5 * (D[(1 + 2 * jj) * PRED_DS + c] - D[(2 + 2 * jj) * PRED_DS + c]);
-        }
-        __syncwarp();   // the old block (rows 24..35, cols 24..35) was consumed by the factorisation: overwrite it
-        auto put = [&](int r, int c, double v, int k) {
-            if (r < 12 && c <= r) PR(r, ROW0 + c) = 0.5 * v + (PIN ? qv[k] : __ldg(Qg + r * 12 + c));
-        };
-        const int r = b_, c = 2 * a_;
-        put(r, c, c00[0], 0); put(r, c + 1, c00[1], 1);
-        put(8 + r, c, c10[0], 2); put(8 + r, c + 1, c10[1], 3);
-        put(8 + r, 8 + c, c11[0], 4); put(8 + r, 8 + c + 1, c11[1], 5);
-    }
-    // ---- Fk = W^T L^-1  <=>  L^T Fk^T = W: lane c back-substitutes column c (:154); L(p,r) = U(p,r) / sqrt(d_r) --
-    if (lane < 12) {
-        double x[12];
-#pragma unroll
-        for (int r = 11; r >= 0; --r) {
-            double sacc = 0.0;
-#pragma unroll
-            for (int p = r + 1; p < 12; ++p) sacc = fma(Ls[C::cb(r) - r + p], x[p], sacc);
-            const double rs = rsd[r];
-            x[r] = (W[r * 12 + lane] - rs * sacc) * rs;
-        }
-#pragma unroll
-        for (int r = 0; r < 12; ++r) Fk[lane * PRED_DS + r] = x[r];
-    }
-    __syncwarp();
-    // ---- cross-covariances with the clones (:191-208): rows 24..35 x cols 0..23  <- Fk * old: 2 x 3 tiles, k = 12 ----
-    double oc[2][3][2];
-    {
-        const int r0 = min(b_, 11), r1 = min(8 + b_, 11);
-#pragma unroll
-        for (int I = 0; I < 2; ++I)
-#pragma unroll
-            for (int J = 0; J < 3; ++J) oc[I][J][0] = oc[I][J][1] = 0.0;
-#pragma unroll
-        for (int k0 = 0; k0 < 12; k0 += 4) {
-            const double fa0 = Fk[r0 * PRED_DS + k0 + a_], fa1 = Fk[r1 * PRED_DS + k0 + a_];
-#pragma unroll
-            for (int J = 0; J < 3; ++J) {
-                const double bv = PR(k0 + a_, 8 * J + b_);  // B[k][n] = old P(24 + k, n)
-                dmma884(oc[0][J][0], oc[0][J][1], fa0, bv);
-                dmma884(oc[1][J][0], oc[1][J][1], fa1, bv);
-            }
-        }
-    }
-    // ---- and with the features (:217-235): feature rows x cols 24..35  <- old * Fk^T: ceil(nf/8) x 2 tiles, k = 12 ----
-    constexpr int NFT = (NF + 7) / 8;
-    double of[NFT > 0 ? NFT : 1][2][2];
-    {
-        const int c0 = min(b_, 11), c1 = min(8 + b_, 11);
-#pragma unroll
-        for (int I = 0; I < NFT; ++I) {
-            of[I][0][0] = of[I][0][1] = of[I][1][0] = of[I][1][1] = 0.0;
-            const int fr = min(8 * I + b_, NF - 1);
-#pragma unroll
-            for (int k0 = 0; k0 < 12; k0 += 4) {
-                const double av = PF(fr, k0 + a_);
-                dmma884(of[I][0][0], of[I][0][1], av, Fk[c0 * PRED_DS + k0 + a_]);  // B[k][n] = Fk[n][k]
-                dmma884(of[I][1][0], of[I][1][1], av, Fk[c1 * PRED_DS + k0 + a_]);
-            }
-        }
-    }
-    __syncwarp();
-    // rows 24..35 x cols 0..23 are off-diagonal tiles of tile rows 3 and 4: one 16-byte store per lane and tile
-#pragma unroll
-    for (int I = 0; I < 2; ++I)
-#pragma unroll
-        for (int J = 0; J < 3; ++J)
-            if (8 * I + b_ < 12)
-                *reinterpret_cast<double2 *>(Ps + prec(N, ROW0 + 8 * I, 8 * J) + 2 * lane) = make_double2(oc[I][J][0], oc[I][J][1]);
-#pragma unroll
-    for (int I = 0; I < NFT; ++I) {
-#pragma unroll
-        for (int J = 0; J < 2; ++J) {
-            const int fr = 8 * I + b_, c = 8 * J + 2 * a_;
-            if (fr < NF && c < 12) { PF(fr, c) = of[I][J][0]; PF(fr, c + 1) = of[I][J][1]; }
-        }
-    }
-    bool finite = true;
-#pragma unroll
-    for (int c = 0; c < 13; ++c) {
-        finite = finite && isfinite(ref[c]);
-        if (lane == c) mus[MU0 + c] = ref[c];
-    }
-    if (!finite) st |= SLB_ST_NONFINITE;
-    __syncwarp();
-    return st;
-}
+// predict12_block's view of the resident tiled record (rows 24..35 and feature rows 36..)
+template <int N>
+struct ResidentView {
+    static constexpr int ROW0 = 24;
+    double *P;
+    SLB_DEV int idx(int r, int c) const { return prec(N, 24 + r, c); }
+    SLB_DEV double &at(int r, int c) const { return P[idx(r, c)]; }
+    SLB_DEV double &feat(int fr, int c) const { return P[prec(N, 36 + fr, 24 + c)]; }
+};
 
 // One instance per warp: record in (TMA bulk load), predict and / or update in shared memory, record out (TMA bulk
 // store).  PRED && UPD is the fused step (slb_usckf_step, the *_step_host paths); UPD alone is slb_usckf_update.
@@ -811,19 +577,17 @@ __global__ void __launch_bounds__(WPB * 32, MINB) usckf_step_kernel(slb::FilterA
     // the measurement and the control input are fetched now: with the zero-copy *_step_host they live in mapped host
     // memory and their PCIe latency must not sit in the middle of the step
     if (UPD && lane < NK) {
-        asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n cp.async.commit_group;\n" ::"r"(saddr(zs + lane)),
-                     "l"(a.z + (size_t)inst * NK + lane)
-                     : "memory");
+        cp_async8(zs + lane, a.z + (size_t)inst * NK + lane);
+        cp_async_commit();
     }
     if (PIN && UPD) {   // lower triangle of this instance's R, packed (Rs[tri(r, c)])
         const double *Ri = a.R + (size_t)inst * a.rs;
         for (int e = lane; e < NK * (NK + 1) / 2; e += 32) {
             int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
             r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
-            asm volatile("cp.async.ca.shared.global [%0], [%1], 8;\n" ::"r"(saddr(Rs + e)), "l"(Ri + r * NK + (e - tri(r, 0)))
-                         : "memory");
+            cp_async8(Rs + e, Ri + r * NK + (e - tri(r, 0)));
         }
-        asm volatile("cp.async.commit_group;\n" ::: "memory");
+        cp_async_commit();
     }
     double qv[PIN && PRED ? 6 : 1];
     if (PIN && PRED) load_q_entries(a.Q + (size_t)inst * a.qs, lane & 3, lane >> 2, qv);
@@ -837,10 +601,12 @@ __global__ void __launch_bounds__(WPB * 32, MINB) usckf_step_kernel(slb::FilterA
     SLB_CTA_SYNC();
     int st = 0;
     bool dirty = false;
-    if (PRED) st |= usckf_predict_smem<PM, NK + NL, PIN>(Ps, mus, scr, u, a.dt, a.Q, qv, lane, dirty);
+    if (PRED) {
+        st = predict12_block<PM, true, PIN>(ResidentView<C::N>{Ps}, mus + 26, u, a.dt, scr, a.Q, qv, NK + NL, mus + 26, lane, dirty);
+    }
     if (PRED) SLB_CTA_SYNC();
     if (UPD) st |= usckf_update_smem<NK, NL, PIN>(Ps, mus, scr, zs, Rs, a, lane, dirty);
-    asm volatile("cp.async.wait_group 0;\n" ::: "memory");   // (an update that bailed out early has not waited for z)
+    cp_async_wait0();   // (an update that bailed out early has not waited for z)
     // ---- record out ----------------------------------------------------------------------------------------------
     if (dirty) {
         fence_proxy_async();
