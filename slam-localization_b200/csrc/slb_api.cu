@@ -26,80 +26,69 @@ int set_error(int code, const char *what, cudaError_t ce) {
 }
 void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
 
-// ---- layout conversion kernels ---------------------------------------------------------------------
-// UKF kind: instance-major host layout <-> SoA
-__global__ void aos_to_soa_mu(const double *aos, double *soa, int B0, int cnt, int QD, int stride) {
+// ---- layout conversion kernels: dense instance-major host arrays <-> the batch (h->L) ---------------------------
+// Means: thread t = (instance, scalar), scalar fastest.  mu_in stores instances [b0, b0 + cnt); mu_out loads the slice
+// [off, off + len) of their q-vectors.
+__global__ void mu_in(const double *src, double *mu, slbd::BatchLayout L, int b0, int cnt) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= cnt * QD) return;
-    const int i = t / QD, c = t - i * QD;
-    soa[(size_t)c * stride + B0 + i] = aos[t];
+    if (t >= cnt * L.QD) return;
+    const int i = t / L.QD, c = t - i * L.QD;
+    mu[L.mu(b0 + i, c)] = src[t];
 }
-__global__ void soa_to_aos_mu(const double *soa, double *aos, int B0, int cnt, int QD, int stride, int off = 0) {
+__global__ void mu_out(const double *mu, double *dst, slbd::BatchLayout L, int b0, int cnt, int off, int len) {
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= cnt * QD) return;
-    const int i = t / QD, c = t - i * QD;
-    aos[t] = soa[(size_t)(off + c) * stride + B0 + i];
+    if (t >= cnt * len) return;
+    const int i = t / len, c = t - i * len;
+    dst[t] = mu[L.mu(b0 + i, off + c)];
 }
-__global__ void dense_to_soa_P(const double *dense, double *soa, int B0, int cnt, int N, int stride) {
-    const int NP = N * (N + 1) / 2;
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= (int64_t)cnt * NP) return;
-    const int e = (int)(t / cnt), i = (int)(t - (int64_t)e * cnt);  // instance fastest: coalesced stores
-    int r = (int)((sqrt(8.0 * e + 1.0) - 1.0) * 0.5);
+// thread t of a launch over `per` entries of each of `cnt` instances -> (instance i, entry k): the instance fastest
+// for SoA, the entry fastest for records, so that consecutive threads store to consecutive doubles of the batch
+SLB_DEV void split(const slbd::BatchLayout &L, int64_t t, int cnt, int per, int &i, int &k) {
+    if (L.soa) { k = (int)(t / cnt); i = (int)(t - (int64_t)k * cnt); }
+    else { i = (int)(t / per); k = (int)(t - (int64_t)i * per); }
+}
+// (r, c), r >= c, of packed lower-triangle entry e
+SLB_DEV void tri_rc(int e, int &r, int &c) {
+    r = (int)((sqrt(8.0 * e + 1.0) - 1.0) * 0.5);
     while (r * (r + 1) / 2 > e) --r;
     while ((r + 1) * (r + 2) / 2 <= e) ++r;
-    const int c = e - r * (r + 1) / 2;
-    soa[(size_t)e * stride + B0 + i] = dense[(size_t)i * N * N + r * N + c];
+    c = e - r * (r + 1) / 2;
 }
-__global__ void soa_to_dense_P(const double *soa, double *dense, int B0, int cnt, int N, int stride) {
+// Covariances: the lower triangle of dense src goes to the batch; P_out writes both triangles of dense dst.
+__global__ void P_in(const double *src, double *P, slbd::BatchLayout L, int b0, int cnt) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (int64_t)cnt * L.NP) return;
+    int i, e, r, c;
+    split(L, t, cnt, L.NP, i, e);
+    tri_rc(e, r, c);
+    P[L.P(b0 + i, r, c)] = src[((size_t)i * L.N + r) * L.N + c];
+}
+__global__ void P_out(const double *P, double *dst, slbd::BatchLayout L, int b0, int cnt) {
+    const int N = L.N;
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= (int64_t)cnt * N * N) return;
     const int i = (int)(t / (N * N)), rc = (int)(t - (int64_t)i * N * N);
     int r = rc / N, c = rc - r * N;
     if (c > r) { const int x = r; r = c; c = x; }
-    dense[t] = soa[(size_t)(r * (r + 1) / 2 + c) * stride + B0 + i];
-}
-// USCKF / MSCKF kinds: instance-major records; P is packed lower (MSCKF, tri) or tiled (USCKF, prec)
-__global__ void aos_to_rec_mu(const double *aos, double *rec, int B0, int cnt, int QD, int qstride) {
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= cnt * QD) return;
-    const int i = t / QD, c = t - i * QD;
-    rec[(size_t)(B0 + i) * qstride + c] = aos[t];
-}
-__global__ void rec_to_aos_mu(const double *rec, double *aos, int B0, int cnt, int QD, int qstride, int off = 0) {
-    const int t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= cnt * QD) return;
-    const int i = t / QD, c = t - i * QD;
-    aos[t] = rec[(size_t)(B0 + i) * qstride + off + c];
-}
-__global__ void dense_to_rec_P(const double *dense, double *rec, int B0, int cnt, int N, int pstride, bool tiled) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= (int64_t)cnt * N * N) return;
-    const int i = (int)(t / (N * N)), rc = (int)(t - (int64_t)i * N * N);
-    const int r = rc / N, c = rc - r * N;
-    if (c <= r) rec[(size_t)(B0 + i) * pstride + (tiled ? slbd::prec(N, r, c) : slbd::tri(r, c))] = dense[t];
-}
-__global__ void rec_to_dense_P(const double *rec, double *dense, int B0, int cnt, int N, int pstride, bool tiled) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= (int64_t)cnt * N * N) return;
-    const int i = (int)(t / (N * N)), rc = (int)(t - (int64_t)i * N * N);
-    int r = rc / N, c = rc - r * N;
-    if (c > r) { const int x = r; r = c; c = x; }
-    dense[t] = rec[(size_t)(B0 + i) * pstride + (tiled ? slbd::prec(N, r, c) : slbd::tri(r, c))];
+    dst[t] = P[L.P(b0 + i, r, c)];
 }
 
-// fleet initialisation: instance i <- instance i % count (Monte-Carlo replicas of `count` priors)
-__global__ void replicate_soa(double *a, int rows, int stride, int B, int count) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= (int64_t)rows * B) return;
-    const int r = (int)(t / B), i = (int)(t - (int64_t)r * B);
-    if (i >= count) a[(size_t)r * stride + i] = a[(size_t)r * stride + i % count];
-}
-__global__ void replicate_rec(double *a, int per, int B, int count) {
+// fleet initialisation: instance i <- instance i % count (Monte-Carlo replicas of `count` priors), the means (a = mu)
+// or the covariances (cov, a = P)
+__global__ void replicate(double *a, slbd::BatchLayout L, int B, int count, bool cov) {
+    const int per = cov ? L.NP : L.QD;
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t >= (int64_t)per * B) return;
-    const int i = (int)(t / per), e = (int)(t - (int64_t)i * per);
-    if (i >= count) a[(size_t)i * per + e] = a[(size_t)(i % count) * per + e];
+    int i, k;
+    split(L, t, B, per, i, k);
+    if (i < count) return;
+    if (cov) {
+        int r, c;
+        tri_rc(k, r, c);
+        a[L.P(i, r, c)] = a[L.P(i % count, r, c)];
+    } else {
+        a[L.mu(i, k)] = a[L.mu(i % count, k)];
+    }
 }
 
 __global__ void status_count(const int32_t *st, int B, unsigned long long *counts) {
@@ -120,17 +109,10 @@ __global__ void status_count(const int32_t *st, int B, unsigned long long *count
 
 // Ensemble statistics: out = {count, sum x, sum x x^T}, x = vectorised mean (log of SO3 blocks).
 // Persistent CTAs, chunks of 64 instances staged in shared memory, register accumulators.
-struct StatLayout {
-    int nblk;
-    unsigned long long so3mask;
-    int nfeat, N, QD;
-    int soa;          // 1: mu is SoA with `stride`; 0: records with `qstride`
-    int stride, qstride;
-};
 constexpr int STAT_CHUNK = 64, STAT_TPB = 256, STAT_MAXACC = 24;
-__global__ void __launch_bounds__(STAT_TPB) ensemble_stats_kernel(const double *mu, int B, StatLayout l, double *out) {
+__global__ void __launch_bounds__(STAT_TPB) ensemble_stats_kernel(const double *mu, int B, slbd::BatchLayout L, double *out) {
     extern __shared__ double xs[];  // [STAT_CHUNK][N]
-    const int N = l.N;
+    const int N = L.N;
     const int nent = N * N + N;
     double acc[STAT_MAXACC];
 #pragma unroll
@@ -144,20 +126,19 @@ __global__ void __launch_bounds__(STAT_TPB) ensemble_stats_kernel(const double *
             const int i = base + threadIdx.x;
             double *x = xs + threadIdx.x * N;
             int o = 0;
-            auto ld = [&](int c) { return l.soa ? mu[(size_t)c * l.stride + i] : mu[(size_t)i * l.qstride + c]; };
-            for (int b = 0; b < l.nblk; ++b) {
-                if ((l.so3mask >> b) & 1ull) {
-                    const double q[4] = {ld(o), ld(o + 1), ld(o + 2), ld(o + 3)};
+            for (int b = 0; b < L.nblk; ++b) {
+                if ((L.so3mask >> b) & 1ull) {
+                    const double q[4] = {mu[L.mu(i, o)], mu[L.mu(i, o + 1)], mu[L.mu(i, o + 2)], mu[L.mu(i, o + 3)]};
                     double v[3];
                     slbd::so3_log(q, v);
                     x[3 * b] = v[0]; x[3 * b + 1] = v[1]; x[3 * b + 2] = v[2];
                     o += 4;
                 } else {
-                    x[3 * b] = ld(o); x[3 * b + 1] = ld(o + 1); x[3 * b + 2] = ld(o + 2);
+                    x[3 * b] = mu[L.mu(i, o)]; x[3 * b + 1] = mu[L.mu(i, o + 1)]; x[3 * b + 2] = mu[L.mu(i, o + 2)];
                     o += 3;
                 }
             }
-            for (int f = 0; f < l.nfeat; ++f) x[3 * l.nblk + f] = ld(o + f);
+            for (int f = 0; f < L.nfeat; ++f) x[3 * L.nblk + f] = mu[L.mu(i, o + f)];
         }
         __syncthreads();
 #pragma unroll
@@ -205,7 +186,7 @@ static FilterArgs make_args(slb_handle h) {
     FilterArgs a;
     memset(&a, 0, sizeof(a));
     a.mu = h->mu; a.P = h->P; a.status = h->status; a.outliers = h->outliers;
-    a.B = h->B; a.stride = h->stride; a.pstride = h->pstride; a.qstride = h->qstride;
+    a.B = h->B; a.stride = h->L.stride; a.pstride = h->L.pstride; a.qstride = h->L.qstride;
     a.nk = h->cfg.nk; a.nl = h->cfg.nl; a.k = h->cfg.nclones;
     a.misc = h->misc_dev;
     a.out_off = h->out_off; a.out_len = h->out_len;
@@ -213,6 +194,54 @@ static FilterArgs make_args(slb_handle h) {
 }
 
 static int pm_nu(int pm) { return pm == SLB_PM_MSCKF_DELTAPOSE ? 13 : 6; }
+
+// The storage of a batch of B instances of a configuration slb_create accepted (DESIGN §3)
+static constexpr slbd::BatchLayout batch_layout(int kind, int layout, int nk, int nl, int nclones, int B) {
+    slbd::BatchLayout L{};
+    switch (kind) {
+        case SLB_KIND_UKF:  // pos, orient [, vel]
+            L.N = layout; L.QD = layout + 1;
+            L.nblk = layout / 3; L.so3mask = 0x2;
+            break;
+        case SLB_KIND_USCKF:  // statek | statek_l | statek_i (pos, orient, velo, angvelo each), featuresk | featuresk_l
+            L.N = 36 + nk + nl; L.QD = 39 + nk + nl;
+            L.nblk = 12; L.so3mask = 0x222; L.nfeat = nk + nl;
+            break;
+        default:  // MSCKF: pos, orient, velo, angvelo, then (pos, orient) per clone
+            L.N = 12 + 6 * nclones; L.QD = 13 + 7 * nclones;
+            L.nblk = 4 + 2 * nclones; L.so3mask = 0x2;
+            for (int j = 0; j < nclones; ++j) L.so3mask |= 1ull << (4 + 2 * j + 1);
+    }
+    L.NP = L.N * (L.N + 1) / 2;
+    L.soa = kind == SLB_KIND_UKF;
+    L.tiled = kind == SLB_KIND_USCKF;
+    L.stride = (B + 31) / 32 * 32;
+    L.pstride = (L.NP + 15) / 16 * 16;
+    L.qstride = (L.QD + 1) / 2 * 2;
+    return L;
+}
+// P(i, ., .) puts the NP entries of each instance on distinct doubles inside the P_size(B) of the batch, a record's in
+// its first NP: with B = 32 a SoA batch is filled without a gap, a record up to its padding
+static constexpr bool P_fills_storage(const slbd::BatchLayout &L, int B) {
+    bool seen[8192] = {};
+    if (L.P_size(B) > 8192) return false;
+    for (int i = 0; i < B; ++i)
+        for (int r = 0; r < L.N; ++r)
+            for (int c = 0; c <= r; ++c) {
+                const size_t o = L.P(i, r, c);
+                if (o >= L.P_size(B) || seen[o]) return false;
+                if (!L.soa && (o < (size_t)i * L.pstride || o >= (size_t)i * L.pstride + L.NP)) return false;
+                seen[o] = true;
+            }
+    return true;
+}
+static_assert(P_fills_storage(batch_layout(SLB_KIND_UKF, SLB_LAYOUT_POSE6, 0, 0, 0, 32), 32), "UKF POSE6 storage");
+static_assert(P_fills_storage(batch_layout(SLB_KIND_UKF, SLB_LAYOUT_MTK9, 0, 0, 0, 32), 32), "UKF MTK9 storage");
+static_assert(P_fills_storage(batch_layout(SLB_KIND_MSCKF, 0, 0, 0, 10, 2), 2), "MSCKF storage");
+#define SLB_USCKF_SHAPE(NK_, NL_) \
+    static_assert(P_fills_storage(batch_layout(SLB_KIND_USCKF, 0, NK_, NL_, 0, 2), 2), "USCKF storage");
+SLB_USCKF_SHAPES(SLB_USCKF_SHAPE)
+#undef SLB_USCKF_SHAPE
 
 }  // namespace slb
 
@@ -239,55 +268,37 @@ int slb_create(const slb_config *cfg, slb_handle *out) {
         int cur = -1;
         if (cudaGetDevice(&cur) != cudaSuccess || cur != cfg->device) return set_error(SLB_ERR_CUDA, "slb_create: cudaSetDevice failed");
     }
+    switch (cfg->kind) {
+        case SLB_KIND_UKF:
+            if (cfg->layout != SLB_LAYOUT_POSE6 && cfg->layout != SLB_LAYOUT_MTK9)
+                return set_error(SLB_ERR_INVALID, "slb_create: UKF layout must be POSE6 or MTK9");
+            break;
+        case SLB_KIND_USCKF:
+            if (!usckf_shape_supported(cfg->nk, cfg->nl))
+                return set_error(SLB_ERR_INVALID,
+                                 "slb_create: USCKF batches are built for nk in {3,6,9}, nl in {0,3,6,9} with nk + nl <= 12");
+            break;
+        case SLB_KIND_MSCKF:
+            if (cfg->nclones < 0 || cfg->nclones > 10) return set_error(SLB_ERR_INVALID, "slb_create: MSCKF supports 0..10 clones");
+            break;
+        default:
+            return set_error(SLB_ERR_INVALID, "slb_create: unknown kind");
+    }
     slb_batch_s *h = new (std::nothrow) slb_batch_s();
     if (!h) return set_error(SLB_ERR_ALLOC, "slb_create: host allocation failed");
     memset(h, 0, sizeof(*h));
     h->cfg = *cfg;
     h->B = cfg->batch;
-    switch (cfg->kind) {
-        case SLB_KIND_UKF:
-            if (cfg->layout != SLB_LAYOUT_POSE6 && cfg->layout != SLB_LAYOUT_MTK9) {
-                delete h;
-                return set_error(SLB_ERR_INVALID, "slb_create: UKF layout must be POSE6 or MTK9");
-            }
-            h->N = cfg->layout;
-            h->QD = cfg->layout + 1;
-            break;
-        case SLB_KIND_USCKF:
-            if (!usckf_shape_supported(cfg->nk, cfg->nl)) {
-                delete h;
-                return set_error(SLB_ERR_INVALID,
-                                 "slb_create: USCKF batches are built for nk in {3,6,9}, nl in {0,3,6,9} with nk + nl <= 12");
-            }
-            h->N = 36 + cfg->nk + cfg->nl;
-            h->QD = 39 + cfg->nk + cfg->nl;
-            break;
-        case SLB_KIND_MSCKF:
-            if (cfg->nclones < 0 || cfg->nclones > 10) {
-                delete h;
-                return set_error(SLB_ERR_INVALID, "slb_create: MSCKF supports 0..10 clones");
-            }
-            h->N = 12 + 6 * cfg->nclones;
-            h->QD = 13 + 7 * cfg->nclones;
-            break;
-        default:
-            delete h;
-            return set_error(SLB_ERR_INVALID, "slb_create: unknown kind");
-    }
-    h->NP = h->N * (h->N + 1) / 2;
+    h->L = batch_layout(cfg->kind, cfg->layout, cfg->nk, cfg->nl, cfg->nclones, cfg->batch);
+    const slbd::BatchLayout &L = h->L;
     h->out_off = 0;
-    h->out_len = h->QD;
-    h->stride = (h->B + 31) / 32 * 32;
-    h->pstride = (h->NP + 15) / 16 * 16;
-    h->qstride = (h->QD + 1) / 2 * 2;
-    const bool soa = cfg->kind == SLB_KIND_UKF;
-    const size_t mu_bytes = soa ? (size_t)h->QD * h->stride * 8 : (size_t)h->B * h->qstride * 8;
-    const size_t P_bytes = soa ? (size_t)h->NP * h->stride * 8 : (size_t)h->B * h->pstride * 8;
+    h->out_len = L.QD;
+    const size_t mu_bytes = L.mu_size(h->B) * 8, P_bytes = L.P_size(h->B) * 8;
     h->stage_bytes = (size_t)64 << 20;
-    const size_t one = (size_t)h->N * h->N * 8;
+    const size_t one = (size_t)L.N * L.N * 8;
     if (h->stage_bytes < one * 32) h->stage_bytes = one * 32;
     // the *_step_host entry points stage u | z | mu_out for the whole batch
-    const size_t io = (size_t)h->B * (h->QD + 16 + (cfg->kind == SLB_KIND_MSCKF ? 104 : 4)) * 8;
+    const size_t io = (size_t)h->B * (L.QD + 16 + (cfg->kind == SLB_KIND_MSCKF ? 104 : 4)) * 8;
     if (h->stage_bytes < io) h->stage_bytes = io;
     cudaError_t e = cudaSuccess;
     if (e == cudaSuccess) e = cudaMalloc(&h->mu, mu_bytes);
@@ -333,7 +344,7 @@ int slb_destroy(slb_handle h) {
 }
 
 int slb_set_output_slice(slb_handle h, int offset, int count) {
-    if (!h || offset < 0 || count < 1 || offset + count > h->QD)
+    if (!h || offset < 0 || count < 1 || offset + count > h->L.QD)
         return set_error(SLB_ERR_INVALID, "slb_set_output_slice: the slice must lie inside the q-vector");
     h->out_off = offset;
     h->out_len = count;
@@ -352,8 +363,8 @@ int slb_set_noise_layout(slb_handle h, int flags) {
 // doubles between consecutive instances' Q / R for a handle's noise layout (0 = shared)
 static int q_stride(slb_handle h, int n) { return (h->noise & SLB_NOISE_Q_PER_INSTANCE) ? n * n : 0; }
 static int r_stride(slb_handle h, int m) { return (h->noise & SLB_NOISE_R_PER_INSTANCE) ? m * m : 0; }
-int slb_dof(slb_handle h) { return h ? h->N : SLB_ERR_INVALID; }
-int slb_qdim(slb_handle h) { return h ? h->QD : SLB_ERR_INVALID; }
+int slb_dof(slb_handle h) { return h ? h->L.N : SLB_ERR_INVALID; }
+int slb_qdim(slb_handle h) { return h ? h->L.QD : SLB_ERR_INVALID; }
 
 int slb_device_ptr(slb_handle h, int field, void **dev) {
     if (!h || !dev) return set_error(SLB_ERR_INVALID, "slb_device_ptr: null argument");
@@ -369,7 +380,7 @@ int slb_device_ptr(slb_handle h, int field, void **dev) {
 static int transfer(slb_handle h, int field, void *host, size_t count, cudaStream_t s, bool up) {
     if (!h || !host) return set_error(SLB_ERR_INVALID, "slb_upload/download: null argument");
     DeviceGuard guard(h->cfg.device);
-    const bool soa = h->cfg.kind == SLB_KIND_UKF, tiled = h->cfg.kind == SLB_KIND_USCKF;
+    const slbd::BatchLayout &L = h->L;
     if (field == SLB_FIELD_STATUS || field == SLB_FIELD_OUTLIERS) {
         if (up) return set_error(SLB_ERR_INVALID, "slb_upload: status fields are read-only");
         if (count != (size_t)h->B) return set_error(SLB_ERR_INVALID, "slb_download: count must equal batch");
@@ -379,8 +390,8 @@ static int transfer(slb_handle h, int field, void *host, size_t count, cudaStrea
         return SLB_OK;
     }
     size_t per;
-    if (field == SLB_FIELD_MU) per = h->QD;
-    else if (field == SLB_FIELD_P) per = (size_t)h->N * h->N;
+    if (field == SLB_FIELD_MU) per = L.QD;
+    else if (field == SLB_FIELD_P) per = (size_t)L.N * L.N;
     else return set_error(SLB_ERR_INVALID, "slb_upload/download: unknown field");
     if (count == 0 || count % per != 0 || count > per * h->B)
         return set_error(SLB_ERR_INVALID, "slb_upload/download: count must be k * per-instance size, 1 <= k <= batch");
@@ -390,28 +401,18 @@ static int transfer(slb_handle h, int field, void *host, size_t count, cudaStrea
     for (int b0 = 0; b0 < nin; b0 += chunk) {
         const int cnt = (nin - b0) < chunk ? (nin - b0) : chunk;
         const size_t bytes = (size_t)cnt * per * 8;
-        const int64_t work = (int64_t)cnt * (field == SLB_FIELD_MU ? h->QD : (up && soa ? h->NP : h->N * h->N));
+        const int64_t work = (int64_t)cnt * (field == SLB_FIELD_MU ? L.QD : up ? L.NP : L.N * L.N);
         const int tpb = 256;
         const int grid = (int)((work + tpb - 1) / tpb);
         if (up) {
             SLB_CUDA(cudaMemcpyAsync(h->stage, hp + (size_t)b0 * per, bytes, cudaMemcpyHostToDevice, s));
-            if (field == SLB_FIELD_MU) {
-                if (soa) aos_to_soa_mu<<<grid, tpb, 0, s>>>(h->stage, h->mu, b0, cnt, h->QD, h->stride);
-                else aos_to_rec_mu<<<grid, tpb, 0, s>>>(h->stage, h->mu, b0, cnt, h->QD, h->qstride);
-            } else {
-                if (soa) dense_to_soa_P<<<grid, tpb, 0, s>>>(h->stage, h->P, b0, cnt, h->N, h->stride);
-                else dense_to_rec_P<<<grid, tpb, 0, s>>>(h->stage, h->P, b0, cnt, h->N, h->pstride, tiled);
-            }
+            if (field == SLB_FIELD_MU) mu_in<<<grid, tpb, 0, s>>>(h->stage, h->mu, L, b0, cnt);
+            else P_in<<<grid, tpb, 0, s>>>(h->stage, h->P, L, b0, cnt);
             count_launch();
             SLB_CUDA(cudaGetLastError());
         } else {
-            if (field == SLB_FIELD_MU) {
-                if (soa) soa_to_aos_mu<<<grid, tpb, 0, s>>>(h->mu, h->stage, b0, cnt, h->QD, h->stride);
-                else rec_to_aos_mu<<<grid, tpb, 0, s>>>(h->mu, h->stage, b0, cnt, h->QD, h->qstride);
-            } else {
-                if (soa) soa_to_dense_P<<<grid, tpb, 0, s>>>(h->P, h->stage, b0, cnt, h->N, h->stride);
-                else rec_to_dense_P<<<grid, tpb, 0, s>>>(h->P, h->stage, b0, cnt, h->N, h->pstride, tiled);
-            }
+            if (field == SLB_FIELD_MU) mu_out<<<grid, tpb, 0, s>>>(h->mu, h->stage, L, b0, cnt, 0, L.QD);
+            else P_out<<<grid, tpb, 0, s>>>(h->P, h->stage, L, b0, cnt);
             count_launch();
             SLB_CUDA(cudaGetLastError());
             SLB_CUDA(cudaMemcpyAsync(hp + (size_t)b0 * per, h->stage, bytes, cudaMemcpyDeviceToHost, s));
@@ -435,17 +436,10 @@ int slb_replicate(slb_handle h, int count, void *stream) {
     cudaStream_t s = S(stream);
     if (count == h->B) return SLB_OK;
     const int tpb = 256;
-    if (h->cfg.kind == SLB_KIND_UKF) {
-        int64_t w = (int64_t)h->QD * h->B;
-        replicate_soa<<<(unsigned)((w + tpb - 1) / tpb), tpb, 0, s>>>(h->mu, h->QD, h->stride, h->B, count);
-        w = (int64_t)h->NP * h->B;
-        replicate_soa<<<(unsigned)((w + tpb - 1) / tpb), tpb, 0, s>>>(h->P, h->NP, h->stride, h->B, count);
-    } else {
-        int64_t w = (int64_t)h->qstride * h->B;
-        replicate_rec<<<(unsigned)((w + tpb - 1) / tpb), tpb, 0, s>>>(h->mu, h->qstride, h->B, count);
-        w = (int64_t)h->pstride * h->B;
-        replicate_rec<<<(unsigned)((w + tpb - 1) / tpb), tpb, 0, s>>>(h->P, h->pstride, h->B, count);
-    }
+    int64_t w = (int64_t)h->L.QD * h->B;
+    replicate<<<(unsigned)((w + tpb - 1) / tpb), tpb, 0, s>>>(h->mu, h->L, h->B, count, false);
+    w = (int64_t)h->L.NP * h->B;
+    replicate<<<(unsigned)((w + tpb - 1) / tpb), tpb, 0, s>>>(h->P, h->L, h->B, count, true);
     count_launch(2);
     SLB_CUDA(cudaGetLastError());
     return SLB_OK;
@@ -460,7 +454,7 @@ static int ukf_call(slb_handle h, int pm, int mm, bool pred, bool upd, const dou
     DeviceGuard guard(h->cfg.device);
     FilterArgs a = make_args(h);
     a.u = u; a.dt = dt; a.Q = Q; a.z = z; a.R = R; a.gate = gate; a.m = 3;
-    a.qs = q_stride(h, h->N); a.rs = r_stride(h, 3);
+    a.qs = q_stride(h, h->L.N); a.rs = r_stride(h, 3);
     return launch_ukf(h->cfg.layout, pm, mm, pred, upd, a, S(stream));
 }
 int slb_ukf_predict(slb_handle h, int pm, const double *u, double dt, const double *Q, void *stream) {
@@ -488,9 +482,8 @@ struct HostStep {
 static int launch_chunk(slb_handle h, const HostStep &hs, int b0, int cnt, const double *du, const double *dz,
                         const double *dQ, const double *dp, const double *dR, cudaStream_t st) {
     FilterArgs a = make_args(h);
-    const bool soa = h->cfg.kind == SLB_KIND_UKF;
-    a.mu += soa ? (size_t)b0 : (size_t)b0 * h->qstride;
-    a.P += soa ? (size_t)b0 : (size_t)b0 * h->pstride;
+    a.mu += h->L.mu(b0, 0);
+    a.P += h->L.P(b0, 0, 0);
     a.status += b0;
     a.outliers += b0;
     a.B = cnt;
@@ -527,7 +520,6 @@ static int step_host_enqueue(slb_handle h, const HostStep &hs, cudaStream_t s) {
         if (forced > 0) nchunk = forced;
     }
     const int per = ((h->B + nchunk - 1) / nchunk + 31) / 32 * 32;
-    const bool soa = h->cfg.kind == SLB_KIND_UKF;
     int used = 0;
     for (int c = 0, b0 = 0; b0 < h->B; ++c, b0 += per) {
         const int cnt = h->B - b0 < per ? h->B - b0 : per;
@@ -540,8 +532,7 @@ static int step_host_enqueue(slb_handle h, const HostStep &hs, cudaStream_t s) {
         if (hs.mu_out) {
             const int OL = h->out_len, work = cnt * OL, tpb = 256;
             double *dst = dmu + (size_t)b0 * OL;
-            if (soa) soa_to_aos_mu<<<(work + tpb - 1) / tpb, tpb, 0, st>>>(h->mu, dst, b0, cnt, OL, h->stride, h->out_off);
-            else rec_to_aos_mu<<<(work + tpb - 1) / tpb, tpb, 0, st>>>(h->mu, dst, b0, cnt, OL, h->qstride, h->out_off);
+            mu_out<<<(work + tpb - 1) / tpb, tpb, 0, st>>>(h->mu, dst, h->L, b0, cnt, h->out_off, OL);
             count_launch();
             SLB_CUDA(cudaGetLastError());
             SLB_CUDA(cudaMemcpyAsync(hs.mu_out + (size_t)b0 * OL, dst, (size_t)cnt * OL * 8, cudaMemcpyDeviceToHost, st));
@@ -583,7 +574,7 @@ static int step_host(slb_handle h, const HostStep &hs, void *stream, bool wait =
     if (!h || !hs.u || !hs.Q || !hs.z || !hs.R) return set_error(SLB_ERR_INVALID, "slb_*_step_host: null argument");
     DeviceGuard guard(h->cfg.device);
     cudaStream_t s = S(stream);
-    const size_t ub = (size_t)h->B * hs.nu * 8, zb = (size_t)h->B * hs.m * 8, mub = (size_t)h->B * h->QD * 8;
+    const size_t ub = (size_t)h->B * hs.nu * 8, zb = (size_t)h->B * hs.m * 8, mub = (size_t)h->B * h->L.QD * 8;
     const size_t small = (size_t)(hs.nq * hs.nq + hs.m * hs.m + hs.nparams) * 8;
     if (ub + zb + mub > h->stage_bytes || small > 128 * 1024)
         return set_error(SLB_ERR_INVALID, "slb_*_step_host: batch / shared inputs too large for the staging buffers");
@@ -668,7 +659,7 @@ static int ukf_step_host(slb_handle h, int pm, int mm, const double *u_host, dou
     if (!h || h->cfg.kind != SLB_KIND_UKF) return set_error(SLB_ERR_INVALID, "slb_ukf_step_host: handle is not a UKF batch");
     if (h->noise) return set_error(SLB_ERR_INVALID, "slb_ukf_step_host: per-instance noise (slb_set_noise_layout) is device-resident only");
     if (mm != SLB_MM_GPS_POS) return set_error(SLB_ERR_INVALID, "ukf: unsupported measurement model");
-    const HostStep hs = {pm, mm, pm_nu(pm), 3, h->N, 0, gate_dof, dt, u_host, Q_host, nullptr, z_host, R_host, mu_out_host};
+    const HostStep hs = {pm, mm, pm_nu(pm), 3, h->L.N, 0, gate_dof, dt, u_host, Q_host, nullptr, z_host, R_host, mu_out_host};
     return step_host(h, hs, stream, wait);
 }
 int slb_ukf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
@@ -938,26 +929,12 @@ int slb_ensemble_stats(slb_handle h, double *out_dev, void *stream) {
     if (!h || !out_dev) return set_error(SLB_ERR_INVALID, "slb_ensemble_stats: null argument");
     DeviceGuard guard(h->cfg.device);
     cudaStream_t s = S(stream);
-    StatLayout l;
-    memset(&l, 0, sizeof(l));
-    l.N = h->N; l.QD = h->QD; l.stride = h->stride; l.qstride = h->qstride;
-    l.soa = h->cfg.kind == SLB_KIND_UKF;
-    auto add_state12 = [&](int at) { l.so3mask |= 1ull << (at + 1); };
-    if (h->cfg.kind == SLB_KIND_UKF) {
-        l.nblk = h->N / 3; l.so3mask = 0x2; l.nfeat = 0;
-    } else if (h->cfg.kind == SLB_KIND_USCKF) {
-        l.nblk = 12; l.nfeat = h->cfg.nk + h->cfg.nl;
-        add_state12(0); add_state12(4); add_state12(8);
-    } else {
-        l.nblk = 4 + 2 * h->cfg.nclones; l.nfeat = 0;
-        add_state12(0);
-        for (int j = 0; j < h->cfg.nclones; ++j) l.so3mask |= 1ull << (4 + 2 * j + 1);
-    }
-    if (l.N * l.N + l.N > STAT_TPB * STAT_MAXACC) return set_error(SLB_ERR_INVALID, "slb_ensemble_stats: state too large");
-    SLB_CUDA(cudaMemsetAsync(out_dev, 0, (size_t)(1 + l.N + l.N * l.N) * 8, s));
+    const int N = h->L.N;
+    if (N * N + N > STAT_TPB * STAT_MAXACC) return set_error(SLB_ERR_INVALID, "slb_ensemble_stats: state too large");
+    SLB_CUDA(cudaMemsetAsync(out_dev, 0, (size_t)(1 + N + N * N) * 8, s));
     const int nchunks = (h->B + STAT_CHUNK - 1) / STAT_CHUNK;
     const int grid = nchunks < 296 ? nchunks : 296;
-    ensemble_stats_kernel<<<grid, STAT_TPB, (size_t)STAT_CHUNK * l.N * 8, s>>>(h->mu, h->B, l, out_dev);
+    ensemble_stats_kernel<<<grid, STAT_TPB, (size_t)STAT_CHUNK * N * 8, s>>>(h->mu, h->B, h->L, out_dev);
     count_launch();
     SLB_CUDA(cudaGetLastError());
     return SLB_OK;
@@ -966,6 +943,8 @@ int slb_ensemble_stats(slb_handle h, double *out_dev, void *stream) {
 // ---- checkSigmaPoints() -----------------------------------------------------------------------------------
 int slb_check_sigma_points(slb_handle h, int32_t *flags_dev, double *diff_dev, void *stream) {
     if (!h || !flags_dev) return set_error(SLB_ERR_INVALID, "slb_check_sigma_points: null argument");
+    if (h->cfg.kind == SLB_KIND_UKF)
+        return set_error(SLB_ERR_INVALID, "slb_check_sigma_points: Usckf / Msckf batches only (the reference's ukfom::ukf has no checkSigmaPoints)");
     DeviceGuard guard(h->cfg.device);
     return launch_check_sigma_points(h, flags_dev, diff_dev, S(stream));
 }
@@ -1042,7 +1021,7 @@ int slb_gather_stats(slb_handle h, void *nccl_comm, double *out_dev, void *strea
     NcclApi &a = nccl_api();
     if (!a.ok) return set_error(SLB_ERR_NCCL, "NCCL is not available (dlopen libnccl.so.2 failed)");
     DeviceGuard guard(h->cfg.device);
-    const size_t n = (size_t)1 + h->N + (size_t)h->N * h->N;
+    const size_t n = (size_t)1 + h->L.N + (size_t)h->L.N * h->L.N;
     const ncclResult_t r = a.AllReduce(out_dev, out_dev, n, ncclDouble, ncclSum, (ncclComm_t)nccl_comm, S(stream));
     return r == ncclSuccess ? SLB_OK : nccl_fail("ncclAllReduce", r);
 }

@@ -11,33 +11,23 @@
 
 namespace slbd {
 
-struct ChkLayout {
-    int nblk;                     // 3-DOF blocks
-    unsigned long long so3mask;   // bit b: block b is SO3
-    int nfeat;                    // trailing plain scalars
-    int N, QD, NP, pstride, qstride;
-    int tiled;                    // 1: P records in the USCKF tile layout (prec), 0: packed row-major (tri)
-};
-
 SLB_DEV double warp_max(double v) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
     return v;
 }
 
-__global__ void __launch_bounds__(32) check_sigma_points_kernel(const double *mu, const double *P, int B, ChkLayout l,
+__global__ void __launch_bounds__(32) check_sigma_points_kernel(const double *mu, const double *P, int B, BatchLayout l,
                                                                 int32_t *flags, double *diff) {
     extern __shared__ double sm[];
     const int lane = threadIdx.x;
     const int N = l.N, QD = l.QD, NP = l.NP, NS = 2 * N + 1;
     double *Lp = sm, *Pa = Lp + NP, *D = Pa + NP, *mus = D + 32 * N, *ref = mus + QD, *md = ref + QD;
     for (int inst = blockIdx.x; inst < B; inst += gridDim.x) {
-        const double *Pg = P + (size_t)inst * l.pstride, *mug = mu + (size_t)inst * l.qstride;
-        auto rec = [&](int i, int j) { return l.tiled ? prec(N, i, j) : tri(i, j); };   // P(i, j), i >= j, in the record
         __syncwarp();
         for (int i = 0; i < N; ++i)
-            for (int j = lane; j <= i; j += 32) { Lp[tri(i, j)] = Pg[rec(i, j)]; Pa[tri(i, j)] = 0.0; }
-        for (int e = lane; e < QD; e += 32) { mus[e] = mug[e]; ref[e] = mug[e]; }
+            for (int j = lane; j <= i; j += 32) { Lp[tri(i, j)] = P[l.P(inst, i, j)]; Pa[tri(i, j)] = 0.0; }
+        for (int e = lane; e < QD; e += 32) { mus[e] = mu[l.mu(inst, e)]; ref[e] = mu[l.mu(inst, e)]; }
         __syncwarp();
         // ---- Eigen::LLT of Pk (lower triangle, Q8), right-looking, rows dealt to lanes -------------------------
         bool ok = true;
@@ -156,7 +146,7 @@ __global__ void __launch_bounds__(32) check_sigma_points_kernel(const double *mu
         __syncwarp();
         double dP = 0.0;
         for (int i = 0; i < N; ++i)
-            for (int j = lane; j <= i; j += 32) dP = fmax(dP, fabs(Pa[tri(i, j)] - Pg[rec(i, j)]));
+            for (int j = lane; j <= i; j += 32) dP = fmax(dP, fabs(Pa[tri(i, j)] - P[l.P(inst, i, j)]));
         dP = warp_max(dP);
         // |muX [-] mu|_inf: ref [-] mus, block per lane
         double dm = 0.0;
@@ -194,20 +184,7 @@ __global__ void __launch_bounds__(32) check_sigma_points_kernel(const double *mu
 namespace slb {
 
 int launch_check_sigma_points(const slb_batch_s *h, int32_t *flags, double *diff, cudaStream_t s) {
-    slbd::ChkLayout l;
-    l.N = h->N; l.QD = h->QD; l.NP = h->NP; l.pstride = h->pstride; l.qstride = h->qstride;
-    l.so3mask = 0;
-    l.tiled = h->cfg.kind == SLB_KIND_USCKF;
-    if (h->cfg.kind == SLB_KIND_USCKF) {
-        l.nblk = 12; l.nfeat = h->cfg.nk + h->cfg.nl;
-        l.so3mask = (1ull << 1) | (1ull << 5) | (1ull << 9);
-    } else if (h->cfg.kind == SLB_KIND_MSCKF) {
-        l.nblk = 4 + 2 * h->cfg.nclones; l.nfeat = 0;
-        l.so3mask = 1ull << 1;
-        for (int j = 0; j < h->cfg.nclones; ++j) l.so3mask |= 1ull << (4 + 2 * j + 1);
-    } else {
-        return set_error(SLB_ERR_INVALID, "slb_check_sigma_points: Usckf / Msckf batches only (the reference's ukfom::ukf has no checkSigmaPoints)");
-    }
+    const slbd::BatchLayout &l = h->L;
     const size_t smem = ((size_t)2 * l.NP + 32 * l.N + 2 * l.QD + l.N) * sizeof(double);
     SLB_CUDA(cudaFuncSetAttribute(slbd::check_sigma_points_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int grid = h->B < 148 * 3 * 8 ? h->B : 148 * 3 * 8;

@@ -4,21 +4,21 @@
 #include <stdint.h>
 
 #include "../../include/slb.h"
+#include "slb_math.cuh"
 
 constexpr int SLB_NXS = 3;  // internal streams of the *_step_host pipelines
 
+// The (featuresk, featuresk_l) sizes the USCKF update is instantiated for.  The reference's feature vectors are dynamic
+// (State.hpp:539-540, setMeasurement resizes Pk, Usckf.hpp:346-348); a batch has fixed sizes chosen at slb_create,
+// which rejects what is not in this list.  N = 36 + nk + nl <= 48 keeps the accumulator tiles in registers.
+#define SLB_USCKF_SHAPES(X) X(3, 0) X(3, 3) X(3, 6) X(3, 9) X(6, 0) X(6, 3) X(6, 6) X(9, 0) X(9, 3)
+
 struct slb_batch_s {
     slb_config cfg;
-    int N;        // tangent dimension of the full filter state
-    int QD;       // q-vector length
-    int NP;       // packed lower-triangle length N(N+1)/2
     int B;        // instances
-    int stride;   // UKF: SoA stride (B rounded up to 32); USCKF/MSCKF: unused
-    int pstride;  // USCKF/MSCKF: doubles per instance record of P (NP rounded up to 16 -> 128 B)
-    int qstride;  // USCKF/MSCKF: doubles per instance record of mu (QD rounded up to 2 -> 16 B)
-    double *mu;   // UKF: [QD][stride] SoA.  USCKF/MSCKF: [B][qstride]
-    double *P;    // UKF: [NP][stride] SoA packed lower.  MSCKF: [B][pstride] packed lower (tri).  USCKF: [B][pstride]
-                  // 8 x 8 tiles in DMMA accumulator order (prec, slb_math.cuh), the same NP doubles
+    slbd::BatchLayout L;  // dimensions and storage of mu and P
+    double *mu;   // L.mu_size(B) doubles
+    double *P;    // L.P_size(B) doubles
     int32_t *status;
     int32_t *outliers;
     // staging for the *_host entry points and upload/download

@@ -45,6 +45,30 @@ SLB_HD constexpr int prec(int N, int i, int j) {
     return tri(8 * I, 0) + 8 * h * J + (J < I ? 8 * (i & 7) + (j & 7) : tri(i & 7, j & 7));
 }
 
+// How a batch is stored (DESIGN §3), filled once by slb_create.  The filter kernels fix their format at compile time;
+// the host-launched utilities (transfers, replication, ensemble statistics, the sigma-point check) address the mean and
+// the covariance only through mu() and P().
+struct BatchLayout {
+    int N, QD, NP;                // tangent dimension, q-vector length, N (N + 1) / 2
+    int stride;                   // SoA row length: instances rounded up to 32
+    int qstride, pstride;         // doubles per mean / covariance record (QD rounded up to 2, NP to 16)
+    bool soa;                     // UKF: mu[c][stride], P[tri(r, c)][stride].  Otherwise instance records
+    bool tiled;                   // USCKF records: P(r, c) at prec(N, r, c).  MSCKF records: at tri(r, c)
+    int nblk;                     // manifold: 3-DOF blocks ...
+    unsigned long long so3mask;   // ... block b is SO3 (4 doubles in the q-vector) if bit b is set, else vect3 ...
+    int nfeat;                    // ... then this many plain feature scalars
+    // offset of mean scalar c of instance i
+    SLB_HD constexpr size_t mu(int i, int c) const { return soa ? (size_t)c * stride + i : (size_t)i * qstride + c; }
+    // offset of P(r, c), r >= c, of instance i
+    SLB_HD constexpr size_t P(int i, int r, int c) const {
+        const int e = tiled ? prec(N, r, c) : tri(r, c);
+        return soa ? (size_t)e * stride + i : (size_t)i * pstride + e;
+    }
+    // doubles of the mean / covariance storage of a batch of B instances
+    SLB_HD constexpr size_t mu_size(int B) const { return soa ? (size_t)QD * stride : (size_t)B * qstride; }
+    SLB_HD constexpr size_t P_size(int B) const { return soa ? (size_t)NP * stride : (size_t)B * pstride; }
+};
+
 // ---- SO3 -----------------------------------------------------------------------------------------
 // Sigma-point deviations are small rotations, so exp / log almost always see small arguments.  Both
 // have a branch-free polynomial fast path (minimax fits, relative error < 5e-18 before rounding) that

@@ -103,10 +103,6 @@ static int launch_predict_t(const FilterArgs &a, cudaStream_t s) {
     return SLB_OK;
 }
 
-// The (featuresk, featuresk_l) sizes the update is instantiated for.  The reference's feature vectors are dynamic
-// (State.hpp:539-540, setMeasurement resizes Pk, Usckf.hpp:346-348); a batch has fixed sizes chosen at slb_create,
-// which rejects what is not in this list.  N = 36 + nk + nl <= 48 keeps the accumulator tiles in registers.
-#define SLB_USCKF_SHAPES(X) X(3, 0) X(3, 3) X(3, 6) X(3, 9) X(6, 0) X(6, 3) X(6, 6) X(9, 0) X(9, 3)
 // the tiled record layout (prec) places every entry of the lower triangle once inside the N(N+1)/2 doubles of the
 // packed one, and every off-diagonal tile row it holds starts on a 16-byte boundary
 static constexpr bool prec_fills_record(int N) {
