@@ -98,7 +98,9 @@ enum {
     SLB_FIELD_MU = 1,     /* batch x qdim q-vectors                              */
     SLB_FIELD_P = 2,      /* batch x N x N row-major covariances                 */
     SLB_FIELD_STATUS = 3, /* batch x int32 (download only; pass an int32_t*)     */
-    SLB_FIELD_OUTLIERS = 4/* batch x int32 outlier count of the last MSCKF update */
+    SLB_FIELD_OUTLIERS = 4,/* batch x int32 outlier count of the last MSCKF update */
+    SLB_FIELD_NIS = 5     /* batch x double NIS of the last UKF / USCKF update (download only, with
+                             slb_set_nis_capture on; see there)                 */
 };
 
 typedef struct {
@@ -172,6 +174,14 @@ int slb_set_output_slice(slb_handle h, int offset, int count);
  * *_step_host_async entry points refuse to run: per-instance noise is device-resident only. */
 enum { SLB_NOISE_Q_PER_INSTANCE = 1, SLB_NOISE_R_PER_INSTANCE = 2 };
 int slb_set_noise_layout(slb_handle h, int flags);
+/* NIS capture: the Mahalanobis distance m2 = nu^T S^-1 nu that update(z, h, R, mt) hands to the caller's `mt` functor
+ * (Usckf.hpp:262,290-294).  on = 1 allocates batch doubles on the handle's device, filled with NaN; from then on every
+ * update-bearing call (slb_ukf_update / step / step_host[_async], slb_usckf_update / step / step_host[_async]) rewrites
+ * all of them with the m2 its gate was given, accepted or rejected, or NaN where the update stopped before forming it
+ * (SLB_ST_CHOL_FAIL).  Predict-only calls leave them alone.  on = 0 stops writing and frees the array.  Read it with
+ * slb_download(SLB_FIELD_NIS) or slb_device_ptr(SLB_FIELD_NIS), both SLB_ERR_INVALID while capture is off.
+ * SLB_ERR_INVALID on an MSCKF handle: its update gates per feature and forms no whole-innovation distance. */
+int slb_set_nis_capture(slb_handle h, int on);
 /* Pipelined flavour: identical, but returns as soon as the step is enqueued on `stream` (no
  * synchronisation), so consecutive steps overlap their host<->device traffic with each other's
  * kernels.  The host buffers must stay valid (and mu_out_host unread) until slb_wait(h, stream);
@@ -318,6 +328,22 @@ int slb_ensemble_stats(slb_handle h, double *out_dev, void *stream);
  * values in place on `stream`.  nccl_comm is an ncclComm_t passed as void* (NULL = this shard only).  NCCL is
  * resolved at run time (dlopen libnccl.so.2); SLB_ERR_NCCL if it is missing or a call fails. */
 int slb_gather_stats(slb_handle h, void *nccl_comm, double *out_dev, void *stream);
+/* Filter consistency (new; the reference has no counterpart -- its user would download every Pk and invert it):
+ * out_dev: 6 doubles, overwritten with {NEES count, sum, sum of squares, NIS count, sum, sum of squares} over this shard.
+ * truth_dev: batch x qdim q-vectors, instance-major dense (slb_upload's SLB_FIELD_MU format), or NULL = no NEES, in
+ * which case t0 = n = 0 and nees_dev is not written.  [t0, t0 + n): the tangent coordinates covered, in
+ * slb_ensemble_stats' vectorisation (3 per 3-DOF block, then the feature scalars); neither end may cut a 3-DOF block.
+ * Per instance NEES = e^T P_sub^-1 e with e = truth [-] mu (MTK: log(mu_q^-1 truth_q) on SO3 blocks, a difference
+ * elsewhere) and P_sub = P[t0:t0+n, t0:t0+n] the marginal covariance, from a Cholesky factorisation of P_sub; a
+ * non-positive or non-finite pivot or a non-finite e gives NaN and leaves the instance out of the count (status bits
+ * are not touched).  nees_dev: batch doubles or NULL.  The NIS triplet sums the finite entries of the captured NIS
+ * (slb_set_nis_capture), zeros when capture is off.  SLB_ERR_INVALID for a bad range, before any device work. */
+int slb_consistency_stats(slb_handle h, const double *truth_dev, int t0, int n, double *nees_dev, double *out_dev,
+                          void *stream);
+/* The same, merged over the ranks of an NCCL communicator: slb_consistency_stats on this shard, then
+ * ncclAllReduce(sum, double) of the 6 values in place on `stream` (nccl_comm NULL = this shard only). */
+int slb_gather_consistency(slb_handle h, void *nccl_comm, const double *truth_dev, int t0, int n, double *nees_dev,
+                           double *out_dev, void *stream);
 /* Communicator helpers for callers without an NCCL binding of their own (ctypes, cgo, the C++ facade):
  * rank 0 calls slb_nccl_unique_id (id128: 128 bytes) and ships the bytes to the other ranks by any means,
  * every rank then calls slb_nccl_comm_init with its rank and CUDA device. */

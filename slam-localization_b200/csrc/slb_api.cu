@@ -190,6 +190,7 @@ static FilterArgs make_args(slb_handle h) {
     a.nk = h->cfg.nk; a.nl = h->cfg.nl; a.k = h->cfg.nclones;
     a.misc = h->misc_dev;
     a.out_off = h->out_off; a.out_len = h->out_len;
+    a.nis = h->nis;
     return a;
 }
 
@@ -331,7 +332,7 @@ int slb_destroy(slb_handle h) {
     if (!h) return SLB_OK;
     DeviceGuard guard(h->cfg.device);
     cudaFree(h->mu); cudaFree(h->P); cudaFree(h->status); cudaFree(h->outliers);
-    cudaFree(h->stage); cudaFree(h->shared_small); cudaFree(h->counts_dev); cudaFree(h->misc_dev);
+    cudaFree(h->stage); cudaFree(h->shared_small); cudaFree(h->counts_dev); cudaFree(h->misc_dev); cudaFree(h->nis);
     for (int i = 0; i < SLB_NXS; ++i) {
         if (h->xs[i]) cudaStreamDestroy(h->xs[i]);
         if (h->ev_done[i]) cudaEventDestroy(h->ev_done[i]);
@@ -360,6 +361,22 @@ int slb_set_noise_layout(slb_handle h, int flags) {
     h->noise = flags;
     return SLB_OK;
 }
+int slb_set_nis_capture(slb_handle h, int on) {
+    if (!h) return set_error(SLB_ERR_INVALID, "slb_set_nis_capture: null handle");
+    if (h->cfg.kind == SLB_KIND_MSCKF)
+        return set_error(SLB_ERR_INVALID, "slb_set_nis_capture: UKF and USCKF batches only (the MSCKF update gates per feature and "
+                                          "forms no whole-innovation distance)");
+    if (on != 0 && on != 1) return set_error(SLB_ERR_INVALID, "slb_set_nis_capture: on must be 0 or 1");
+    DeviceGuard guard(h->cfg.device);
+    if (!on) {
+        if (h->nis) SLB_CUDA(cudaFree(h->nis));   // (cudaFree waits for the kernels that still write it)
+        h->nis = nullptr;
+        return SLB_OK;
+    }
+    if (!h->nis) SLB_CUDA(cudaMalloc(&h->nis, (size_t)h->B * 8));
+    SLB_CUDA(cudaMemset(h->nis, 0xff, (size_t)h->B * 8));   // all-ones bytes: a NaN in every entry
+    return SLB_OK;
+}
 // doubles between consecutive instances' Q / R for a handle's noise layout (0 = shared)
 static int q_stride(slb_handle h, int n) { return (h->noise & SLB_NOISE_Q_PER_INSTANCE) ? n * n : 0; }
 static int r_stride(slb_handle h, int m) { return (h->noise & SLB_NOISE_R_PER_INSTANCE) ? m * m : 0; }
@@ -373,6 +390,10 @@ int slb_device_ptr(slb_handle h, int field, void **dev) {
         case SLB_FIELD_P: *dev = h->P; return SLB_OK;
         case SLB_FIELD_STATUS: *dev = h->status; return SLB_OK;
         case SLB_FIELD_OUTLIERS: *dev = h->outliers; return SLB_OK;
+        case SLB_FIELD_NIS:
+            if (!h->nis) return set_error(SLB_ERR_INVALID, "slb_device_ptr: NIS capture is off (slb_set_nis_capture)");
+            *dev = h->nis;
+            return SLB_OK;
     }
     return set_error(SLB_ERR_INVALID, "slb_device_ptr: unknown field");
 }
@@ -386,6 +407,14 @@ static int transfer(slb_handle h, int field, void *host, size_t count, cudaStrea
         if (count != (size_t)h->B) return set_error(SLB_ERR_INVALID, "slb_download: count must equal batch");
         SLB_CUDA(cudaMemcpyAsync(host, field == SLB_FIELD_STATUS ? h->status : h->outliers, (size_t)h->B * 4,
                                  cudaMemcpyDeviceToHost, s));
+        SLB_CUDA(cudaStreamSynchronize(s));
+        return SLB_OK;
+    }
+    if (field == SLB_FIELD_NIS) {
+        if (up) return set_error(SLB_ERR_INVALID, "slb_upload: the NIS field is read-only");
+        if (!h->nis) return set_error(SLB_ERR_INVALID, "slb_download: NIS capture is off (slb_set_nis_capture)");
+        if (count != (size_t)h->B) return set_error(SLB_ERR_INVALID, "slb_download: count must equal batch");
+        SLB_CUDA(cudaMemcpyAsync(host, h->nis, (size_t)h->B * 8, cudaMemcpyDeviceToHost, s));
         SLB_CUDA(cudaStreamSynchronize(s));
         return SLB_OK;
     }
@@ -486,6 +515,7 @@ static int launch_chunk(slb_handle h, const HostStep &hs, int b0, int cnt, const
     a.P += h->L.P(b0, 0, 0);
     a.status += b0;
     a.outliers += b0;
+    if (a.nis) a.nis += b0;
     a.B = cnt;
     a.u = du; a.dt = hs.dt; a.Q = dQ; a.z = dz; a.R = dR; a.params = dp; a.gate = hs.gate; a.m = hs.m;
     switch (h->cfg.kind) {
@@ -620,10 +650,11 @@ static int step_host(slb_handle h, const HostStep &hs, void *stream, bool wait =
         return SLB_OK;
     }
     const int ki[8] = {hs.pm, hs.mm, hs.nu, hs.m, hs.nq, hs.nparams, hs.gate, h->out_off * 4096 + h->out_len};
-    const void *kp[6] = {hs.u, hs.Q, hs.params, hs.z, hs.R, hs.mu_out};
+    // the NIS array is a key too: toggling slb_set_nis_capture re-captures, so no replay writes a freed array or skips it
+    const void *kp[7] = {hs.u, hs.Q, hs.params, hs.z, hs.R, hs.mu_out, h->nis};
     bool same = h->step_exec != nullptr && h->step_key_dt == hs.dt;
     for (int i = 0; i < 8 && same; ++i) same = h->step_key_i[i] == ki[i];
-    for (int i = 0; i < 6 && same; ++i) same = h->step_key_p[i] == kp[i];
+    for (int i = 0; i < 7 && same; ++i) same = h->step_key_p[i] == kp[i];
     if (!same) {
         if (h->step_exec) { cudaGraphExecDestroy(h->step_exec); h->step_exec = nullptr; }
         const int64_t n0 = slb_launch_count();
@@ -647,7 +678,7 @@ static int step_host(slb_handle h, const HostStep &hs, void *stream, bool wait =
         h->step_kernels = nk;
         h->step_key_dt = hs.dt;
         for (int i = 0; i < 8; ++i) h->step_key_i[i] = ki[i];
-        for (int i = 0; i < 6; ++i) h->step_key_p[i] = kp[i];
+        for (int i = 0; i < 7; ++i) h->step_key_p[i] = kp[i];
     }
     SLB_CUDA(cudaGraphLaunch(h->step_exec, s));
     count_launch(h->step_kernels);
@@ -940,6 +971,28 @@ int slb_ensemble_stats(slb_handle h, double *out_dev, void *stream) {
     return SLB_OK;
 }
 
+// ---- filter consistency: NEES against a per-instance truth, NIS of the last update --------------------------------
+// t0 and t0 + n must not cut a 3-DOF block; n = 0 (with no truth) asks for the NIS sums only
+static bool consistency_range_ok(const slbd::BatchLayout &L, const double *truth, int t0, int n) {
+    if (!truth) return n == 0 && t0 == 0;
+    const int nb3 = 3 * L.nblk;
+    if (n <= 0 || t0 < 0 || t0 + n > L.N) return false;
+    if (t0 < nb3 && t0 % 3 != 0) return false;
+    if (t0 + n < nb3 && (t0 + n) % 3 != 0) return false;
+    return true;
+}
+int slb_consistency_stats(slb_handle h, const double *truth_dev, int t0, int n, double *nees_dev, double *out_dev,
+                          void *stream) {
+    if (!h || !out_dev) return set_error(SLB_ERR_INVALID, "slb_consistency_stats: null argument");
+    if (!consistency_range_ok(h->L, truth_dev, t0, n))
+        return set_error(SLB_ERR_INVALID, "slb_consistency_stats: [t0, t0 + n) must be a non-empty range of the tangent "
+                                          "coordinates that cuts no 3-DOF block (n = 0 and t0 = 0 without a truth)");
+    DeviceGuard guard(h->cfg.device);
+    cudaStream_t s = S(stream);
+    SLB_CUDA(cudaMemsetAsync(out_dev, 0, 6 * sizeof(double), s));
+    return launch_consistency(h, truth_dev, t0, n, nees_dev, out_dev, s);
+}
+
 // ---- checkSigmaPoints() -----------------------------------------------------------------------------------
 int slb_check_sigma_points(slb_handle h, int32_t *flags_dev, double *diff_dev, void *stream) {
     if (!h || !flags_dev) return set_error(SLB_ERR_INVALID, "slb_check_sigma_points: null argument");
@@ -1023,6 +1076,17 @@ int slb_gather_stats(slb_handle h, void *nccl_comm, double *out_dev, void *strea
     DeviceGuard guard(h->cfg.device);
     const size_t n = (size_t)1 + h->L.N + (size_t)h->L.N * h->L.N;
     const ncclResult_t r = a.AllReduce(out_dev, out_dev, n, ncclDouble, ncclSum, (ncclComm_t)nccl_comm, S(stream));
+    return r == ncclSuccess ? SLB_OK : nccl_fail("ncclAllReduce", r);
+}
+int slb_gather_consistency(slb_handle h, void *nccl_comm, const double *truth_dev, int t0, int n, double *nees_dev,
+                           double *out_dev, void *stream) {
+    if (!h || !out_dev) return set_error(SLB_ERR_INVALID, "slb_gather_consistency: null argument");
+    const int rc = slb_consistency_stats(h, truth_dev, t0, n, nees_dev, out_dev, stream);
+    if (rc != SLB_OK || !nccl_comm) return rc;   // no communicator: this device's shard only
+    NcclApi &a = nccl_api();
+    if (!a.ok) return set_error(SLB_ERR_NCCL, "NCCL is not available (dlopen libnccl.so.2 failed)");
+    DeviceGuard guard(h->cfg.device);
+    const ncclResult_t r = a.AllReduce(out_dev, out_dev, 6, ncclDouble, ncclSum, (ncclComm_t)nccl_comm, S(stream));
     return r == ncclSuccess ? SLB_OK : nccl_fail("ncclAllReduce", r);
 }
 

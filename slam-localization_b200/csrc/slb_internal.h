@@ -35,10 +35,11 @@ struct slb_batch_s {
     int step_kernels;          // kernel launches inside the captured step
     int step_key_i[8];
     double step_key_dt;
-    const void *step_key_p[6];
+    const void *step_key_p[7];   // the host buffers, and the NIS array the captured kernels write (slb_set_nis_capture)
     cudaEvent_t ev_start, ev_done[SLB_NXS];
     int out_off, out_len;      // slb_set_output_slice: part of the q-vector the *_step_host entry points copy back
     int noise;                 // slb_set_noise_layout: SLB_NOISE_* flags (0 = Q and R shared by the batch)
+    double *nis;               // slb_set_nis_capture: B doubles, the m2 of every instance's last update (nullptr = off)
     // zero-copy *_step_host: host copy of the Q | R last uploaded to shared_small (the upload is skipped while the caller
     // keeps passing the same values: two tiny DMA operations per step are 10 % of a UKFoM step)
     double qr_cache[144 + 81];
@@ -96,8 +97,12 @@ struct FilterArgs {
     int rs;
     double *mu_out;   // optional instance-major copy of the posterior means (may be mapped host memory), B x out_len
     int out_off, out_len;  // the slice [out_off, out_off + out_len) of the q-vector that goes to mu_out
+    // NIS capture (slb_set_nis_capture): the UKF / USCKF update writes the m2 its gate was given to nis[inst] (NaN when
+    // the update stopped before forming it); the launchers select the kernels' NIS instantiations when it is set.  The
+    // last member, so every other one keeps its offset and the kernels without NIS compile as before.
+    double *nis;
 };
-static_assert(sizeof(FilterArgs) == 152, "FilterArgs layout");
+static_assert(sizeof(FilterArgs) == 160, "FilterArgs layout");
 
 // slb_ukf.cu
 int launch_ukf(int layout, int pm, int mm, bool predict, bool update, const FilterArgs &a, cudaStream_t s);
@@ -112,6 +117,8 @@ int launch_msckf_update(int mm, const FilterArgs &a, cudaStream_t s);
 int launch_msckf_update_ekf(int mm, const FilterArgs &a, cudaStream_t s);
 // slb_check.cu
 int launch_check_sigma_points(const slb_batch_s *h, int32_t *flags, double *diff, cudaStream_t s);
+// slb_consistency.cu: out[6] += {NEES count, sum, sum of squares, NIS count, sum, sum of squares} (out zeroed by the caller)
+int launch_consistency(const slb_batch_s *h, const double *truth, int t0, int n, double *nees, double *out, cudaStream_t s);
 // slb_fusion.cu
 int launch_fusion(int d, int64_t n, int op, const double *x1, const double *C1, const double *x2,
                   const double *C2, double *xo, double *Co, cudaStream_t s);

@@ -220,7 +220,9 @@ SLB_DEV void group_cov(double *sig, double *ps, const double *Qp, int sub, const
 // lane the 6 lower entries of R as the update starts; the warp's shared Qp is not used (8 per-instance copies per warp
 // would cost a CTA).  Issued together with the record's copies they kept 18 more registers live through the predict and
 // the fused MTK9 step spilled 264 / 308 B instead of 216 / 260 B.
-template <class L, int PM, class MM, int G, int TPB, int MINB, bool PRED, bool UPD, bool PIN = false>
+// NIS: lane sub == 0 of each group stores the m2 its gate is given to a.nis[inst], NaN when the update's factorisation
+// of P (or the predict before it) failed.
+template <class L, int PM, class MM, int G, int TPB, int MINB, bool PRED, bool UPD, bool PIN = false, bool NIS = false>
 __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
     typedef Rec<L, MM::M, G> R;
     constexpr int N = L::N, QD = L::QD, NP = L::NP, NS = 2 * N + 1, M = MM::M, MP = M * (M + 1) / 2;
@@ -469,6 +471,7 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
             }
         }
         __syncwarp();
+        if (NIS && sub == 0 && valid) a.nis[inst] = upd ? m2 : __longlong_as_double(0x7ff8000000000000ll);
         const bool accept = chi2_accept(m2, a.gate);
         if (upd && !accept) st |= SLB_ST_GATE_REJECT;
         const bool apply = upd && accept;
@@ -574,8 +577,8 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
 
 namespace slb {
 
-// Per-instance noise (a.qs / a.rs set by slb_set_noise_layout) selects the PIN instantiations; the shared-noise
-// kernels are unchanged.
+// Per-instance noise (a.qs / a.rs set by slb_set_noise_layout) selects the PIN instantiations, NIS capture (a.nis) the
+// NIS ones of the update-bearing kernels; the shared-noise kernels are unchanged.
 template <class L, int PM, class MM>
 static int launch_ukf_t(bool predict, bool update, const FilterArgs &a, cudaStream_t s) {
     constexpr int G = 4, TPB = 128, MINB = 3;
@@ -592,6 +595,12 @@ static int launch_ukf_t(bool predict, bool update, const FilterArgs &a, cudaStre
         return SLB_OK;
     };
     const bool pin = (predict && a.qs) || (update && a.rs);
+    if (update && a.nis) {
+        if (pin) return predict ? go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true, true, true>)
+                                : go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true, true, true>);
+        return predict ? go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true, false, true>)
+                       : go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true, false, true>);
+    }
     if (pin) {
         if (predict && update) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true, true>);
         if (predict) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, false, true>);

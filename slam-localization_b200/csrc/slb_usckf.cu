@@ -128,8 +128,9 @@ bool usckf_shape_supported(int nk, int nl) {
     return false;
 }
 
-// record-resident kernel (slb_usckf_step.cuh): PRED && UPD = the fused step, UPD alone = update; PIN = per-instance noise
-template <int NK, int NL, bool PRED, bool UPD, bool PIN>
+// record-resident kernel (slb_usckf_step.cuh): PRED && UPD = the fused step, UPD alone = update; PIN = per-instance noise,
+// NIS = capture of the update's Mahalanobis distance
+template <int NK, int NL, bool PRED, bool UPD, bool PIN, bool NIS = false>
 static int launch_step_t(const FilterArgs &a, cudaStream_t s) {
     typedef slbd::StepCfg<NK, NL> C;
     // CTA shape: the register file (168 registers) holds 12 warps per SM.  Measured on the (3,9) fleet, 524 288 instances
@@ -158,7 +159,7 @@ static int launch_step_t(const FilterArgs &a, cudaStream_t s) {
         static_assert(!PIN || (WPB == WPB0 && fit >= (fit0 < 12 / WPB0 ? fit0 : 12 / WPB0)), "PIN costs occupancy");
     }
 #endif
-    auto kern = slbd::usckf_step_kernel<SLB_PM_USCKF_TEST, NK, NL, PRED, UPD, WPB, MINB, PIN>;
+    auto kern = slbd::usckf_step_kernel<SLB_PM_USCKF_TEST, NK, NL, PRED, UPD, WPB, MINB, PIN, NIS>;
     SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     // L2 prefetch distance in instances: SLB_USCKF_PREFETCH waves of (SMs x resident warps); default off (measured: no
     // gain at 0 / 1 / 2 / 4 waves, and 16 % more DRAM reads at the full fleet size)
@@ -184,11 +185,15 @@ static int launch_step_t(const FilterArgs &a, cudaStream_t s) {
     return SLB_OK;
 }
 
+template <int NK, int NL, bool NIS>
+static int launch_step_pin(bool predict, const FilterArgs &a, cudaStream_t s) {
+    if ((predict && a.qs) || a.rs)
+        return predict ? launch_step_t<NK, NL, true, true, true, NIS>(a, s) : launch_step_t<NK, NL, false, true, true, NIS>(a, s);
+    return predict ? launch_step_t<NK, NL, true, true, false, NIS>(a, s) : launch_step_t<NK, NL, false, true, false, NIS>(a, s);
+}
 template <int NK, int NL>
 static int launch_step_nknl(bool predict, const FilterArgs &a, cudaStream_t s) {
-    if ((predict && a.qs) || a.rs)
-        return predict ? launch_step_t<NK, NL, true, true, true>(a, s) : launch_step_t<NK, NL, false, true, true>(a, s);
-    return predict ? launch_step_t<NK, NL, true, true, false>(a, s) : launch_step_t<NK, NL, false, true, false>(a, s);
+    return a.nis ? launch_step_pin<NK, NL, true>(predict, a, s) : launch_step_pin<NK, NL, false>(predict, a, s);
 }
 
 int launch_usckf(int pm, int mm, bool predict, bool update, const FilterArgs &a, cudaStream_t s) {

@@ -340,11 +340,12 @@ struct PanelStep<C, C::NPAN> {
     SLB_DEV static void run(UpdState<C> &, const double *, double *, double *, double *, double *, int) {}
 };
 
-// update of the resident record.  Returns status bits; `dirty` is set when Ps / mus changed.
+// update of the resident record.  Returns status bits; `dirty` is set when Ps / mus changed, `m2out` (left as it is by
+// the early returns) receives the Mahalanobis distance the gate is given.
 // PIN: R comes from `Rs`, this instance's packed lower triangle staged in shared memory (cp.async, issued with z).
 template <int NK, int NL, bool PIN = false>
 SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double *zs, const double *Rs,
-                              const slb::FilterArgs &a, int lane, bool &dirty) {
+                              const slb::FilterArgs &a, int lane, bool &dirty, double &m2out) {
     typedef StepCfg<NK, NL> C;
     constexpr int N = C::N, NT = C::NT, NPAD = C::NPAD, JLAST = C::JLAST, KP = C::KP;
     const int a_ = lane & 3, b_ = lane >> 2;
@@ -445,6 +446,7 @@ SLB_DEV int usckf_update_smem(double *Ps, double *mus, double *scr, const double
         m2 = fma(nu[r], t, m2);
     }
     if (!sok) return SLB_ST_CHOL_FAIL;
+    m2out = m2;
     if (!chi2_accept(m2, a.gate)) return SLB_ST_GATE_REJECT;
     // covXZ from the accumulator tiles into the rows of Cs, then lane i turns row i into K, -covXZ and K nu
 #pragma unroll
@@ -553,7 +555,8 @@ struct ResidentView {
 // PIN: per-instance noise (slb_set_noise_layout), Q at a.Q + inst * a.qs and R at a.R + inst * a.rs (stride 0 = shared).
 // Both are fetched with the record: R's lower triangle by cp.async into RP extra doubles of the warp's area, the 6 Q
 // entries a lane adds into registers.
-template <int PM, int NK, int NL, bool PRED, bool UPD, int WPB, int MINB, bool PIN = false>
+// NIS: lane 0 stores the update's m2 to a.nis[inst] (NaN when the update returned before forming it).
+template <int PM, int NK, int NL, bool PRED, bool UPD, int WPB, int MINB, bool PIN = false, bool NIS = false>
 __global__ void __launch_bounds__(WPB * 32, MINB) usckf_step_kernel(slb::FilterArgs a) {
     typedef StepCfg<NK, NL> C;
     constexpr int SMW = PIN ? C::SMP : C::SM;
@@ -605,7 +608,9 @@ __global__ void __launch_bounds__(WPB * 32, MINB) usckf_step_kernel(slb::FilterA
         st = predict12_block<PM, true, PIN>(ResidentView<C::N>{Ps}, mus + 26, u, a.dt, scr, a.Q, qv, NK + NL, mus + 26, lane, dirty);
     }
     if (PRED) SLB_CTA_SYNC();
-    if (UPD) st |= usckf_update_smem<NK, NL, PIN>(Ps, mus, scr, zs, Rs, a, lane, dirty);
+    double m2 = __longlong_as_double(0x7ff8000000000000ll);   // NaN
+    if (UPD) st |= usckf_update_smem<NK, NL, PIN>(Ps, mus, scr, zs, Rs, a, lane, dirty, m2);
+    if (NIS && lane == 0) a.nis[inst] = m2;
     cp_async_wait0();   // (an update that bailed out early has not waited for z)
     // ---- record out ----------------------------------------------------------------------------------------------
     if (dirty) {

@@ -18,7 +18,7 @@ LAYOUT_POSE6, LAYOUT_MTK9 = 6, 9
 PM_UKFOM_IMU, PM_UKFOM_IMU_REFBUG, PM_POSE6_ODOM, PM_USCKF_TEST, PM_MSCKF_DELTAPOSE = 1, 2, 3, 4, 5
 MM_GPS_POS, MM_USCKF_VO, MM_MSCKF_REPROJ = 101, 102, 103
 STATEK, STATEK_L, STATEK_I = 1, 2, 3
-FIELD_MU, FIELD_P, FIELD_STATUS, FIELD_OUTLIERS = 1, 2, 3, 4
+FIELD_MU, FIELD_P, FIELD_STATUS, FIELD_OUTLIERS, FIELD_NIS = 1, 2, 3, 4, 5
 ST_CHOL_FAIL, ST_MEAN_NOCONV, ST_GATE_REJECT, ST_NONFINITE, ST_QR_ROWS = 1, 2, 4, 8, 16
 NSTATUS = 5
 NOISE_Q_PER_INSTANCE, NOISE_R_PER_INSTANCE = 1, 2
@@ -34,6 +34,7 @@ EXPORTS = [
     "slb_datamodel_safe_fuse", "slb_msckf_update_ekf", "slb_transform_compose", "slb_deadreckon_update_pose",
     "slb_ukf_step_host_async", "slb_usckf_step_host_async", "slb_msckf_step_host_async", "slb_wait",
     "slb_set_output_slice", "slb_set_noise_layout", "slb_check_sigma_points", "slb_gather_stats", "slb_nccl_unique_id", "slb_nccl_comm_init", "slb_nccl_comm_destroy",
+    "slb_set_nis_capture", "slb_consistency_stats", "slb_gather_consistency",
 ]
 
 
@@ -80,6 +81,9 @@ def lib():
         L.slb_wait.argtypes = [vp, vp]
         L.slb_set_output_slice.argtypes = [vp, i32, i32]
         L.slb_set_noise_layout.argtypes = [vp, i32]
+        L.slb_set_nis_capture.argtypes = [vp, i32]
+        L.slb_consistency_stats.argtypes = [vp, dp, i32, i32, dp, dp, vp]
+        L.slb_gather_consistency.argtypes = [vp, vp, dp, i32, i32, dp, dp, vp]
         L.slb_check_sigma_points.argtypes = [vp, vp, vp, vp]
         L.slb_gather_stats.argtypes = [vp, vp, dp, vp]
         L.slb_nccl_unique_id.argtypes = [vp]
@@ -304,6 +308,41 @@ class Batch:
         out = out if out is not None else DeviceArray(shape=(1 + self.N + self.N * self.N,))
         check(lib().slb_gather_stats(self.h, comm.c if comm is not None else None, out.ptr, _stream()))
         return out
+
+    def set_nis_capture(self, on):
+        """slb_set_nis_capture: while on, every update-bearing call stores each instance's Mahalanobis distance
+        m2 = nu^T S^-1 nu (what the reference hands to `mt`), NaN where the update failed before forming it."""
+        check(lib().slb_set_nis_capture(self.h, 1 if on else 0))
+
+    def nis(self):
+        """The captured NIS of the last update, (B,) float64 (SlbError while capture is off)."""
+        out = np.empty(self.B)
+        check(lib().slb_download(self.h, FIELD_NIS, _hp(out), out.size, _stream()))
+        return out
+
+    def _consistency(self, fn, comm, truth, t0, n, nees):
+        if truth is None:
+            t, n = None, 0 if n is None else n
+        else:
+            t = dev(truth)
+            if tuple(t.t.shape) != (self.B, self.QD):
+                raise ValueError("truth must have shape (%d, %d), got %s" % (self.B, self.QD, tuple(t.t.shape)))
+            n = self.N - t0 if n is None else n
+        out = DeviceArray(shape=(6,))
+        ne = DeviceArray(shape=(self.B,)) if nees else None
+        args = (t.ptr if t is not None else None, t0, n, ne.ptr if ne is not None else None, out.ptr, _stream())
+        check(fn(self.h, *args) if comm is False else fn(self.h, comm.c if comm is not None else None, *args))
+        return (out.numpy(), ne.numpy()) if nees else out.numpy()
+
+    def consistency_stats(self, truth=None, t0=0, n=None, nees=False):
+        """slb_consistency_stats: {NEES count, sum, sum of squares, NIS count, sum, sum of squares} over this batch.
+        truth: (B, qdim) q-vectors (None = NIS only); [t0, t0 + n) the tangent coordinates of the NEES (n=None: to the
+        end of the state).  nees=True also returns the per-instance NEES, NaN where P_sub is not positive definite."""
+        return self._consistency(lib().slb_consistency_stats, False, truth, t0, n, nees)
+
+    def gather_consistency(self, comm=None, truth=None, t0=0, n=None, nees=False):
+        """slb_gather_consistency: consistency_stats all-reduced over an NcclComm (None: this shard only)."""
+        return self._consistency(lib().slb_gather_consistency, comm, truth, t0, n, nees)
 
     def check_sigma_points(self):
         """checkSigmaPoints() (Usckf.hpp:769-789, Msckf.hpp:818-838): returns (flags[B] int32, diff[B, 2])."""

@@ -135,6 +135,30 @@ class Batch {
         out.download(v);
         return v;
     }
+    // NIS capture (slb_set_nis_capture, Ukf / Usckf only): while on, every update stores the distance its gate was given
+    void setNisCapture(bool on) { check(slb_set_nis_capture(h_, on ? 1 : 0), "slb_set_nis_capture"); }
+    // The m2 = nu^T S^-1 nu of every instance's last update: what the reference passes to update()'s `mt` functor
+    // (Usckf.hpp:262,290-294).  NaN where the update failed before forming it.  Needs setNisCapture(true).
+    Vec mahalanobis() const {
+        Vec v((size_t)B_);
+        check(slb_download(h_, SLB_FIELD_NIS, v.data(), v.size(), nullptr), "slb_download(nis)");
+        return v;
+    }
+    // {NEES count, sum, sum of squares, NIS count, sum, sum of squares} (slb_gather_consistency): NEES of `truth`
+    // (batch x qdim q-vectors; empty = NIS only, with t0 = n = 0) over the tangent coordinates [t0, t0 + n), merged over
+    // an NCCL communicator when one is given.
+    Vec consistencyStats(const Vec &truth, int t0, int n, void *nccl_comm = nullptr) const {
+        if (!truth.empty() && truth.size() != (size_t)B_ * QD_)
+            throw Error(SLB_ERR_INVALID, "consistencyStats: truth must hold batch * qdim doubles");
+        DevBuf dt;
+        if (!truth.empty()) dt.assign(truth.data(), truth.size());
+        DevOut out((size_t)6);
+        check(slb_gather_consistency(h_, nccl_comm, truth.empty() ? nullptr : dt.get(), t0, n, nullptr, out.get(), nullptr),
+              "slb_gather_consistency");
+        Vec v;
+        out.download(v);
+        return v;
+    }
   protected:
     // checkSigmaPoints() (Usckf.hpp:769-789, Msckf.hpp:818-838).  The reference assert()s; a batch returns per-instance
     // flags: bit 0 max|Pktest - Pk| > 1e-6, bit 1 the sigma-point mean moved away from mu_state, bit 2 LLT failed.
