@@ -297,8 +297,7 @@ __global__ void __launch_bounds__(WPB * 32) ekf_update_kernel(int64_t n, const d
     // lower triangle of the dense matrix -> packed rows: one flat loop over the packed index (a nested row / column loop
     // diverges on every row and spent 2 300 instructions per warp issuing 33 copies per lane)
     for (int e = lane; e < C::NP; e += 32) {
-        int i = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-        i += (tri(i + 1, 0) <= e) - (tri(i, 0) > e);
+        const int i = tri_row(e);
         cp_async8(Pl + e, Pg + i * N + (e - tri(i, 0)));
     }
     for (int e = lane; e < M * N; e += 32) Hs[e] = __ldg(H + e);

@@ -32,6 +32,13 @@ typedef Layout<3, 0x2> LayMtk9;     // pos, orient, vel                 (mtk_sta
 typedef Layout<4, 0x2> LayState12;  // pos, orient, velo, angvelo       (State)
 
 SLB_HD constexpr int tri(int i, int j) { return i * (i + 1) / 2 + j; }  // i >= j
+// row r of the packed index e = tri(r, c) (the column is then e - tri(r, 0)): a float square-root estimate and a +-1
+// fix-up, exact for e < 2^20
+SLB_DEV int tri_row(int e) {
+    int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
+    r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
+    return r;
+}
 
 // Offset of P(i, j), i >= j, in a USCKF record of dimension N: the lower block triangle of 8 x 8 tiles, tile rows in
 // order, within a tile row the off-diagonal tiles first (row-major, 8 columns each), then the diagonal tile (its packed

@@ -99,128 +99,158 @@ __device__ long long ms_phase_dbg[4 * 32];
 constexpr int MS_PS = 1600;
 constexpr int MS_NXL = 2400;   // offset in region C of the next instance's factor (above the <= 32 x 72 partial sums of the mean)
 SLB_DEV int ps_idx(int srow, int k) { return srow * 8 + ((k + 4 * ((srow >> 1) & 1)) & 7); }
+// inverse of the diagonal block at p0, row-major 8 x 8 at the end of PS, double-buffered by panel parity: the look-ahead
+// writes the next panel's while the right-hand-side tasks still read the current one (staging uses < 184 of the 200 rows)
+SLB_DEV double *dinv_of(double *PS, int p0) { return PS + MS_PS - 128 + 64 * ((p0 >> 3) & 1); }
+
+// The pieces of one panel of the blocked Cholesky below.  chol_blocked and chol_dual schedule them differently over the
+// warps; a piece's arithmetic does not depend on which warp runs it, so both factor a matrix bit for bit alike.
+//
+// 8x8 diagonal block at p0 on one warp, two entries per lane in the DMMA accumulator layout (row fr, columns 2 fk and
+// 2 fk + 1; a0, a1 are 0 outside the lower triangle).  Right-looking and square-root-free: step k broadcasts d_k = a_kk,
+// a_ik and a_jk by shuffles, then a_ij -= (a_ik / d_k) a_jk is ONE FMA per entry -- the dependent chain per column is
+// shuffle + reciprocal + multiply + FMA and there is hardly any other instruction to issue (lane-per-row needed up to 7
+// shuffle + FMA pairs per step).  The same Gauss transforms are accumulated on the identity (M = prod (I - v_k e_k^T)):
+// diag(1 / L_ii) M is the inverse of the block (into dinv_of(PS, p0)), which turns the panel solve below it from an 8-step
+// forward substitution per row into 36 independent FMAs per row.  All square roots are taken after the loop.
+// INVD: also store invd[p0 + i] = 1 / L_ii (a compile-time flag, so that chol_dual's blocks carry neither the store nor a test).
+template <bool INVD>
+SLB_DEV void factor_diag(double *A, int n, int p0, double a0, double a1, double *PS, double *invd, int *ok_flag) {
+    const int lane = threadIdx.x & 31, fr = lane >> 2, fk = lane & 3;
+    const int pb = min(8, n - p0);
+    const int i = fr, j0 = 2 * fk, j1 = j0 + 1;
+    double *dinv = dinv_of(PS, p0);
+    double m0 = (i == j0) ? 1.0 : 0.0, m1 = (i == j1) ? 1.0 : 0.0;
+    double di = 1.0, dj0 = 1.0, dj1 = 1.0;   // pivots of this lane's row and of its two columns
+    bool ok = true;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+        if (k < pb) {
+            const int kh = k >> 1;
+            const double ak = (k & 1) ? a1 : a0;                       // this lane's entry in column pair kh
+            const double d = bcast(ak, 4 * k + kh);                    // a_kk
+            const double aik = __shfl_sync(0xffffffffu, ak, 4 * i + kh);
+            ok = ok && (d > 0.0);
+            if (i == k) di = d;
+            if (j0 == k) dj0 = d;
+            if (j1 == k) dj1 = d;
+            if (k < 7) {
+                const double ajk0 = __shfl_sync(0xffffffffu, ak, 4 * j0 + kh), ajk1 = __shfl_sync(0xffffffffu, ak, 4 * j1 + kh);
+                const double mk0 = bcast(m0, 4 * k + fk), mk1 = bcast(m1, 4 * k + fk);
+                const double v = aik * rcp_fast(d);
+                if (j0 > k) a0 = fma(-v, ajk0, a0);
+                if (j1 > k) a1 = fma(-v, ajk1, a1);
+                const double vm = i > k ? v : 0.0;
+                m0 = fma(-vm, mk0, m0);
+                m1 = fma(-vm, mk1, m1);
+            }
+        }
+    }
+    double si, ri, s0, r0c, s1, r1c;
+    sqrt_rsqrt(di, si, ri);
+    sqrt_rsqrt(dj0, s0, r0c);
+    sqrt_rsqrt(dj1, s1, r1c);
+    if (i < pb) {
+        if (INVD && fk == 0) invd[p0 + i] = ri;
+        if (j0 <= i) A[tri(p0 + i, p0 + j0)] = (j0 == i) ? s0 : a0 * r0c;
+        if (j1 <= i) A[tri(p0 + i, p0 + j1)] = (j1 == i) ? s1 : a1 * r1c;
+    }
+    *reinterpret_cast<double2 *>(dinv + i * 8 + j0) = make_double2(j0 <= i ? ri * m0 : 0.0, j1 <= i ? ri * m1 : 0.0);
+    ok = __all_sync(0xffffffffu, ok);
+    if (!ok && lane == 0) *ok_flag = 0;
+}
+
+// this lane's two entries of the first diagonal block, in factor_diag's layout
+SLB_DEV void first_diag(const double *A, int n, double &a0, double &a1) {
+    const int lane = threadIdx.x & 31, fr = lane >> 2, fk = lane & 3;
+    const int pb = min(8, n);
+    a0 = (fr < pb && 2 * fk <= fr) ? A[tri(fr, 2 * fk)] : 0.0;
+    a1 = (fr < pb && 2 * fk + 1 <= fr) ? A[tri(fr, 2 * fk + 1)] : 0.0;
+}
+
+// Panel solve of row tile rt below the diagonal block at p0 (the panel's rows start at r0, na of them): rows * inv(L_pp)^T
+// as two DMMAs (B[k][c] = Dinv[c][k]).  The result goes back in place and, as dense swizzled 8-wide rows, into PS for the
+// fragment loads of the trailing update.  na > 0 implies a full panel (pb == 8).
+SLB_DEV void panel_solve(double *A, double *PS, int p0, int r0, int na, int rt) {
+    const int lane = threadIdx.x & 31, fr = lane >> 2, fk = lane & 3;
+    const double *dinv = dinv_of(PS, p0);
+    const int w = 8 * rt + fr, wc = min(w, na - 1);
+    const double *Ai = A + tri(r0 + wc, p0);
+    double x0 = 0.0, x1 = 0.0;
+    dmma884(x0, x1, Ai[fk], dinv[fr * 8 + fk]);
+    dmma884(x0, x1, Ai[fk + 4], dinv[fr * 8 + fk + 4]);
+    __syncwarp();   // every lane has read its fragment of the rows before they are overwritten
+    if (w < na) {
+        double *Ao = A + tri(r0 + w, p0) + 2 * fk;
+        Ao[0] = x0;
+        Ao[1] = x1;
+        *reinterpret_cast<double2 *>(PS + ps_idx(w, 2 * fk)) = make_double2(x0, x1);
+    }
+}
+
+// Look-ahead: the trailing update of the next diagonal block (at r0; both operands are the staged rows 0..7) leaves the
+// block in the accumulator layout, which is the layout factor_diag works in: no round trip through shared memory.
+SLB_DEV void next_diag(const double *A, const double *PS, int r0, int na, double &a0, double &a1) {
+    const int lane = threadIdx.x & 31, fr = lane >> 2, fk = lane & 3;
+    const int rr = min(fr, na - 1), pbn = min(8, na);
+    const int i = r0 + fr, j = r0 + 2 * fk;
+    const bool v0 = fr < pbn && 2 * fk <= fr, v1 = fr < pbn && 2 * fk + 1 <= fr;
+    const double x0 = PS[ps_idx(rr, fk)], x1 = PS[ps_idx(rr, fk + 4)];
+    const double c0 = v0 ? A[tri(i, j)] : 0.0, c1 = v1 ? A[tri(i, j + 1)] : 0.0;
+    double d0 = 0.0, d1 = 0.0;
+    dmma884(d0, d1, x0, x0);
+    dmma884(d0, d1, x1, x1);
+    a0 = v0 ? c0 - d0 : 0.0;
+    a1 = v1 ? c1 - d1 : 0.0;
+}
+
+// Trailing tile t >= 1 of the panel (tile 0 is the next diagonal block), operands from the staged panel.  Rows / columns
+// beyond the matrix only feed accumulator entries that are never stored: their addresses are clamped, not masked; a
+// trailing update only exists after a full 8-wide panel (pb == 8), so the k-loop needs no bound either.
+SLB_DEV void trailing_tile(double *A, const double *PS, int n, int r0, int na, int t) {
+    const int lane = threadIdx.x & 31, fr = lane >> 2, fk = lane & 3;
+    int tr, tc;
+    tri_tile(t, tr, tc);
+    const int i0 = r0 + 8 * tr, j0 = r0 + 8 * tc;
+    double d0 = 0.0, d1 = 0.0;
+    const int ra = min(8 * tr + fr, na - 1), rb = min(8 * tc + fr, na - 1);
+    const int i = i0 + fr, j = j0 + 2 * fk;
+    const bool v0 = i < n && j <= i, v1 = i < n && j + 1 <= i;
+    double *po = A + tri(min(i, n - 1), min(j, i));   // old values requested together with the operands
+    const double c0 = v0 ? po[0] : 0.0, c1 = v1 ? po[1] : 0.0;
+    dmma884(d0, d1, PS[ps_idx(ra, fk)], PS[ps_idx(rb, fk)]);
+    dmma884(d0, d1, PS[ps_idx(ra, fk + 4)], PS[ps_idx(rb, fk + 4)]);
+    if (v0) po[0] = c0 - d0;
+    if (v1) po[1] = c1 - d1;
+}
+
 SLB_DEV void chol_blocked(double *A, int n, int *ok_flag, double *invd, double *PS, double *X = nullptr, int nx = 0,
                           int xs = 0, double *xe = nullptr, double *Wp = nullptr) {
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int fr = lane >> 2, fk = lane & 3;
     const int nxr = X ? nx + 1 : 0, nxt = (nxr + 7) >> 3;
-    // inverse of a diagonal block, row-major 8 x 8, double-buffered by panel parity: the look-ahead writes the next panel's
-    // while the right-hand-side tasks still read the current one (staging uses < 184 of the 200 rows of PS)
-    auto dinv_of = [&](int p0) { return PS + MS_PS - 128 + 64 * ((p0 >> 3) & 1); };
-    // 8x8 diagonal block on one warp, two entries per lane in the DMMA accumulator layout (row fr, columns 2 fk and
-    // 2 fk + 1).  Right-looking and square-root-free: step k broadcasts d_k = a_kk, a_ik and a_jk by shuffles, then
-    // a_ij -= (a_ik / d_k) a_jk is ONE FMA per entry -- the dependent chain per column is shuffle + reciprocal + multiply +
-    // FMA and there is hardly any other instruction to issue (lane-per-row needed up to 7 shuffle + FMA pairs per step).
-    // The same Gauss transforms are accumulated on the identity (M = prod (I - v_k e_k^T)): diag(1 / L_ii) M is the inverse
-    // of the block, which turns the panel solve below it from an 8-step forward substitution per row into 36 independent
-    // FMAs per row.  All square roots are taken after the loop.
-    auto factor_diag = [&](int p0, double a0, double a1) {   // a0, a1: this lane's two entries (0 outside the lower triangle)
-        const int pb = min(8, n - p0);
-        const int i = fr, j0 = 2 * fk, j1 = j0 + 1;
-        double *dinv = dinv_of(p0);
-        double m0 = (i == j0) ? 1.0 : 0.0, m1 = (i == j1) ? 1.0 : 0.0;
-        double di = 1.0, dj0 = 1.0, dj1 = 1.0;   // pivots of this lane's row and of its two columns
-        bool ok = true;
-#pragma unroll
-        for (int k = 0; k < 8; ++k) {
-            if (k < pb) {
-                const int kh = k >> 1;
-                const double ak = (k & 1) ? a1 : a0;                       // this lane's entry in column pair kh
-                const double d = bcast(ak, 4 * k + kh);                    // a_kk
-                const double aik = __shfl_sync(0xffffffffu, ak, 4 * i + kh);
-                ok = ok && (d > 0.0);
-                if (i == k) di = d;
-                if (j0 == k) dj0 = d;
-                if (j1 == k) dj1 = d;
-                if (k < 7) {
-                    const double ajk0 = __shfl_sync(0xffffffffu, ak, 4 * j0 + kh), ajk1 = __shfl_sync(0xffffffffu, ak, 4 * j1 + kh);
-                    const double mk0 = bcast(m0, 4 * k + fk), mk1 = bcast(m1, 4 * k + fk);
-                    const double v = aik * rcp_fast(d);
-                    if (j0 > k) a0 = fma(-v, ajk0, a0);
-                    if (j1 > k) a1 = fma(-v, ajk1, a1);
-                    const double vm = i > k ? v : 0.0;
-                    m0 = fma(-vm, mk0, m0);
-                    m1 = fma(-vm, mk1, m1);
-                }
-            }
-        }
-        double si, ri, s0, r0c, s1, r1c;
-        sqrt_rsqrt(di, si, ri);
-        sqrt_rsqrt(dj0, s0, r0c);
-        sqrt_rsqrt(dj1, s1, r1c);
-        if (i < pb) {
-            if (fk == 0) invd[p0 + i] = ri;
-            if (j0 <= i) A[tri(p0 + i, p0 + j0)] = (j0 == i) ? s0 : a0 * r0c;
-            if (j1 <= i) A[tri(p0 + i, p0 + j1)] = (j1 == i) ? s1 : a1 * r1c;
-        }
-        *reinterpret_cast<double2 *>(dinv + i * 8 + j0) = make_double2(j0 <= i ? ri * m0 : 0.0, j1 <= i ? ri * m1 : 0.0);
-        ok = __all_sync(0xffffffffu, ok);
-        if (!ok && lane == 0) *ok_flag = 0;
-    };
     if (warp == 0) {
-        const int pb = min(8, n);
-        factor_diag(0, (fr < pb && 2 * fk <= fr) ? A[tri(fr, 2 * fk)] : 0.0, (fr < pb && 2 * fk + 1 <= fr) ? A[tri(fr, 2 * fk + 1)] : 0.0);
+        double a0, a1;
+        first_diag(A, n, a0, a1);
+        factor_diag<true>(A, n, 0, a0, a1, PS, invd, ok_flag);
     }
     __syncthreads();
     for (int p0 = 0; p0 < n; p0 += 8) {
         const int pb = min(8, n - p0);
         const int r0 = p0 + pb, na = n - r0;
-        const double *dinv = dinv_of(p0);
+        const double *dinv = dinv_of(PS, p0);
         CHOL_T(p0 >> 3, 0);
-        // panel below the diagonal block: rows * inv(L_pp)^T, one 8-row tile per warp as two DMMAs (B[k][c] = Dinv[c][k]); the
-        // result goes back in place and, as dense swizzled 8-wide rows, into the staging area for the fragment loads of the
-        // trailing update.  na > 0 implies a full panel (pb == 8).
-        for (int rt = warp; 8 * rt < na; rt += MS_W) {
-            const int w = 8 * rt + fr, wc = min(w, na - 1);
-            const double *Ai = A + tri(r0 + wc, p0);
-            double x0 = 0.0, x1 = 0.0;
-            dmma884(x0, x1, Ai[fk], dinv[fr * 8 + fk]);
-            dmma884(x0, x1, Ai[fk + 4], dinv[fr * 8 + fk + 4]);
-            __syncwarp();   // every lane has read its fragment of the rows before they are overwritten
-            if (w < na) {
-                double *Ao = A + tri(r0 + w, p0) + 2 * fk;
-                Ao[0] = x0;
-                Ao[1] = x1;
-                *reinterpret_cast<double2 *>(PS + ps_idx(w, 2 * fk)) = make_double2(x0, x1);
-            }
-        }
+        for (int rt = warp; 8 * rt < na; rt += MS_W) panel_solve(A, PS, p0, r0, na, rt);   // one 8-row tile per warp
         CHOL_T(p0 >> 3, 1);
         __syncthreads();
         CHOL_T(p0 >> 3, 2);
-        // rows / columns beyond the matrix only feed accumulator entries that are never stored: their addresses are clamped,
-        // not masked; a trailing update only exists after a full 8-wide panel (pb == 8), so the k-loop needs no bound either
         const int nt = (na + 7) >> 3, ntiles = nt * (nt + 1) / 2;
-        // operands come from the staged panel; rows beyond the matrix are clamped (their accumulator rows are dropped)
-        auto a_tile = [&](int t) {
-            int tr, tc;
-            tri_tile(t, tr, tc);
-            const int i0 = r0 + 8 * tr, j0 = r0 + 8 * tc;
-            double d0 = 0.0, d1 = 0.0;
-            const int ra = min(8 * tr + fr, na - 1), rb = min(8 * tc + fr, na - 1);
-            const int i = i0 + fr, j = j0 + 2 * fk;
-            const bool v0 = i < n && j <= i, v1 = i < n && j + 1 <= i;
-            double *po = A + tri(min(i, n - 1), min(j, i));   // old values requested together with the operands
-            const double c0 = v0 ? po[0] : 0.0, c1 = v1 ? po[1] : 0.0;
-            dmma884(d0, d1, PS[ps_idx(ra, fk)], PS[ps_idx(rb, fk)]);
-            dmma884(d0, d1, PS[ps_idx(ra, fk + 4)], PS[ps_idx(rb, fk + 4)]);
-            if (v0) po[0] = c0 - d0;
-            if (v1) po[1] = c1 - d1;
-        };
         if (warp == 0) {
-            if (ntiles > 0) {
-                // look-ahead: warp 0 owns the next diagonal block.  Its trailing update (both operands are the staged rows
-                // 0..7) leaves the block in the accumulator layout, which is the layout factor_diag works in: no round trip
-                // through shared memory; the factorisation runs while the other warps update their tiles.
-                const int rr = min(fr, na - 1), pbn = min(8, na);
-                const int i = r0 + fr, j = r0 + 2 * fk;
-                const bool v0 = fr < pbn && 2 * fk <= fr, v1 = fr < pbn && 2 * fk + 1 <= fr;
-                const double x0 = PS[ps_idx(rr, fk)], x1 = PS[ps_idx(rr, fk + 4)];
-                const double c0 = v0 ? A[tri(i, j)] : 0.0, c1 = v1 ? A[tri(i, j + 1)] : 0.0;
-                double d0 = 0.0, d1 = 0.0;
-                dmma884(d0, d1, x0, x0);
-                dmma884(d0, d1, x1, x1);
+            if (ntiles > 0) {   // warp 0 owns the next diagonal block: it is factored while the other warps run their tasks
+                double a0, a1;
+                next_diag(A, PS, r0, na, a0, a1);
                 CHOL_T(p0 >> 3, 3);
-                factor_diag(r0, v0 ? c0 - d0 : 0.0, v1 ? c1 - d1 : 0.0);
+                factor_diag<true>(A, n, r0, a0, a1, PS, invd, ok_flag);
             }
         } else {
             // Work list of the 15 other warps, longest tasks first:
@@ -314,7 +344,7 @@ SLB_DEV void chol_blocked(double *A, int n, int *ok_flag, double *invd, double *
                     if (v1) Wp[tri(c0 + 1, wi)] = f1;
                     continue;
                 }
-                a_tile(t - nxq - nwt + 1);
+                trailing_tile(A, PS, n, r0, na, t - nxq - nwt + 1);
             }
         }
         CHOL_T(p0 >> 3, 4);
@@ -330,116 +360,38 @@ SLB_DEV void chol_blocked(double *A, int n, int *ok_flag, double *invd, double *
 // A Cholesky without right-hand sides keeps one warp busy (the diagonal-block chain) and 15 waiting.  chol(P_new) of the
 // current instance and chol(P) of the NEXT instance (its record is already in shared memory) are independent, so they are
 // factored panel by panel in the same phases: warp 0 owns the diagonal blocks of A1, warp 1 (another scheduler) those of
-// A2, the panel solves and trailing tiles of both are spread over the other warps.  Same arithmetic per matrix as
-// chol_blocked (bitwise: the per-matrix operations and their order do not depend on which warp runs them).
-SLB_DEV void dual_factor_diag(double *A, int n, int p0, double a0, double a1, double *dinv, int *ok_flag, int lane) {
-    const int fr = lane >> 2, fk = lane & 3;
-    const int pb = min(8, n - p0);
-    const int i = fr, j0 = 2 * fk, j1 = j0 + 1;
-    double m0 = (i == j0) ? 1.0 : 0.0, m1 = (i == j1) ? 1.0 : 0.0;
-    double di = 1.0, dj0 = 1.0, dj1 = 1.0;
-    bool ok = true;
-#pragma unroll
-    for (int k = 0; k < 8; ++k) {
-        if (k < pb) {
-            const int kh = k >> 1;
-            const double ak = (k & 1) ? a1 : a0;
-            const double d = bcast(ak, 4 * k + kh);
-            const double aik = __shfl_sync(0xffffffffu, ak, 4 * i + kh);
-            ok = ok && (d > 0.0);
-            if (i == k) di = d;
-            if (j0 == k) dj0 = d;
-            if (j1 == k) dj1 = d;
-            if (k < 7) {
-                const double ajk0 = __shfl_sync(0xffffffffu, ak, 4 * j0 + kh), ajk1 = __shfl_sync(0xffffffffu, ak, 4 * j1 + kh);
-                const double mk0 = bcast(m0, 4 * k + fk), mk1 = bcast(m1, 4 * k + fk);
-                const double v = aik * rcp_fast(d);
-                if (j0 > k) a0 = fma(-v, ajk0, a0);
-                if (j1 > k) a1 = fma(-v, ajk1, a1);
-                const double vm = i > k ? v : 0.0;
-                m0 = fma(-vm, mk0, m0);
-                m1 = fma(-vm, mk1, m1);
-            }
-        }
-    }
-    double si, ri, s0, r0c, s1, r1c;
-    sqrt_rsqrt(di, si, ri);
-    sqrt_rsqrt(dj0, s0, r0c);
-    sqrt_rsqrt(dj1, s1, r1c);
-    if (i < pb) {
-        if (j0 <= i) A[tri(p0 + i, p0 + j0)] = (j0 == i) ? s0 : a0 * r0c;
-        if (j1 <= i) A[tri(p0 + i, p0 + j1)] = (j1 == i) ? s1 : a1 * r1c;
-    }
-    *reinterpret_cast<double2 *>(dinv + i * 8 + j0) = make_double2(j0 <= i ? ri * m0 : 0.0, j1 <= i ? ri * m1 : 0.0);
-    ok = __all_sync(0xffffffffu, ok);
-    if (!ok && lane == 0) *ok_flag = 0;
-}
-
+// A2, the panel solves and trailing tiles of both are spread over the other warps.  The pieces are chol_blocked's, so each
+// matrix is factored bit for bit as chol_blocked factors it.
 SLB_DEV void chol_dual(double *A1, double *A2, int n, int *ok1, int *ok2, double *PS1, double *PS2) {
-    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const int fr = lane >> 2, fk = lane & 3;
-    auto dinv_of = [&](double *PS, int p0) { return PS + MS_PS - 128 + 64 * ((p0 >> 3) & 1); };
+    const int warp = threadIdx.x >> 5;
     if (warp < 2) {
         double *A = warp ? A2 : A1;
-        const int pb = min(8, n);
-        dual_factor_diag(A, n, 0, (fr < pb && 2 * fk <= fr) ? A[tri(fr, 2 * fk)] : 0.0, (fr < pb && 2 * fk + 1 <= fr) ? A[tri(fr, 2 * fk + 1)] : 0.0,
-                         dinv_of(warp ? PS2 : PS1, 0), warp ? ok2 : ok1, lane);
+        double a0, a1;
+        first_diag(A, n, a0, a1);
+        factor_diag<false>(A, n, 0, a0, a1, warp ? PS2 : PS1, nullptr, warp ? ok2 : ok1);
     }
     __syncthreads();
     for (int p0 = 0; p0 < n; p0 += 8) {
         const int pb = min(8, n - p0);
         const int r0 = p0 + pb, na = n - r0;
-        const int ntl = (na + 7) >> 3;
-        for (int t = warp; t < 2 * ntl; t += MS_W) {   // panel solve: rows * inv(L_pp)^T, one 8-row tile per warp
-            const int m = t >= ntl, rt = t - m * ntl;
-            double *A = m ? A2 : A1, *PS = m ? PS2 : PS1;
-            const double *dinv = dinv_of(PS, p0);
-            const int w = 8 * rt + fr, wc = min(w, na - 1);
-            const double *Ai = A + tri(r0 + wc, p0);
-            double x0 = 0.0, x1 = 0.0;
-            dmma884(x0, x1, Ai[fk], dinv[fr * 8 + fk]);
-            dmma884(x0, x1, Ai[fk + 4], dinv[fr * 8 + fk + 4]);
-            __syncwarp();
-            if (w < na) {
-                double *Ao = A + tri(r0 + w, p0) + 2 * fk;
-                Ao[0] = x0;
-                Ao[1] = x1;
-                *reinterpret_cast<double2 *>(PS + ps_idx(w, 2 * fk)) = make_double2(x0, x1);
-            }
+        const int nt = (na + 7) >> 3, ntiles = nt * (nt + 1) / 2;
+        for (int t = warp; t < 2 * nt; t += MS_W) {   // one 8-row tile per warp
+            const int m = t >= nt;
+            panel_solve(m ? A2 : A1, m ? PS2 : PS1, p0, r0, na, t - m * nt);
         }
         __syncthreads();
-        const int nt = (na + 7) >> 3, ntiles = nt * (nt + 1) / 2;
         if (warp < 2) {
             if (ntiles > 0) {   // look-ahead on the next diagonal block of this warp's matrix
                 double *A = warp ? A2 : A1, *PS = warp ? PS2 : PS1;
-                const int rr = min(fr, na - 1), pbn = min(8, na);
-                const int i = r0 + fr, j = r0 + 2 * fk;
-                const bool v0 = fr < pbn && 2 * fk <= fr, v1 = fr < pbn && 2 * fk + 1 <= fr;
-                const double x0 = PS[ps_idx(rr, fk)], x1 = PS[ps_idx(rr, fk + 4)];
-                const double c0 = v0 ? A[tri(i, j)] : 0.0, c1 = v1 ? A[tri(i, j + 1)] : 0.0;
-                double d0 = 0.0, d1 = 0.0;
-                dmma884(d0, d1, x0, x0);
-                dmma884(d0, d1, x1, x1);
-                dual_factor_diag(A, n, r0, v0 ? c0 - d0 : 0.0, v1 ? c1 - d1 : 0.0, dinv_of(PS, r0), warp ? ok2 : ok1, lane);
+                double a0, a1;
+                next_diag(A, PS, r0, na, a0, a1);
+                factor_diag<false>(A, n, r0, a0, a1, PS, nullptr, warp ? ok2 : ok1);
             }
         } else {
             const int nat = max(ntiles - 1, 0);
             for (int t = warp - 2; t < 2 * nat; t += MS_W - 2) {
-                const int m = t >= nat, tt = t - m * nat + 1;
-                double *A = m ? A2 : A1, *PS = m ? PS2 : PS1;
-                int tr, tc;
-                tri_tile(tt, tr, tc);
-                const int i0 = r0 + 8 * tr, j0 = r0 + 8 * tc;
-                double d0 = 0.0, d1 = 0.0;
-                const int ra = min(8 * tr + fr, na - 1), rb = min(8 * tc + fr, na - 1);
-                const int i = i0 + fr, j = j0 + 2 * fk;
-                const bool v0 = i < n && j <= i, v1 = i < n && j + 1 <= i;
-                double *po = A + tri(min(i, n - 1), min(j, i));
-                const double c0 = v0 ? po[0] : 0.0, c1 = v1 ? po[1] : 0.0;
-                dmma884(d0, d1, PS[ps_idx(ra, fk)], PS[ps_idx(rb, fk)]);
-                dmma884(d0, d1, PS[ps_idx(ra, fk + 4)], PS[ps_idx(rb, fk + 4)]);
-                if (v0) po[0] = c0 - d0;
-                if (v1) po[1] = c1 - d1;
+                const int m = t >= nat;
+                trailing_tile(m ? A2 : A1, m ? PS2 : PS1, n, r0, na, t - m * nat + 1);
             }
         }
         __syncthreads();
@@ -467,6 +419,70 @@ SLB_DEV int gate_remove_pair(int *kept, int len, int i, int lane) {
         len = num;
     }
     return len;
+}
+
+// The reference's sequential outlier scan (removeOutliers, quirk Q6) on one warp, 32 positions at a time: every lane tests one
+// position against the current index list kept[0..len), the first rejection (if any) is applied, and the scan resumes from
+// there.  m2_at(ii) is the Mahalanobis distance of scan position ii; the 2-dof 5 % bound rejects NaN too.
+// Returns (kept length, outlier count).
+template <class M2>
+SLB_DEV int2 gate_scan(int *kept, int M, int lane, M2 m2_at) {
+    int len = M, out = 0, i = 0;
+    for (int e = lane; e < M; e += 32) kept[e] = e;
+    __syncwarp();
+    while (i < len / 2) {
+        const int ii = i + lane;
+        const bool rj = ii < len / 2 && !chi2_accept(m2_at(ii), 2);
+        const unsigned bal = __ballot_sync(0xffffffffu, rj);
+        if (!bal) {
+            i += 32;
+            continue;
+        }
+        i += __ffs(bal) - 1;
+        len = gate_remove_pair(kept, len, i, lane);
+        ++out;
+    }
+    return make_int2(len, out);
+}
+
+// UKF flavour: nu_p^T S_pp^-1 nu_p of the measurement pair p = (ia, ib), S packed lower
+SLB_DEV double m2_pair_S(const double *S, const double *nu, int ia, int ib) {
+    const double s00 = S[tri(ia, ia)], s11 = S[tri(ib, ib)], s10 = ib > ia ? S[tri(ib, ia)] : S[tri(ia, ib)];
+    const double det = s00 * s11 - s10 * s10;
+    const double v0 = nu[ia], v1 = nu[ib];
+    return (v0 * (s11 * v0 - s10 * v1) + v1 * (s00 * v1 - s10 * v0)) / det;
+}
+
+// EKF flavour: (v0, v1) I (v0, v1)^T with I = [i00 i10; i10 i11], a 2x2 diagonal block of the information matrix
+SLB_DEV double m2_pair_info(double i00, double i10, double i11, double v0, double v1) {
+    return v0 * (i00 * v0 + i10 * v1) + v1 * (i10 * v0 + i11 * v1);
+}
+
+// dst = src - Y Y^T (:262 / :336) over the lower 8x8 tiles of an N x N matrix, src and dst packed lower; Y is N x K with
+// row stride ys (one ragged k-step when K is not a multiple of 4).  The old values are requested before the k-loop so
+// that their latency hides behind it.
+SLB_DEV void sub_yyt(const double *Y, int ys, int N, int K, const double *src, double *dst) {
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, fr = lane >> 2, fk = lane & 3;
+    const int nrt = (N + 7) >> 3, ntiles = nrt * (nrt + 1) / 2;
+    for (int t = warp; t < ntiles; t += MS_W) {
+        int tr, tc;
+        tri_tile(t, tr, tc);
+        const int r = 8 * tr + fr, c = 8 * tc + 2 * fk;
+        const double *pa = Y + min(r, N - 1) * ys + fk, *pb = Y + min(8 * tc + fr, N - 1) * ys + fk;
+        const double g0 = (r < N && c <= r) ? src[tri(r, c)] : 0.0, g1 = (r < N && c + 1 <= r) ? src[tri(r, c + 1)] : 0.0;
+        double d0 = 0.0, d1 = 0.0;
+        const int kfull = K & ~3;
+#pragma unroll 4
+        for (int k0 = 0; k0 < kfull; k0 += 4) dmma884(d0, d1, pa[k0], pb[k0]);
+        if (kfull < K) {
+            const bool in = kfull + fk < K;
+            dmma884(d0, d1, in ? pa[kfull] : 0.0, in ? pb[kfull] : 0.0);
+        }
+        if (r < N) {
+            if (c <= r) dst[tri(r, c)] = g0 - d0;
+            if (c + 1 <= r) dst[tri(r, c + 1)] = g1 - d1;
+        }
+    }
 }
 
 SLB_DEV int ms_qoff(int b) { return b < 4 ? (b == 0 ? 0 : b == 1 ? 3 : b == 2 ? 7 : 10) : 13 + 7 * ((b - 4) >> 1) + (((b - 4) & 1) ? 3 : 0); }
@@ -646,42 +662,10 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_update_kernel(slb::FilterArgs a
         if (a.gate) {
             // every feature against the 2-dof 5% bound in parallel first: while nothing is rejected the reference's
             // sequential scan keeps the identity indexing, so "all accepted" needs no scan at all
-            bool rej = false;
-            if (tid < NF) {
-                const int ia = 2 * tid, ib = ia + 1;
-                const double s00 = RA[tri(ia, ia)], s11 = RA[tri(ib, ib)], s10 = RA[tri(ib, ia)];
-                const double det = s00 * s11 - s10 * s10;
-                const double v0 = nu[ia], v1 = nu[ib];
-                const double m2 = (v0 * (s11 * v0 - s10 * v1) + v1 * (s00 * v1 - s10 * v0)) / det;
-                rej = !(m2 < 5.99);
-            }
+            const bool rej = tid < NF && !chi2_accept(m2_pair_S(RA, nu, 2 * tid, 2 * tid + 1), 2);
             if (__syncthreads_or(rej) && warp == 0) {
-                // the reference's sequential scan, 32 positions at a time: every lane tests one position against the
-                // current index list, the first rejection (if any) is applied, and the scan resumes from there
-                int len = M, out = 0, i = 0;
-                for (int e = lane; e < M; e += 32) kept[e] = e;
-                __syncwarp();
-                while (i < len / 2) {
-                    const int ii = i + lane;
-                    bool rj = false;
-                    if (ii < len / 2) {
-                        const int ia = kept[2 * ii], ib = kept[2 * ii + 1];
-                        const double s00 = RA[tri(ia, ia)], s11 = RA[tri(ib, ib)], s10 = ib > ia ? RA[tri(ib, ia)] : RA[tri(ia, ib)];
-                        const double det = s00 * s11 - s10 * s10;
-                        const double v0 = nu[ia], v1 = nu[ib];
-                        const double m2 = (v0 * (s11 * v0 - s10 * v1) + v1 * (s00 * v1 - s10 * v0)) / det;
-                        rj = !(m2 < 5.99);
-                    }
-                    const unsigned bal = __ballot_sync(0xffffffffu, rj);
-                    if (!bal) {
-                        i += 32;
-                        continue;
-                    }
-                    i += __ffs(bal) - 1;
-                    len = gate_remove_pair(kept, len, i, lane);
-                    ++out;
-                }
-                if (lane == 0) { flags[1] = len; flags[2] = out; }
+                const int2 g = gate_scan(kept, M, lane, [=](int ii) { return m2_pair_S(RA, nu, kept[2 * ii], kept[2 * ii + 1]); });
+                if (lane == 0) { flags[1] = g.x; flags[2] = g.y; }
             }
         }
         __syncthreads();
@@ -693,9 +677,7 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_update_kernel(slb::FilterArgs a
         if (mk < M) {
             // compact S -> region B (Z is dead), covXZ in place (kept[] is increasing, kept[p] >= p)
             for (int e = tid; e < mk * (mk + 1) / 2; e += MS_T) {
-                int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-                r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
-                const int c = e - tri(r, 0);
+                const int r = tri_row(e), c = e - tri(r, 0);
                 RB[e] = RA[tri(kept[r], kept[c])];
             }
             // a warp per row of covXZ: the row is gathered into registers before it is overwritten (m <= 128 = 4 per lane)
@@ -748,32 +730,9 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_update_kernel(slb::FilterArgs a
             if (lane == 0) dl[i] = s;
         }
         MS_PH(11);
-        // ---- P_new = Pk - Y Y^T (:262) into region A from the HBM record: lower 8x8 tiles, K = mk ------------
+        // ---- P_new = Pk - Y Y^T (:262) into region A from the HBM record, K = mk ------------------------------------
         __syncthreads();
-        {
-            const int ntiles = nrt * (nrt + 1) / 2;
-            for (int t = warp; t < ntiles; t += MS_W) {
-                int tr, tc;
-                tri_tile(t, tr, tc);
-                const int ai = 8 * tr + fr;
-                const double *pa = Xz + min(ai, N - 1) * MS_ZS + fk, *pb = Xz + min(8 * tc + fr, N - 1) * MS_ZS + fk;
-                double d0 = 0.0, d1 = 0.0;
-                const int r = ai, c = 8 * tc + 2 * fk;
-                // the record's entries are requested before the k-loop so that their L2 latency hides behind it
-                const double g0 = (r < N && c <= r) ? Pg[tri(r, c)] : 0.0, g1 = (r < N && c + 1 <= r) ? Pg[tri(r, c + 1)] : 0.0;
-                const int kfull = mk & ~3;   // mk is even: at most one ragged k-step
-#pragma unroll 4
-                for (int k0 = 0; k0 < kfull; k0 += 4) dmma884(d0, d1, pa[k0], pb[k0]);
-                if (kfull < mk) {
-                    const bool in = kfull + fk < mk;
-                    dmma884(d0, d1, in ? pa[kfull] : 0.0, in ? pb[kfull] : 0.0);
-                }
-                if (r < N) {
-                    if (c <= r) RA[tri(r, c)] = g0 - d0;
-                    if (c + 1 <= r) RA[tri(r, c + 1)] = g1 - d1;
-                }
-            }
-        }
+        sub_yyt(Xz, MS_ZS, N, mk, Pg, RA);
         cp_async_wait_all();
         __syncthreads();
         MS_PH(12);
@@ -995,7 +954,6 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_ekf_update_kernel(slb::FilterAr
     const int fr = lane >> 2, fk = lane & 3;
     const int k = a.k, N = 12 + 6 * k, QD = 13 + 7 * k, M = a.m, NF = M / 2, NB = 4 + 2 * k;
     const int NP = N * (N + 1) / 2;
-    const int nrt = (N + 7) >> 3;
     auto Psym = [&](int i, int j) { return i >= j ? RA[tri(i, j)] : RA[tri(j, i)]; };
     constexpr int QP = ME_QP;
 
@@ -1081,9 +1039,7 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_ekf_update_kernel(slb::FilterAr
             }
             __syncthreads();
             for (int e = tid; e < M * (M + 1) / 2; e += MS_T) {
-                int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-                r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
-                const int c = e - tri(r, 0);
+                const int r = tri_row(e), c = e - tri(r, 0);
                 const int a1 = 12 + 6 * ((c >> 1) % k);
                 double sacc = __ldg(a.R + r * M + c);
 #pragma unroll
@@ -1121,35 +1077,15 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_ekf_update_kernel(slb::FilterAr
                 }
                 if (part == 0 && f < NF) {
                     info[3 * f] = i00; info[3 * f + 1] = i10; info[3 * f + 2] = i11;
-                    const double v0 = nu[ia], v1 = nu[ib];
-                    const double m2 = v0 * (i00 * v0 + i10 * v1) + v1 * (i10 * v0 + i11 * v1);
-                    rej = !(m2 < 5.99);
+                    rej = !chi2_accept(m2_pair_info(i00, i10, i11, nu[ia], nu[ib]), 2);
                 }
             }
             // while nothing is rejected the sequential scan keeps the identity indexing: "all accepted" needs no scan
             if (__syncthreads_or(rej) && warp == 0) {
-                int len = M, out = 0, i = 0;
-                for (int e = lane; e < M; e += 32) kept[e] = e;
-                __syncwarp();
-                while (i < len / 2) {  // 32 scan positions per round, the first rejection is applied (see the UKF flavour)
-                    const int ii = i + lane;
-                    bool rj = false;
-                    if (ii < len / 2) {
-                        const double v0 = nu[kept[2 * ii]], v1 = nu[kept[2 * ii + 1]];
-                        const double i00 = info[3 * ii], i10 = info[3 * ii + 1], i11 = info[3 * ii + 2];  // position, not feature (:773)
-                        const double m2 = v0 * (i00 * v0 + i10 * v1) + v1 * (i10 * v0 + i11 * v1);
-                        rj = !(m2 < 5.99);
-                    }
-                    const unsigned bal = __ballot_sync(0xffffffffu, rj);
-                    if (!bal) {
-                        i += 32;
-                        continue;
-                    }
-                    i += __ffs(bal) - 1;
-                    len = gate_remove_pair(kept, len, i, lane);  // removeRow(2i); removeRow(2i+1): not re-based (Q6)
-                    ++out;
-                }
-                if (lane == 0) { flags[1] = len; flags[2] = out; }
+                const int2 g = gate_scan(kept, M, lane, [=](int ii) {   // info by position, not by feature (:773)
+                    return m2_pair_info(info[3 * ii], info[3 * ii + 1], info[3 * ii + 2], nu[kept[2 * ii]], nu[kept[2 * ii + 1]]);
+                });
+                if (lane == 0) { flags[1] = g.x; flags[2] = g.y; }
             }
             __syncthreads();
             mk = flags[1];
@@ -1204,9 +1140,7 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_ekf_update_kernel(slb::FilterAr
             if (compact || !a.gate) {
                 // S' = Hc covXZ' + R' (packed lower) and its Cholesky factor; otherwise RS still holds chol(S) from the gate
                 for (int e = tid; e < mk * (mk + 1) / 2; e += MS_T) {
-                    int pr = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-                    pr += (tri(pr + 1, 0) <= e) - (tri(pr, 0) > e);
-                    const int pc = e - tri(pr, 0);
+                    const int pr = tri_row(e), pc = e - tri(pr, 0);
                     const int rr = compact ? kept[pr] : pr, rc = compact ? kept[pc] : pc;
                     const int a0 = 12 + 6 * ((rr >> 1) % k);
                     double sacc = __ldg(a.R + (size_t)rr * M + rc);
@@ -1363,9 +1297,7 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_ekf_update_kernel(slb::FilterAr
             if (tid < mk) wv[tid] = __ldg(a.R + (size_t)(compact ? kept[tid] : tid) * (M + 1));
             __syncthreads();
             for (int e = tid; e < NP; e += MS_T) {
-                int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-                r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
-                const int c = e - tri(r, 0);
+                const int r = tri_row(e), c = e - tri(r, 0);
                 double s0 = 0.0, s1 = 0.0;
                 int i = 0;
                 for (; i + 1 < mk; i += 2) {
@@ -1407,9 +1339,7 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_ekf_update_kernel(slb::FilterAr
         __syncthreads();
         // ---- S = Hr covXZ + Rr (:330), packed lower in RS ---------------------------------------------------------
         for (int e = tid; e < NP; e += MS_T) {
-            int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-            r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
-            const int c = e - tri(r, 0);
+            const int r = tri_row(e), c = e - tri(r, 0);
             double sacc = RS[e];
             for (int l = r; l < N; ++l) sacc = fma(RQ[r * ME_HS + l], RH[l * ME_HS + c], sacc);
             RS[e] = sacc;
@@ -1471,29 +1401,8 @@ __global__ void __launch_bounds__(MS_T, 1) msckf_ekf_update_kernel(slb::FilterAr
             sacc = warp_sum(sacc);
             if (lane == 0) dl[i] = sacc;
         }
-        // ---- Pk -= K S K^T = Y Y^T (:336) straight to the HBM record: lower 8x8 tiles, K = mq ----------------------
-        {
-            const int ntiles = nrt * (nrt + 1) / 2;
-            for (int t = warp; t < ntiles; t += MS_W) {
-                int tr, tc;
-                tri_tile(t, tr, tc);
-                const int ai = 8 * tr + fr;
-                const double *pa = Yb + min(ai, N - 1) * ys + fk, *pb = Yb + min(8 * tc + fr, N - 1) * ys + fk;
-                double d0 = 0.0, d1 = 0.0;
-                const int kfull = mq & ~3;   // mq is even: at most one ragged k-step
-#pragma unroll 4
-                for (int k0 = 0; k0 < kfull; k0 += 4) dmma884(d0, d1, pa[k0], pb[k0]);
-                if (kfull < mq) {
-                    const bool in = kfull + fk < mq;
-                    dmma884(d0, d1, in ? pa[kfull] : 0.0, in ? pb[kfull] : 0.0);
-                }
-                const int r = ai, c = 8 * tc + 2 * fk;
-                if (r < N) {
-                    if (c <= r) Pg[tri(r, c)] = RA[tri(r, c)] - d0;
-                    if (c + 1 <= r) Pg[tri(r, c + 1)] = RA[tri(r, c + 1)] - d1;
-                }
-            }
-        }
+        // ---- Pk -= K S K^T = Y Y^T (:336) straight to the HBM record, K = mq ----------------------------------------
+        sub_yyt(Yb, ys, N, mq, RA, Pg);
         __syncthreads();
         // ---- mu = mu [+] K nu (:337), thread per block --------------------------------------------------------------
         bool finite = true;

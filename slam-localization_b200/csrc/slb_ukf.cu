@@ -293,8 +293,7 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
         }
         if (PRED && !PIN) {
             for (int e = lane; e < NP; e += 32) {
-                int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);  // packed index -> (r, c), exact for e < 2^20
-                r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
+                const int r = tri_row(e);
                 Qp[e] = __ldg(a.Q + r * N + (e - tri(r, 0)));
             }
         }
@@ -350,8 +349,7 @@ __global__ void __launch_bounds__(TPB, MINB) ukf_kernel(slb::FilterArgs a) {
 #pragma unroll
             for (int k = 0; k < QK; ++k) {
                 const int e = sub + G * k;
-                int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-                r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
+                const int r = tri_row(e);
                 qreg[k] = e < NP ? __ldg(Qi + r * N + (e - tri(r, 0))) : 0.0;
             }
         }

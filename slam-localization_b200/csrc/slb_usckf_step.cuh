@@ -586,8 +586,7 @@ __global__ void __launch_bounds__(WPB * 32, MINB) usckf_step_kernel(slb::FilterA
     if (PIN && UPD) {   // lower triangle of this instance's R, packed (Rs[tri(r, c)])
         const double *Ri = a.R + (size_t)inst * a.rs;
         for (int e = lane; e < NK * (NK + 1) / 2; e += 32) {
-            int r = (int)((sqrtf(8.0f * e + 1.0f) - 1.0f) * 0.5f);
-            r += (tri(r + 1, 0) <= e) - (tri(r, 0) > e);
+            const int r = tri_row(e);
             cp_async8(Rs + e, Ri + r * NK + (e - tri(r, 0)));
         }
         cp_async_commit();
