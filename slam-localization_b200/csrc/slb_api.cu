@@ -25,6 +25,15 @@ int set_error(int code, const char *what, cudaError_t ce) {
     return code;
 }
 void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
+int need_device(const char *msg, int *ndev) {
+    int n = 0;
+    if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) {
+        cudaGetLastError();
+        return set_error(SLB_ERR_NO_DEVICE, msg);
+    }
+    if (ndev) *ndev = n;
+    return SLB_OK;
+}
 
 // ---- layout conversion kernels: dense instance-major host arrays <-> the batch (h->L) ---------------------------
 // Means: thread t = (instance, scalar), scalar fastest.  mu_in stores instances [b0, b0 + cnt); mu_out loads the slice
@@ -258,10 +267,7 @@ int slb_create(const slb_config *cfg, slb_handle *out) {
     if (!cfg || !out) return set_error(SLB_ERR_INVALID, "slb_create: null argument");
     *out = nullptr;
     int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return set_error(SLB_ERR_NO_DEVICE, "slb_create: no CUDA device (this engine has no CPU fallback)");
-    }
+    if (need_device("slb_create: no CUDA device (this engine has no CPU fallback)", &ndev) != SLB_OK) return SLB_ERR_NO_DEVICE;
     if (cfg->device < 0 || cfg->device >= ndev) return set_error(SLB_ERR_INVALID, "slb_create: bad device ordinal");
     if (cfg->batch <= 0) return set_error(SLB_ERR_INVALID, "slb_create: batch must be positive");
     DeviceGuard guard(cfg->device);  // no lasting side effect on the caller's current device
@@ -292,6 +298,8 @@ int slb_create(const slb_config *cfg, slb_handle *out) {
     h->B = cfg->batch;
     h->L = batch_layout(cfg->kind, cfg->layout, cfg->nk, cfg->nl, cfg->nclones, cfg->batch);
     const slbd::BatchLayout &L = h->L;
+    h->nq = cfg->kind == SLB_KIND_UKF ? L.N : 12;
+    h->m = cfg->kind == SLB_KIND_UKF ? 3 : cfg->kind == SLB_KIND_USCKF ? cfg->nk : 0;
     h->out_off = 0;
     h->out_len = L.QD;
     const size_t mu_bytes = L.mu_size(h->B) * 8, P_bytes = L.P_size(h->B) * 8;
@@ -377,8 +385,8 @@ int slb_set_nis_capture(slb_handle h, int on) {
     SLB_CUDA(cudaMemset(h->nis, 0xff, (size_t)h->B * 8));   // all-ones bytes: a NaN in every entry
     return SLB_OK;
 }
-// doubles between consecutive instances' Q / R for a handle's noise layout (0 = shared)
-static int q_stride(slb_handle h, int n) { return (h->noise & SLB_NOISE_Q_PER_INSTANCE) ? n * n : 0; }
+// doubles between consecutive instances' Q / R (R m x m) for a handle's noise layout (0 = shared)
+static int q_stride(slb_handle h) { return (h->noise & SLB_NOISE_Q_PER_INSTANCE) ? h->nq * h->nq : 0; }
 static int r_stride(slb_handle h, int m) { return (h->noise & SLB_NOISE_R_PER_INSTANCE) ? m * m : 0; }
 int slb_dof(slb_handle h) { return h ? h->L.N : SLB_ERR_INVALID; }
 int slb_qdim(slb_handle h) { return h ? h->L.QD : SLB_ERR_INVALID; }
@@ -474,27 +482,105 @@ int slb_replicate(slb_handle h, int count, void *stream) {
     return SLB_OK;
 }
 
-// ---- ukfom::ukf --------------------------------------------------------------------------------------
-static int ukf_call(slb_handle h, int pm, int mm, bool pred, bool upd, const double *u, double dt, const double *Q,
-                    const double *z, const double *R, int gate, void *stream) {
-    if (!h || h->cfg.kind != SLB_KIND_UKF) return set_error(SLB_ERR_INVALID, "slb_ukf_*: handle is not a UKF batch");
-    if (pred && (!u || !Q)) return set_error(SLB_ERR_INVALID, "slb_ukf_predict: u and Q are required");
-    if (upd && (!z || !R)) return set_error(SLB_ERR_INVALID, "slb_ukf_update: z and R are required");
+// ---- filters: every predict / update / step goes entry point -> filter_call or step_host_entry -> launch_filter ------
+// The one map from a batch kind to its launchers.  An MSCKF step is its predict, then its update.
+static int launch_filter(slb_handle h, int pm, int mm, bool pred, bool upd, const FilterArgs &a, cudaStream_t s) {
+    switch (h->cfg.kind) {
+        case SLB_KIND_UKF: return launch_ukf(h->cfg.layout, pm, mm, pred, upd, a, s);
+        case SLB_KIND_USCKF: return launch_usckf(pm, mm, pred, upd, a, s);
+        default: {
+            const int rc = pred ? launch_msckf_predict(pm, a, s) : SLB_OK;
+            return rc != SLB_OK || !upd ? rc : launch_msckf_update(mm, a, s);
+        }
+    }
+}
+
+// A device entry point: the kind it serves and its refusals of a handle of another kind, of a predict without u / Q
+// and of an update without its inputs (the messages name the entry point)
+struct FilterEntry {
+    int kind;
+    const char *not_kind, *no_pred, *no_upd;
+};
+static const FilterEntry UKF_CALL = {SLB_KIND_UKF, "slb_ukf_*: handle is not a UKF batch",
+                                     "slb_ukf_predict: u and Q are required", "slb_ukf_update: z and R are required"};
+static const FilterEntry USCKF_CALL = {SLB_KIND_USCKF, "slb_usckf_*: handle is not a USCKF batch",
+                                       "slb_usckf_predict: u and Q are required", "slb_usckf_update: z and R are required"};
+static const FilterEntry MSCKF_PREDICT = {SLB_KIND_MSCKF, "slb_msckf_predict: handle is not an MSCKF batch",
+                                          "slb_msckf_predict: u and Q are required", nullptr};
+static const FilterEntry MSCKF_UPDATE = {SLB_KIND_MSCKF, "slb_msckf_update: handle is not an MSCKF batch", nullptr,
+                                         "slb_msckf_update: bad arguments"};
+
+// The device-resident predict / update / step of every kind.  An MSCKF update also takes the landmarks (params) and its
+// measurement dimension m, which the batch does not fix: stacked 2-D reprojections, so m is even.
+static int filter_call(slb_handle h, const FilterEntry &e, int pm, int mm, bool pred, bool upd, const double *u, double dt,
+                       const double *Q, const double *params, int m, const double *z, const double *R, int gate, void *stream) {
+    if (!h || h->cfg.kind != e.kind) return set_error(SLB_ERR_INVALID, e.not_kind);
+    if (pred && (!u || !Q)) return set_error(SLB_ERR_INVALID, e.no_pred);
+    if (upd && (!z || !R || (e.kind == SLB_KIND_MSCKF && (!params || m <= 0 || (m & 1)))))
+        return set_error(SLB_ERR_INVALID, e.no_upd);
     DeviceGuard guard(h->cfg.device);
     FilterArgs a = make_args(h);
-    a.u = u; a.dt = dt; a.Q = Q; a.z = z; a.R = R; a.gate = gate; a.m = 3;
-    a.qs = q_stride(h, h->L.N); a.rs = r_stride(h, 3);
-    return launch_ukf(h->cfg.layout, pm, mm, pred, upd, a, S(stream));
+    a.u = u; a.dt = dt; a.Q = Q; a.params = params; a.z = z; a.R = R; a.gate = gate; a.m = h->m ? h->m : m;
+    a.qs = q_stride(h); a.rs = r_stride(h, a.m);
+    return launch_filter(h, pm, mm, pred, upd, a, S(stream));
 }
+
+// ukfom::ukf
 int slb_ukf_predict(slb_handle h, int pm, const double *u, double dt, const double *Q, void *stream) {
-    return ukf_call(h, pm, 0, true, false, u, dt, Q, nullptr, nullptr, 0, stream);
+    return filter_call(h, UKF_CALL, pm, 0, true, false, u, dt, Q, nullptr, 0, nullptr, nullptr, 0, stream);
 }
 int slb_ukf_update(slb_handle h, int mm, const double *z, const double *R, int gate_dof, void *stream) {
-    return ukf_call(h, 0, mm, false, true, nullptr, 0.0, nullptr, z, R, gate_dof, stream);
+    return filter_call(h, UKF_CALL, 0, mm, false, true, nullptr, 0.0, nullptr, nullptr, 0, z, R, gate_dof, stream);
 }
 int slb_ukf_step(slb_handle h, int pm, int mm, const double *u, double dt, const double *Q, const double *z,
                  const double *R, int gate_dof, void *stream) {
-    return ukf_call(h, pm, mm, true, true, u, dt, Q, z, R, gate_dof, stream);
+    return filter_call(h, UKF_CALL, pm, mm, true, true, u, dt, Q, nullptr, 0, z, R, gate_dof, stream);
+}
+
+// localization::Usckf
+int slb_usckf_predict(slb_handle h, int pm, const double *u, double dt, const double *Q, void *stream) {
+    return filter_call(h, USCKF_CALL, pm, 0, true, false, u, dt, Q, nullptr, 0, nullptr, nullptr, 0, stream);
+}
+int slb_usckf_update(slb_handle h, int mm, const double *z, const double *R, int gate_dof, void *stream) {
+    return filter_call(h, USCKF_CALL, 0, mm, false, true, nullptr, 0.0, nullptr, nullptr, 0, z, R, gate_dof, stream);
+}
+int slb_usckf_step(slb_handle h, int pm, int mm, const double *u, double dt, const double *Q, const double *z,
+                   const double *R, int gate_dof, void *stream) {
+    return filter_call(h, USCKF_CALL, pm, mm, true, true, u, dt, Q, nullptr, 0, z, R, gate_dof, stream);
+}
+int slb_usckf_clone(slb_handle h, int mode, void *stream) {
+    if (!h || h->cfg.kind != SLB_KIND_USCKF) return set_error(SLB_ERR_INVALID, "slb_usckf_clone: handle is not a USCKF batch");
+    DeviceGuard guard(h->cfg.device);
+    FilterArgs a = make_args(h);
+    return launch_usckf_clone(mode, a, S(stream));
+}
+int slb_usckf_set_measurement(slb_handle h, int mode, const double *z, const double *R, void *stream) {
+    if (!h || h->cfg.kind != SLB_KIND_USCKF) return set_error(SLB_ERR_INVALID, "slb_usckf_set_measurement: handle is not a USCKF batch");
+    if (!z || !R) return set_error(SLB_ERR_INVALID, "slb_usckf_set_measurement: z and R are required");
+    DeviceGuard guard(h->cfg.device);
+    FilterArgs a = make_args(h);
+    a.z = z; a.R = R;
+    a.rs = r_stride(h, mode == SLB_STATEK ? h->cfg.nk : h->cfg.nl);
+    return launch_usckf_set_measurement(mode, a, S(stream));
+}
+
+// localization::Msckf
+int slb_msckf_predict(slb_handle h, int pm, const double *u, double dt, const double *Q, void *stream) {
+    return filter_call(h, MSCKF_PREDICT, pm, 0, true, false, u, dt, Q, nullptr, 0, nullptr, nullptr, 0, stream);
+}
+int slb_msckf_update(slb_handle h, int mm, const double *params, int m, const double *z, const double *R, int gate,
+                     void *stream) {
+    return filter_call(h, MSCKF_UPDATE, 0, mm, false, true, nullptr, 0.0, nullptr, params, m, z, R, gate, stream);
+}
+// the EKF-flavoured update is a kernel of its own, not a step of the batch's filter
+int slb_msckf_update_ekf(slb_handle h, int mm, const double *params, int m, const double *z, const double *R, int gate,
+                         void *stream) {
+    if (!h || h->cfg.kind != SLB_KIND_MSCKF) return set_error(SLB_ERR_INVALID, "slb_msckf_update_ekf: handle is not an MSCKF batch");
+    if (!params || !z || !R || m <= 0 || (m & 1)) return set_error(SLB_ERR_INVALID, "slb_msckf_update_ekf: bad arguments");
+    DeviceGuard guard(h->cfg.device);
+    FilterArgs a = make_args(h);
+    a.params = params; a.m = m; a.z = z; a.R = R; a.gate = gate;
+    return launch_msckf_update_ekf(mm, a, S(stream));
 }
 
 // Shared host-buffer step: the batch is cut into chunks that travel on a small ring of internal streams, so
@@ -518,14 +604,7 @@ static int launch_chunk(slb_handle h, const HostStep &hs, int b0, int cnt, const
     if (a.nis) a.nis += b0;
     a.B = cnt;
     a.u = du; a.dt = hs.dt; a.Q = dQ; a.z = dz; a.R = dR; a.params = dp; a.gate = hs.gate; a.m = hs.m;
-    switch (h->cfg.kind) {
-        case SLB_KIND_UKF: return launch_ukf(h->cfg.layout, hs.pm, hs.mm, true, true, a, st);
-        case SLB_KIND_USCKF: return launch_usckf(hs.pm, hs.mm, true, true, a, st);
-        default: {
-            int rc = launch_msckf_predict(hs.pm, a, st);
-            return rc != SLB_OK ? rc : launch_msckf_update(hs.mm, a, st);
-        }
-    }
+    return launch_filter(h, hs.pm, hs.mm, true, true, a, st);
 }
 
 // Enqueues one predict+update step with host buffers on `s` (and the chunk ring forked from it): no synchronisation.
@@ -643,8 +722,7 @@ static int step_host(slb_handle h, const HostStep &hs, void *stream, bool wait =
         FilterArgs a = make_args(h);
         a.u = zu; a.dt = hs.dt; a.Q = dQ; a.z = zz; a.R = dR; a.gate = hs.gate; a.m = hs.m;
         a.mu_out = zmu;
-        const int rc = h->cfg.kind == SLB_KIND_UKF ? launch_ukf(h->cfg.layout, hs.pm, hs.mm, true, true, a, s)
-                                                   : launch_usckf(hs.pm, hs.mm, true, true, a, s);
+        const int rc = launch_filter(h, hs.pm, hs.mm, true, true, a, s);
         if (rc != SLB_OK) return rc;
         if (wait) SLB_CUDA(cudaStreamSynchronize(s));
         return SLB_OK;
@@ -685,21 +763,59 @@ static int step_host(slb_handle h, const HostStep &hs, void *stream, bool wait =
     if (wait) SLB_CUDA(cudaStreamSynchronize(s));
     return SLB_OK;
 }
-static int ukf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
-                         const double *z_host, const double *R_host, int gate_dof, double *mu_out_host, void *stream, bool wait) {
-    if (!h || h->cfg.kind != SLB_KIND_UKF) return set_error(SLB_ERR_INVALID, "slb_ukf_step_host: handle is not a UKF batch");
-    if (h->noise) return set_error(SLB_ERR_INVALID, "slb_ukf_step_host: per-instance noise (slb_set_noise_layout) is device-resident only");
-    if (mm != SLB_MM_GPS_POS) return set_error(SLB_ERR_INVALID, "ukf: unsupported measurement model");
-    const HostStep hs = {pm, mm, pm_nu(pm), 3, h->L.N, 0, gate_dof, dt, u_host, Q_host, nullptr, z_host, R_host, mu_out_host};
+// A *_step_host entry point: the kind it serves and its refusals of a handle of another kind and of per-instance noise
+struct HostEntry {
+    int kind;
+    const char *not_kind, *noise;
+};
+static const HostEntry UKF_HOST = {SLB_KIND_UKF, "slb_ukf_step_host: handle is not a UKF batch",
+                                   "slb_ukf_step_host: per-instance noise (slb_set_noise_layout) is device-resident only"};
+static const HostEntry USCKF_HOST = {SLB_KIND_USCKF, "slb_usckf_step_host: handle is not a USCKF batch",
+                                     "slb_usckf_step_host: per-instance noise (slb_set_noise_layout) is device-resident only"};
+static const HostEntry MSCKF_HOST = {SLB_KIND_MSCKF, "slb_msckf_step_host: handle is not an MSCKF batch",
+                                     "slb_msckf_step_host: per-instance noise (slb_set_noise_layout) is device-resident only"};
+
+// predict + update with HOST buffers (the end-to-end arm of bench.py) for every kind: u | z staged on the device, the
+// posterior means copied back.  Q, R and, for an MSCKF, the landmark parameters are small shared inputs.
+static int step_host_entry(slb_handle h, const HostEntry &e, int pm, int mm, const double *u, double dt, const double *Q,
+                           const double *params, int nparams, int m, const double *z, const double *R, int gate,
+                           double *mu_out, void *stream, bool wait) {
+    if (!h || h->cfg.kind != e.kind) return set_error(SLB_ERR_INVALID, e.not_kind);
+    if (h->noise) return set_error(SLB_ERR_INVALID, e.noise);
+    if (e.kind == SLB_KIND_UKF && mm != SLB_MM_GPS_POS) return set_error(SLB_ERR_INVALID, "ukf: unsupported measurement model");
+    if (e.kind == SLB_KIND_MSCKF) {
+        if (!u || !Q || !params || !z || !R || m <= 0 || nparams <= 0)
+            return set_error(SLB_ERR_INVALID, "slb_msckf_step_host: null argument");
+        if (mm != SLB_MM_MSCKF_REPROJ || (m & 1)) return set_error(SLB_ERR_INVALID, "slb_msckf_step_host: bad measurement model / m");
+    }
+    const HostStep hs = {pm, mm, pm_nu(pm), h->m ? h->m : m, h->nq, nparams, gate, dt, u, Q, params, z, R, mu_out};
     return step_host(h, hs, stream, wait);
 }
 int slb_ukf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
                       const double *z_host, const double *R_host, int gate_dof, double *mu_out_host, void *stream) {
-    return ukf_step_host(h, pm, mm, u_host, dt, Q_host, z_host, R_host, gate_dof, mu_out_host, stream, true);
+    return step_host_entry(h, UKF_HOST, pm, mm, u_host, dt, Q_host, nullptr, 0, 0, z_host, R_host, gate_dof, mu_out_host, stream, true);
 }
 int slb_ukf_step_host_async(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
                             const double *z_host, const double *R_host, int gate_dof, double *mu_out_host, void *stream) {
-    return ukf_step_host(h, pm, mm, u_host, dt, Q_host, z_host, R_host, gate_dof, mu_out_host, stream, false);
+    return step_host_entry(h, UKF_HOST, pm, mm, u_host, dt, Q_host, nullptr, 0, 0, z_host, R_host, gate_dof, mu_out_host, stream, false);
+}
+int slb_usckf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
+                        const double *z_host, const double *R_host, int gate_dof, double *mu_out_host, void *stream) {
+    return step_host_entry(h, USCKF_HOST, pm, mm, u_host, dt, Q_host, nullptr, 0, 0, z_host, R_host, gate_dof, mu_out_host, stream, true);
+}
+int slb_usckf_step_host_async(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
+                              const double *z_host, const double *R_host, int gate_dof, double *mu_out_host, void *stream) {
+    return step_host_entry(h, USCKF_HOST, pm, mm, u_host, dt, Q_host, nullptr, 0, 0, z_host, R_host, gate_dof, mu_out_host, stream, false);
+}
+int slb_msckf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
+                        const double *params_host, int nparams, int m, const double *z_host, const double *R_host,
+                        int gate, double *mu_out_host, void *stream) {
+    return step_host_entry(h, MSCKF_HOST, pm, mm, u_host, dt, Q_host, params_host, nparams, m, z_host, R_host, gate, mu_out_host, stream, true);
+}
+int slb_msckf_step_host_async(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
+                              const double *params_host, int nparams, int m, const double *z_host, const double *R_host,
+                              int gate, double *mu_out_host, void *stream) {
+    return step_host_entry(h, MSCKF_HOST, pm, mm, u_host, dt, Q_host, params_host, nparams, m, z_host, R_host, gate, mu_out_host, stream, false);
 }
 // Completes every step enqueued on `stream` by the *_step_host_async entry points (the host buffers passed to them
 // may be reused / read afterwards).
@@ -708,116 +824,6 @@ int slb_wait(slb_handle h, void *stream) {
     DeviceGuard guard(h->cfg.device);
     SLB_CUDA(cudaStreamSynchronize(S(stream)));
     return SLB_OK;
-}
-
-// ---- localization::Usckf -----------------------------------------------------------------------------
-static int usckf_call(slb_handle h, int pm, int mm, bool pred, bool upd, const double *u, double dt, const double *Q,
-                      const double *z, const double *R, int gate, void *stream) {
-    if (!h || h->cfg.kind != SLB_KIND_USCKF) return set_error(SLB_ERR_INVALID, "slb_usckf_*: handle is not a USCKF batch");
-    if (pred && (!u || !Q)) return set_error(SLB_ERR_INVALID, "slb_usckf_predict: u and Q are required");
-    if (upd && (!z || !R)) return set_error(SLB_ERR_INVALID, "slb_usckf_update: z and R are required");
-    DeviceGuard guard(h->cfg.device);
-    FilterArgs a = make_args(h);
-    a.u = u; a.dt = dt; a.Q = Q; a.z = z; a.R = R; a.gate = gate; a.m = h->cfg.nk;
-    a.qs = q_stride(h, 12); a.rs = r_stride(h, h->cfg.nk);
-    return launch_usckf(pm, mm, pred, upd, a, S(stream));
-}
-int slb_usckf_predict(slb_handle h, int pm, const double *u, double dt, const double *Q, void *stream) {
-    return usckf_call(h, pm, 0, true, false, u, dt, Q, nullptr, nullptr, 0, stream);
-}
-int slb_usckf_update(slb_handle h, int mm, const double *z, const double *R, int gate_dof, void *stream) {
-    return usckf_call(h, 0, mm, false, true, nullptr, 0.0, nullptr, z, R, gate_dof, stream);
-}
-int slb_usckf_step(slb_handle h, int pm, int mm, const double *u, double dt, const double *Q, const double *z,
-                   const double *R, int gate_dof, void *stream) {
-    return usckf_call(h, pm, mm, true, true, u, dt, Q, z, R, gate_dof, stream);
-}
-static int usckf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
-                           const double *z_host, const double *R_host, int gate_dof, double *mu_out_host, void *stream, bool wait) {
-    if (!h || h->cfg.kind != SLB_KIND_USCKF) return set_error(SLB_ERR_INVALID, "slb_usckf_step_host: handle is not a USCKF batch");
-    if (h->noise) return set_error(SLB_ERR_INVALID, "slb_usckf_step_host: per-instance noise (slb_set_noise_layout) is device-resident only");
-    const HostStep hs = {pm, mm, pm_nu(pm), h->cfg.nk, 12, 0, gate_dof, dt, u_host, Q_host, nullptr, z_host, R_host, mu_out_host};
-    return step_host(h, hs, stream, wait);
-}
-int slb_usckf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
-                        const double *z_host, const double *R_host, int gate_dof, double *mu_out_host, void *stream) {
-    return usckf_step_host(h, pm, mm, u_host, dt, Q_host, z_host, R_host, gate_dof, mu_out_host, stream, true);
-}
-int slb_usckf_step_host_async(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
-                              const double *z_host, const double *R_host, int gate_dof, double *mu_out_host, void *stream) {
-    return usckf_step_host(h, pm, mm, u_host, dt, Q_host, z_host, R_host, gate_dof, mu_out_host, stream, false);
-}
-int slb_usckf_clone(slb_handle h, int mode, void *stream) {
-    if (!h || h->cfg.kind != SLB_KIND_USCKF) return set_error(SLB_ERR_INVALID, "slb_usckf_clone: handle is not a USCKF batch");
-    DeviceGuard guard(h->cfg.device);
-    FilterArgs a = make_args(h);
-    return launch_usckf_clone(mode, a, S(stream));
-}
-int slb_usckf_set_measurement(slb_handle h, int mode, const double *z, const double *R, void *stream) {
-    if (!h || h->cfg.kind != SLB_KIND_USCKF) return set_error(SLB_ERR_INVALID, "slb_usckf_set_measurement: handle is not a USCKF batch");
-    if (!z || !R) return set_error(SLB_ERR_INVALID, "slb_usckf_set_measurement: z and R are required");
-    DeviceGuard guard(h->cfg.device);
-    FilterArgs a = make_args(h);
-    a.z = z; a.R = R;
-    a.rs = r_stride(h, mode == SLB_STATEK ? h->cfg.nk : h->cfg.nl);
-    return launch_usckf_set_measurement(mode, a, S(stream));
-}
-
-// ---- localization::Msckf -----------------------------------------------------------------------------
-int slb_msckf_predict(slb_handle h, int pm, const double *u, double dt, const double *Q, void *stream) {
-    if (!h || h->cfg.kind != SLB_KIND_MSCKF) return set_error(SLB_ERR_INVALID, "slb_msckf_predict: handle is not an MSCKF batch");
-    if (!u || !Q) return set_error(SLB_ERR_INVALID, "slb_msckf_predict: u and Q are required");
-    DeviceGuard guard(h->cfg.device);
-    FilterArgs a = make_args(h);
-    a.u = u; a.dt = dt; a.Q = Q;
-    a.qs = q_stride(h, 12);
-    return launch_msckf_predict(pm, a, S(stream));
-}
-int slb_msckf_update(slb_handle h, int mm, const double *params, int m, const double *z, const double *R, int gate,
-                     void *stream) {
-    if (!h || h->cfg.kind != SLB_KIND_MSCKF) return set_error(SLB_ERR_INVALID, "slb_msckf_update: handle is not an MSCKF batch");
-    if (!params || !z || !R || m <= 0 || (m & 1)) return set_error(SLB_ERR_INVALID, "slb_msckf_update: bad arguments");
-    DeviceGuard guard(h->cfg.device);
-    FilterArgs a = make_args(h);
-    a.params = params; a.m = m; a.z = z; a.R = R; a.gate = gate;
-    return launch_msckf_update(mm, a, S(stream));
-}
-
-int slb_msckf_update_ekf(slb_handle h, int mm, const double *params, int m, const double *z, const double *R, int gate,
-                         void *stream) {
-    if (!h || h->cfg.kind != SLB_KIND_MSCKF) return set_error(SLB_ERR_INVALID, "slb_msckf_update_ekf: handle is not an MSCKF batch");
-    if (!params || !z || !R || m <= 0 || (m & 1)) return set_error(SLB_ERR_INVALID, "slb_msckf_update_ekf: bad arguments");
-    DeviceGuard guard(h->cfg.device);
-    FilterArgs a = make_args(h);
-    a.params = params; a.m = m; a.z = z; a.R = R; a.gate = gate;
-    return launch_msckf_update_ekf(mm, a, S(stream));
-}
-
-// predict + update with HOST buffers (the end-to-end arm of bench.py): u | z staged on the device, the
-// posterior means copied back.  Q, R and the landmark parameters are small shared inputs.
-static int msckf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
-                           const double *params_host, int nparams, int m, const double *z_host, const double *R_host,
-                           int gate, double *mu_out_host, void *stream, bool wait);
-int slb_msckf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
-                        const double *params_host, int nparams, int m, const double *z_host, const double *R_host,
-                        int gate, double *mu_out_host, void *stream) {
-    return msckf_step_host(h, pm, mm, u_host, dt, Q_host, params_host, nparams, m, z_host, R_host, gate, mu_out_host, stream, true);
-}
-int slb_msckf_step_host_async(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
-                              const double *params_host, int nparams, int m, const double *z_host, const double *R_host,
-                              int gate, double *mu_out_host, void *stream) {
-    return msckf_step_host(h, pm, mm, u_host, dt, Q_host, params_host, nparams, m, z_host, R_host, gate, mu_out_host, stream, false);
-}
-static int msckf_step_host(slb_handle h, int pm, int mm, const double *u_host, double dt, const double *Q_host,
-                           const double *params_host, int nparams, int m, const double *z_host, const double *R_host,
-                           int gate, double *mu_out_host, void *stream, bool wait) {
-    if (!h || h->cfg.kind != SLB_KIND_MSCKF) return set_error(SLB_ERR_INVALID, "slb_msckf_step_host: handle is not an MSCKF batch");
-    if (h->noise) return set_error(SLB_ERR_INVALID, "slb_msckf_step_host: per-instance noise (slb_set_noise_layout) is device-resident only");
-    if (!u_host || !Q_host || !params_host || !z_host || !R_host || m <= 0 || nparams <= 0)
-        return set_error(SLB_ERR_INVALID, "slb_msckf_step_host: null argument");
-    const HostStep hs = {pm, mm, pm_nu(pm), m, 12, nparams, gate, dt, u_host, Q_host, params_host, z_host, R_host, mu_out_host};
-    if (mm != SLB_MM_MSCKF_REPROJ || (m & 1)) return set_error(SLB_ERR_INVALID, "slb_msckf_step_host: bad measurement model / m");
-    return step_host(h, hs, stream, wait);
 }
 
 // ---- localization::DataModel -------------------------------------------------------------------------
@@ -834,11 +840,7 @@ int slb_datamodel_addsub(int d, int64_t n, int sign, const double *x1, const dou
 int slb_datamodel_fuse_host(int d, int64_t n, const double *x1, const double *C1, const double *x2, const double *C2,
                             double *xo, double *Co) {
     if (!x1 || !C1 || !x2 || !C2 || !xo || !Co || n < 0) return set_error(SLB_ERR_INVALID, "slb_datamodel_fuse_host: bad arguments");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return set_error(SLB_ERR_NO_DEVICE, "slb_datamodel_fuse_host: no CUDA device (no CPU fallback)");
-    }
+    if (need_device("slb_datamodel_fuse_host: no CUDA device (no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
     if (n == 0) return SLB_OK;
     // Page-locked buffers: zero-copy.  The kernel stages its covariance tiles with coalesced LDGSTS and writes its
     // results with coalesced stores, which work just as well against mapped host memory: the 1 GB of H2D / D2H
@@ -876,11 +878,7 @@ int slb_datamodel_fuse_host(int d, int64_t n, const double *x1, const double *C1
 // ---- device buffers ----------------------------------------------------------------------------------
 int slb_dev_alloc(size_t bytes, void **dev) {
     if (!dev) return set_error(SLB_ERR_INVALID, "slb_dev_alloc: null argument");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return set_error(SLB_ERR_NO_DEVICE, "slb_dev_alloc: no CUDA device (this engine has no CPU fallback)");
-    }
+    if (need_device("slb_dev_alloc: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
     SLB_CUDA(cudaMalloc(dev, bytes ? bytes : 8));
     return SLB_OK;
 }
@@ -921,11 +919,7 @@ int slb_clear_status(slb_handle h, void *stream) {
 }
 int slb_bench_fp64_peak(double *tflops_out) {
     if (!tflops_out) return set_error(SLB_ERR_INVALID, "slb_bench_fp64_peak: null argument");
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return set_error(SLB_ERR_NO_DEVICE, "slb_bench_fp64_peak: no CUDA device");
-    }
+    if (need_device("slb_bench_fp64_peak: no CUDA device") != SLB_OK) return SLB_ERR_NO_DEVICE;
     int dev = 0, sms = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);

@@ -553,15 +553,6 @@ __global__ void __launch_bounds__(64) dr_update_pose_kernel(int64_t n, double dt
 
 using namespace slb;
 
-static int need_device(const char *who) {
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return set_error(SLB_ERR_NO_DEVICE, who);
-    }
-    return SLB_OK;
-}
-
 extern "C" {
 
 int slb_datamodel_safe_fuse(int64_t n, const double *x1, const double *C1, const double *x2, const double *C2, double *xo, double *Co,

@@ -407,11 +407,7 @@ extern "C" {
 int slb_ekf_predict(int64_t n, double *err, double *P, const double *F, const double *Q, void *stream) {
     if (n < 0 || !err || !P || !F || !Q) return set_error(SLB_ERR_INVALID, "slb_ekf_predict: bad argument");
     if (n == 0) return SLB_OK;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return set_error(SLB_ERR_NO_DEVICE, "slb_ekf_predict: no CUDA device (this engine has no CPU fallback)");
-    }
+    if (need_device("slb_ekf_predict: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
     constexpr int WPB = 8;
     constexpr size_t smem = (size_t)WPB * slbd::EKP_SM * 8;
     auto kern = slbd::ekf_predict_kernel<WPB>;
@@ -427,11 +423,7 @@ int slb_ekf_update(int64_t n, int m, const double *mu, double *P, const double *
     if (n < 0 || !mu || !P || !z || !H || !R || !ret || !accepted) return set_error(SLB_ERR_INVALID, "slb_ekf_update: bad argument");
     if (m != 3) return set_error(SLB_ERR_INVALID, "slb_ekf_update: built for m = 3 (delay-position / velocity measurements)");
     if (n == 0) return SLB_OK;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return set_error(SLB_ERR_NO_DEVICE, "slb_ekf_update: no CUDA device (this engine has no CPU fallback)");
-    }
+    if (need_device("slb_ekf_update: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
     constexpr int WPB = 8;
     constexpr size_t smem = (size_t)WPB * (slbd::EkuCfg<45, 3>::SM + 46) * 8;
     auto kern = slbd::ekf_update_kernel<3, WPB>;
@@ -447,11 +439,7 @@ int slb_ekf_single_update(int64_t n, int m, double *mu, const double *err, doubl
     if (n < 0 || !mu || !err || !P || !z || !H || !R || !accepted) return set_error(SLB_ERR_INVALID, "slb_ekf_single_update: bad argument");
     if (m != 3) return set_error(SLB_ERR_INVALID, "slb_ekf_single_update: built for m = 3");
     if (n == 0) return SLB_OK;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return set_error(SLB_ERR_NO_DEVICE, "slb_ekf_single_update: no CUDA device (this engine has no CPU fallback)");
-    }
+    if (need_device("slb_ekf_single_update: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
     constexpr int WPB = 8;
     constexpr size_t smem = (size_t)WPB * (slbd::EkuCfg<15, 3>::SM + 16) * 8;
     auto kern = slbd::ekf_single_update_kernel<3, WPB>;
@@ -464,11 +452,7 @@ int slb_ekf_single_update(int64_t n, int m, double *mu, const double *err, doubl
 int slb_ekf_clone(int64_t n, double *mu, double *err, double *P, void *stream) {
     if (n < 0 || !mu || !err || !P) return set_error(SLB_ERR_INVALID, "slb_ekf_clone: bad argument");
     if (n == 0) return SLB_OK;
-    int ndev = 0;
-    if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-        cudaGetLastError();
-        return set_error(SLB_ERR_NO_DEVICE, "slb_ekf_clone: no CUDA device (this engine has no CPU fallback)");
-    }
+    if (need_device("slb_ekf_clone: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
     const int64_t work = n * (45 * 45 + 32 + 30);
     slbd::ekf_clone_kernel<<<(unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n, mu, err, P);
     count_launch();

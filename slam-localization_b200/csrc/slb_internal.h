@@ -17,6 +17,8 @@ struct slb_batch_s {
     slb_config cfg;
     int B;        // instances
     slbd::BatchLayout L;  // dimensions and storage of mu and P
+    // call dimensions of the kind: Q is nq x nq, R m x m (m = 0: MSCKF, whose m comes with each update)
+    int nq, m;
     double *mu;   // L.mu_size(B) doubles
     double *P;    // L.P_size(B) doubles
     int32_t *status;
@@ -50,6 +52,9 @@ namespace slb {
 
 int set_error(int code, const char *what, cudaError_t ce = cudaSuccess);
 void count_launch(int n = 1);
+// SLB_ERR_NO_DEVICE with message `msg` when no CUDA device is visible (there is no CPU fallback), else SLB_OK and the
+// device count in *ndev
+int need_device(const char *msg, int *ndev = nullptr);
 
 #define SLB_CUDA(call)                                                        \
     do {                                                                      \

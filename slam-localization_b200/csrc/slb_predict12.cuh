@@ -466,3 +466,21 @@ __global__ void __launch_bounds__(WPB * 32, 2) predict12_kernel(slb::FilterArgs 
 }
 
 }  // namespace slbd
+
+namespace slb {
+
+// predict12_kernel over a batch, one instance per warp, 8 warps per CTA; per-instance Q (a.qs != 0) selects PIN
+template <int PM, int ROW0, int MU0, bool CROSS>
+int launch_predict12(const FilterArgs &a, cudaStream_t s) {
+    constexpr int WPB = 8;
+    constexpr size_t smem = (size_t)WPB * slbd::PRED_SM * sizeof(double);
+    auto kern = a.qs ? slbd::predict12_kernel<PM, WPB, ROW0, MU0, CROSS, true>
+                     : slbd::predict12_kernel<PM, WPB, ROW0, MU0, CROSS, false>;
+    SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kern<<<(a.B + WPB - 1) / WPB, WPB * 32, smem, s>>>(a);
+    count_launch();
+    SLB_CUDA(cudaGetLastError());
+    return SLB_OK;
+}
+
+}  // namespace slb

@@ -91,18 +91,6 @@ __global__ void usckf_set_measurement_kernel(slb::FilterArgs a, int mode) {
 
 namespace slb {
 
-template <int PM, bool PIN>
-static int launch_predict_t(const FilterArgs &a, cudaStream_t s) {
-    constexpr int WPB = 8;
-    constexpr size_t smem = (size_t)WPB * slbd::PRED_SM * sizeof(double);
-    auto kern = slbd::predict12_kernel<PM, WPB, 24, 26, true, PIN>;
-    SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<(a.B + WPB - 1) / WPB, WPB * 32, smem, s>>>(a);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
-}
-
 // the tiled record layout (prec) places every entry of the lower triangle once inside the N(N+1)/2 doubles of the
 // packed one, and every off-diagonal tile row it holds starts on a 16-byte boundary
 static constexpr bool prec_fills_record(int N) {
@@ -201,7 +189,7 @@ int launch_usckf(int pm, int mm, bool predict, bool update, const FilterArgs &a,
     if (update && mm != SLB_MM_USCKF_VO) return set_error(SLB_ERR_INVALID, "usckf: unsupported measurement model");
     // predict alone touches rows 24..35 of the record only: the partial-record kernel of slb_predict12.cuh
     if (predict && !update)
-        return a.qs ? launch_predict_t<SLB_PM_USCKF_TEST, true>(a, s) : launch_predict_t<SLB_PM_USCKF_TEST, false>(a, s);
+        return launch_predict12<SLB_PM_USCKF_TEST, 24, 26, true>(a, s);
     if (update) {
 #define SLB_USCKF_SHAPE(NK_, NL_) \
     if (a.nk == NK_ && a.nl == NL_) return launch_step_nknl<NK_, NL_>(predict, a, s);
