@@ -25,6 +25,13 @@ int set_error(int code, const char *what, cudaError_t ce) {
     return code;
 }
 void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
+// (a failed query leaves its error to the cudaGetLastError() of the launch that follows)
+int sm_count() {
+    int dev = 0, n = 1;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
+    return n;
+}
 int need_device(const char *msg, int *ndev) {
     int n = 0;
     if (cudaGetDeviceCount(&n) != cudaSuccess || n == 0) {
@@ -443,15 +450,13 @@ static int transfer(slb_handle h, int field, void *host, size_t count, cudaStrea
         const int grid = (int)((work + tpb - 1) / tpb);
         if (up) {
             SLB_CUDA(cudaMemcpyAsync(h->stage, hp + (size_t)b0 * per, bytes, cudaMemcpyHostToDevice, s));
-            if (field == SLB_FIELD_MU) mu_in<<<grid, tpb, 0, s>>>(h->stage, h->mu, L, b0, cnt);
-            else P_in<<<grid, tpb, 0, s>>>(h->stage, h->P, L, b0, cnt);
-            count_launch();
-            SLB_CUDA(cudaGetLastError());
+            const int rc = field == SLB_FIELD_MU ? launch(mu_in, grid, tpb, 0, s, h->stage, h->mu, L, b0, cnt)
+                                                 : launch(P_in, grid, tpb, 0, s, h->stage, h->P, L, b0, cnt);
+            if (rc != SLB_OK) return rc;
         } else {
-            if (field == SLB_FIELD_MU) mu_out<<<grid, tpb, 0, s>>>(h->mu, h->stage, L, b0, cnt, 0, L.QD);
-            else P_out<<<grid, tpb, 0, s>>>(h->P, h->stage, L, b0, cnt);
-            count_launch();
-            SLB_CUDA(cudaGetLastError());
+            const int rc = field == SLB_FIELD_MU ? launch(mu_out, grid, tpb, 0, s, h->mu, h->stage, L, b0, cnt, 0, L.QD)
+                                                 : launch(P_out, grid, tpb, 0, s, h->P, h->stage, L, b0, cnt);
+            if (rc != SLB_OK) return rc;
             SLB_CUDA(cudaMemcpyAsync(hp + (size_t)b0 * per, h->stage, bytes, cudaMemcpyDeviceToHost, s));
         }
         // the staging buffer is reused by the next chunk (and by later calls)
@@ -474,12 +479,10 @@ int slb_replicate(slb_handle h, int count, void *stream) {
     if (count == h->B) return SLB_OK;
     const int tpb = 256;
     int64_t w = (int64_t)h->L.QD * h->B;
-    replicate<<<(unsigned)((w + tpb - 1) / tpb), tpb, 0, s>>>(h->mu, h->L, h->B, count, false);
+    const int rc = launch(replicate, (unsigned)((w + tpb - 1) / tpb), tpb, 0, s, h->mu, h->L, h->B, count, false);
+    if (rc != SLB_OK) return rc;
     w = (int64_t)h->L.NP * h->B;
-    replicate<<<(unsigned)((w + tpb - 1) / tpb), tpb, 0, s>>>(h->P, h->L, h->B, count, true);
-    count_launch(2);
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(replicate, (unsigned)((w + tpb - 1) / tpb), tpb, 0, s, h->P, h->L, h->B, count, true);
 }
 
 // ---- filters: every predict / update / step goes entry point -> filter_call or step_host_entry -> launch_filter ------
@@ -624,10 +627,6 @@ static int step_host_enqueue(slb_handle h, const HostStep &hs, cudaStream_t s) {
     int nchunk = h->cfg.kind == SLB_KIND_UKF ? h->B / 20000 : h->B / 8192;
     const int cmax = h->cfg.kind == SLB_KIND_UKF ? 3 : 8;
     nchunk = nchunk < 1 ? 1 : nchunk > cmax ? cmax : nchunk;
-    {
-        static const int forced = [] { const char *e = getenv("SLB_HOST_CHUNKS"); return e ? atoi(e) : 0; }();
-        if (forced > 0) nchunk = forced;
-    }
     const int per = ((h->B + nchunk - 1) / nchunk + 31) / 32 * 32;
     int used = 0;
     for (int c = 0, b0 = 0; b0 < h->B; ++c, b0 += per) {
@@ -636,14 +635,13 @@ static int step_host_enqueue(slb_handle h, const HostStep &hs, cudaStream_t s) {
         if (c < SLB_NXS) { SLB_CUDA(cudaStreamWaitEvent(st, h->ev_start, 0)); used = c + 1; }
         SLB_CUDA(cudaMemcpyAsync(du + (size_t)b0 * hs.nu, hs.u + (size_t)b0 * hs.nu, (size_t)cnt * hs.nu * 8, cudaMemcpyHostToDevice, st));
         SLB_CUDA(cudaMemcpyAsync(dz + (size_t)b0 * hs.m, hs.z + (size_t)b0 * hs.m, (size_t)cnt * hs.m * 8, cudaMemcpyHostToDevice, st));
-        const int rc = launch_chunk(h, hs, b0, cnt, du + (size_t)b0 * hs.nu, dz + (size_t)b0 * hs.m, dQ, dp, dR, st);
+        int rc = launch_chunk(h, hs, b0, cnt, du + (size_t)b0 * hs.nu, dz + (size_t)b0 * hs.m, dQ, dp, dR, st);
         if (rc != SLB_OK) return rc;
         if (hs.mu_out) {
             const int OL = h->out_len, work = cnt * OL, tpb = 256;
             double *dst = dmu + (size_t)b0 * OL;
-            mu_out<<<(work + tpb - 1) / tpb, tpb, 0, st>>>(h->mu, dst, h->L, b0, cnt, h->out_off, OL);
-            count_launch();
-            SLB_CUDA(cudaGetLastError());
+            rc = launch(mu_out, (work + tpb - 1) / tpb, tpb, 0, st, h->mu, dst, h->L, b0, cnt, h->out_off, OL);
+            if (rc != SLB_OK) return rc;
             SLB_CUDA(cudaMemcpyAsync(hs.mu_out + (size_t)b0 * OL, dst, (size_t)cnt * OL * 8, cudaMemcpyDeviceToHost, st));
         }
     }
@@ -652,6 +650,14 @@ static int step_host_enqueue(slb_handle h, const HostStep &hs, cudaStream_t s) {
         SLB_CUDA(cudaStreamWaitEvent(s, h->ev_done[i], 0));
     }
     return SLB_OK;
+}
+
+// SLB_ZERO_COPY=0 turns the zero-copy branches of the host-buffer entry points off, so that page-locked buffers take
+// the copy pipeline.  For a UKF or USCKF batch that is the only way to run (and test) the captured CUDA graph of that
+// pipeline in step_host.
+static bool zero_copy() {
+    static const bool on = [] { const char *e = getenv("SLB_ZERO_COPY"); return !e || atoi(e) != 0; }();
+    return on;
 }
 
 static bool is_pinned(const void *p) {
@@ -698,11 +704,10 @@ static int step_host(slb_handle h, const HostStep &hs, void *stream, bool wait =
     }
     // UKF: zero-copy.  The step is as short as its PCIe transfers, so instead of staging copies the kernel reads u / z
     // from the mapped (page-locked, UVA) host buffers and writes the posterior means straight back: transfers overlap
-    // compute warp by warp.  Only the small shared Q / R are copied.  (SLB_ZERO_COPY=0 selects the copy pipeline.)
-    static const bool zero_copy = [] { const char *e = getenv("SLB_ZERO_COPY"); return !e || atoi(e) != 0; }();
+    // compute warp by warp.  Only the small shared Q / R are copied.
     const double *zu = dev_alias(hs.u), *zz = dev_alias(hs.z);
     double *zmu = dev_alias_m(hs.mu_out);
-    if (zero_copy && zu && zz && (zmu || !hs.mu_out) && (h->cfg.kind == SLB_KIND_UKF || h->cfg.kind == SLB_KIND_USCKF)) {
+    if (zero_copy() && zu && zz && (zmu || !hs.mu_out) && (h->cfg.kind == SLB_KIND_UKF || h->cfg.kind == SLB_KIND_USCKF)) {
         double *dQ = h->shared_small, *dR = dQ + hs.nq * hs.nq;
         const size_t qb = (size_t)hs.nq * hs.nq * 8, rb = (size_t)hs.m * hs.m * 8;
         const bool cacheable = hs.nq <= 12 && hs.m <= 9;
@@ -846,10 +851,9 @@ int slb_datamodel_fuse_host(int d, int64_t n, const double *x1, const double *C1
     // results with coalesced stores, which work just as well against mapped host memory: the 1 GB of H2D / D2H
     // traffic of a 1M-pair step overlaps in both directions and with the arithmetic, and nothing is allocated.
     {
-        static const bool zero_copy = [] { const char *e = getenv("SLB_ZERO_COPY"); return !e || atoi(e) != 0; }();
         const double *a1 = dev_alias(x1), *A1 = dev_alias(C1), *a2 = dev_alias(x2), *A2 = dev_alias(C2);
         double *ao = dev_alias_m(xo), *Ao = dev_alias_m(Co);
-        if (zero_copy && is_pinned(x1) && is_pinned(C1) && is_pinned(x2) && is_pinned(C2) && is_pinned(xo) && is_pinned(Co) &&
+        if (zero_copy() && is_pinned(x1) && is_pinned(C1) && is_pinned(x2) && is_pinned(C2) && is_pinned(xo) && is_pinned(Co) &&
             a1 && A1 && a2 && A2 && ao && Ao) {
             const int rc = launch_fusion(d, n, 0, a1, A1, a2, A2, ao, Ao, 0);
             if (rc != SLB_OK) return rc;
@@ -900,11 +904,9 @@ int slb_status_ex(slb_handle h, int64_t *counts, int nbits, void *stream) {
     DeviceGuard guard(h->cfg.device);
     cudaStream_t s = S(stream);
     SLB_CUDA(cudaMemsetAsync(h->counts_dev, 0, 8 * sizeof(int64_t), s));
-    int grid = (h->B + 255) / 256;
-    if (grid > 1184) grid = 1184;
-    status_count<<<grid, 256, 0, s>>>(h->status, h->B, (unsigned long long *)h->counts_dev);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
+    const int grid = (h->B + 255) / 256, cap = sm_count() * 8;
+    const int rc = launch(status_count, grid < cap ? grid : cap, 256, 0, s, h->status, h->B, (unsigned long long *)h->counts_dev);
+    if (rc != SLB_OK) return rc;
     SLB_CUDA(cudaMemcpyAsync(counts, h->counts_dev, (size_t)nbits * sizeof(int64_t), cudaMemcpyDeviceToHost, s));
     SLB_CUDA(cudaStreamSynchronize(s));
     return SLB_OK;
@@ -920,15 +922,12 @@ int slb_clear_status(slb_handle h, void *stream) {
 int slb_bench_fp64_peak(double *tflops_out) {
     if (!tflops_out) return set_error(SLB_ERR_INVALID, "slb_bench_fp64_peak: null argument");
     if (need_device("slb_bench_fp64_peak: no CUDA device") != SLB_OK) return SLB_ERR_NO_DEVICE;
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     double *sink = nullptr;
     SLB_CUDA(cudaMalloc(&sink, 8));
     cudaEvent_t e0, e1;
     cudaEventCreate(&e0);
     cudaEventCreate(&e1);
-    const int iters = 4096, grid = sms * 8;
+    const int iters = 4096, grid = sm_count() * 8;
     double best = 0.0;
     for (int rep = 0; rep < 5; ++rep) {
         cudaEventRecord(e0, 0);
@@ -957,12 +956,9 @@ int slb_ensemble_stats(slb_handle h, double *out_dev, void *stream) {
     const int N = h->L.N;
     if (N * N + N > STAT_TPB * STAT_MAXACC) return set_error(SLB_ERR_INVALID, "slb_ensemble_stats: state too large");
     SLB_CUDA(cudaMemsetAsync(out_dev, 0, (size_t)(1 + N + N * N) * 8, s));
-    const int nchunks = (h->B + STAT_CHUNK - 1) / STAT_CHUNK;
-    const int grid = nchunks < 296 ? nchunks : 296;
-    ensemble_stats_kernel<<<grid, STAT_TPB, (size_t)STAT_CHUNK * N * 8, s>>>(h->mu, h->B, h->L, out_dev);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    const int nchunks = (h->B + STAT_CHUNK - 1) / STAT_CHUNK, cap = sm_count() * 2;
+    return launch(ensemble_stats_kernel, nchunks < cap ? nchunks : cap, STAT_TPB, (size_t)STAT_CHUNK * N * 8, s, h->mu, h->B,
+                  h->L, out_dev);
 }
 
 // ---- filter consistency: NEES against a per-instance truth, NIS of the last update --------------------------------

@@ -186,12 +186,8 @@ namespace slb {
 int launch_check_sigma_points(const slb_batch_s *h, int32_t *flags, double *diff, cudaStream_t s) {
     const slbd::BatchLayout &l = h->L;
     const size_t smem = ((size_t)2 * l.NP + 32 * l.N + 2 * l.QD + l.N) * sizeof(double);
-    SLB_CUDA(cudaFuncSetAttribute(slbd::check_sigma_points_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int grid = h->B < 148 * 3 * 8 ? h->B : 148 * 3 * 8;
-    slbd::check_sigma_points_kernel<<<grid, 32, smem, s>>>(h->mu, h->P, h->B, l, flags, diff);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    const int cap = sm_count() * 24;
+    return launch(slbd::check_sigma_points_kernel, h->B < cap ? h->B : cap, 32, smem, s, h->mu, h->P, h->B, l, flags, diff);
 }
 
 }  // namespace slb

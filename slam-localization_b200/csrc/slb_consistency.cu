@@ -107,17 +107,13 @@ namespace slb {
 int launch_consistency(const slb_batch_s *h, const double *truth, int t0, int n, double *nees, double *out, cudaStream_t s) {
     const size_t smem = truth ? (size_t)slbd::CONS_WPB * (((n + 1) * (n + 2) / 2 + 1) / 2 * 2) * sizeof(double) : 0;
     auto kern = slbd::consistency_kernel;
-    SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int dev = 0, sms = 148, per_sm = 1;
-    SLB_CUDA(cudaGetDevice(&dev));
-    SLB_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+    if (allow_smem(kern, smem) != SLB_OK) return SLB_ERR_CUDA;   // before the occupancy query, which judges by it
+    int per_sm = 1;
     SLB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, slbd::CONS_WPB * 32, smem));
     const int need = (h->B + slbd::CONS_WPB - 1) / slbd::CONS_WPB;
-    const int cap = sms * (per_sm < 1 ? 1 : per_sm);
-    kern<<<need < cap ? need : cap, slbd::CONS_WPB * 32, smem, s>>>(h->mu, h->P, h->nis, h->B, h->L, truth, t0, n, nees, out);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    const int cap = sm_count() * (per_sm < 1 ? 1 : per_sm);
+    return launch(kern, need < cap ? need : cap, slbd::CONS_WPB * 32, smem, s, h->mu, h->P, h->nis, h->B, h->L, truth, t0, n,
+                  nees, out);
 }
 
 }  // namespace slb

@@ -560,10 +560,7 @@ int slb_datamodel_safe_fuse(int64_t n, const double *x1, const double *C1, const
     if (n < 0 || !x1 || !C1 || !x2 || !C2 || !xo || !Co) return set_error(SLB_ERR_INVALID, "slb_datamodel_safe_fuse: bad argument");
     if (n == 0) return SLB_OK;
     if (need_device("slb_datamodel_safe_fuse: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
-    slbd::safe_fusion_kernel<<<(unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream>>>(n, x1, C1, x2, C2, xo, Co);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(slbd::safe_fusion_kernel, (unsigned)((n + 127) / 128), 128, 0, (cudaStream_t)stream, n, x1, C1, x2, C2, xo, Co);
 }
 
 int slb_transform_compose(int64_t n, const double *pose2, const double *cov2, const double *pose1, const double *cov1, double *pose_out,
@@ -572,10 +569,8 @@ int slb_transform_compose(int64_t n, const double *pose2, const double *cov2, co
         return set_error(SLB_ERR_INVALID, "slb_transform_compose: bad argument");
     if (n == 0) return SLB_OK;
     if (need_device("slb_transform_compose: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
-    slbd::transform_compose_kernel<<<(unsigned)((n + 63) / 64), 64, 0, (cudaStream_t)stream>>>(n, pose2, cov2, pose1, cov1, pose_out, cov_out);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(slbd::transform_compose_kernel, (unsigned)((n + 63) / 64), 64, 0, (cudaStream_t)stream, n, pose2, cov2, pose1,
+                  cov1, pose_out, cov_out);
 }
 
 int slb_deadreckon_update_pose(int64_t n, double dt, const double *vel0, const double *vel1, const double *velcov, const double *prev_pose,
@@ -585,11 +580,8 @@ int slb_deadreckon_update_pose(int64_t n, double dt, const double *vel0, const d
         return set_error(SLB_ERR_INVALID, "slb_deadreckon_update_pose: bad argument");
     if (n == 0) return SLB_OK;
     if (need_device("slb_deadreckon_update_pose: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
-    slbd::dr_update_pose_kernel<<<(unsigned)((n + 63) / 64), 64, 0, (cudaStream_t)stream>>>(n, dt, vel0, vel1, velcov, prev_pose, prev_cov,
-                                                                                          post_pose, post_cov, delta_pose, delta_cov);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(slbd::dr_update_pose_kernel, (unsigned)((n + 63) / 64), 64, 0, (cudaStream_t)stream, n, dt, vel0, vel1, velcov,
+                  prev_pose, prev_cov, post_pose, post_cov, delta_pose, delta_cov);
 }
 
 }  // extern "C"

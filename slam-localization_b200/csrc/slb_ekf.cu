@@ -410,12 +410,8 @@ int slb_ekf_predict(int64_t n, double *err, double *P, const double *F, const do
     if (need_device("slb_ekf_predict: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
     constexpr int WPB = 8;
     constexpr size_t smem = (size_t)WPB * slbd::EKP_SM * 8;
-    auto kern = slbd::ekf_predict_kernel<WPB>;
-    SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<(unsigned)((n + WPB - 1) / WPB), WPB * 32, smem, (cudaStream_t)stream>>>(n, err, P, F, Q);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(slbd::ekf_predict_kernel<WPB>, (unsigned)((n + WPB - 1) / WPB), WPB * 32, smem, (cudaStream_t)stream, n, err, P,
+                  F, Q);
 }
 
 int slb_ekf_update(int64_t n, int m, const double *mu, double *P, const double *z, const double *H, const double *R, int gate,
@@ -426,12 +422,8 @@ int slb_ekf_update(int64_t n, int m, const double *mu, double *P, const double *
     if (need_device("slb_ekf_update: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
     constexpr int WPB = 8;
     constexpr size_t smem = (size_t)WPB * (slbd::EkuCfg<45, 3>::SM + 46) * 8;
-    auto kern = slbd::ekf_update_kernel<3, WPB>;
-    SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<(unsigned)((n + WPB - 1) / WPB), WPB * 32, smem, (cudaStream_t)stream>>>(n, mu, P, z, H, R, gate, ret, accepted);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(slbd::ekf_update_kernel<3, WPB>, (unsigned)((n + WPB - 1) / WPB), WPB * 32, smem, (cudaStream_t)stream, n, mu, P,
+                  z, H, R, gate, ret, accepted);
 }
 
 int slb_ekf_single_update(int64_t n, int m, double *mu, const double *err, double *P, const double *z, const double *H,
@@ -442,11 +434,8 @@ int slb_ekf_single_update(int64_t n, int m, double *mu, const double *err, doubl
     if (need_device("slb_ekf_single_update: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
     constexpr int WPB = 8;
     constexpr size_t smem = (size_t)WPB * (slbd::EkuCfg<15, 3>::SM + 16) * 8;
-    auto kern = slbd::ekf_single_update_kernel<3, WPB>;
-    kern<<<(unsigned)((n + WPB - 1) / WPB), WPB * 32, smem, (cudaStream_t)stream>>>(n, mu, err, P, z, H, R, gate, accepted);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(slbd::ekf_single_update_kernel<3, WPB>, (unsigned)((n + WPB - 1) / WPB), WPB * 32, smem, (cudaStream_t)stream, n,
+                  mu, err, P, z, H, R, gate, accepted);
 }
 
 int slb_ekf_clone(int64_t n, double *mu, double *err, double *P, void *stream) {
@@ -454,10 +443,7 @@ int slb_ekf_clone(int64_t n, double *mu, double *err, double *P, void *stream) {
     if (n == 0) return SLB_OK;
     if (need_device("slb_ekf_clone: no CUDA device (this engine has no CPU fallback)") != SLB_OK) return SLB_ERR_NO_DEVICE;
     const int64_t work = n * (45 * 45 + 32 + 30);
-    slbd::ekf_clone_kernel<<<(unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream>>>(n, mu, err, P);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(slbd::ekf_clone_kernel, (unsigned)((work + 255) / 256), 256, 0, (cudaStream_t)stream, n, mu, err, P);
 }
 
 }  // extern "C"

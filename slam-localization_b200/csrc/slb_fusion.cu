@@ -284,20 +284,13 @@ namespace slb {
 template <int D, int OP>
 static int launch_dm(int64_t n, const double *x1, const double *C1, const double *x2, const double *C2,
                      double *xo, double *Co, cudaStream_t s) {
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
     const int64_t tiles = (n + 31) / 32;
     int64_t blocks = (tiles + slbd::FUSE_WARPS - 1) / slbd::FUSE_WARPS;
-    const int64_t cap = (int64_t)sms * 16;  // persistent: a multiple of the SM count
+    const int64_t cap = (int64_t)sm_count() * 16;  // persistent: a multiple of the SM count
     if (blocks > cap) blocks = cap;
     if (blocks < 1) blocks = 1;
-    auto kern = slbd::datamodel_kernel<D, OP>;
-    SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)slbd::FuseCfg<D>::SMEM));
-    kern<<<(int)blocks, slbd::FUSE_WARPS * 32, slbd::FuseCfg<D>::SMEM, s>>>(n, x1, C1, x2, C2, xo, Co);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(slbd::datamodel_kernel<D, OP>, (int)blocks, slbd::FUSE_WARPS * 32, slbd::FuseCfg<D>::SMEM, s, n, x1, C1, x2,
+                  C2, xo, Co);
 }
 
 int launch_fusion(int d, int64_t n, int op, const double *x1, const double *C1, const double *x2,

@@ -52,6 +52,7 @@ namespace slb {
 
 int set_error(int code, const char *what, cudaError_t ce = cudaSuccess);
 void count_launch(int n = 1);
+int sm_count();  // SMs of the current device
 // SLB_ERR_NO_DEVICE with message `msg` when no CUDA device is visible (there is no CPU fallback), else SLB_OK and the
 // device count in *ndev
 int need_device(const char *msg, int *ndev = nullptr);
@@ -61,6 +62,26 @@ int need_device(const char *msg, int *ndev = nullptr);
         cudaError_t e_ = (call);                                              \
         if (e_ != cudaSuccess) return slb::set_error(SLB_ERR_CUDA, #call, e_); \
     } while (0)
+
+// More than 48 KB of dynamic shared memory needs the kernel's opt-in.  (Static shared memory counts against the 48 KB
+// too; the one kernel with both, consistency_kernel, adds 384 bytes to requests that skip the range 47.6 .. 48 KB.)
+// The occupancy calculator judges a kernel by the opt-in it already has, so a launcher that asks it opts in first.
+template <class... P>
+int allow_smem(void (*kern)(P...), size_t smem) {
+    if (smem > 48 * 1024) SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    return SLB_OK;
+}
+
+// Every kernel launch of the library: the shared-memory opt-in, the launch, one count of slb_launch_count, and
+// SLB_ERR_CUDA if the launch failed.
+template <class... P, class... A>
+int launch(void (*kern)(P...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, A... args) {
+    if (allow_smem(kern, smem) != SLB_OK) return SLB_ERR_CUDA;
+    kern<<<grid, block, smem, s>>>(args...);
+    count_launch();
+    SLB_CUDA(cudaGetLastError());
+    return SLB_OK;
+}
 
 // Every entry point that takes a handle runs on the handle's device and leaves the caller's current device as it
 // found it (several handles on several devices may be driven from one thread).
@@ -94,11 +115,10 @@ struct FilterArgs {
     int gate;
     int nk, nl, k;
     // per-instance noise (slb_set_noise_layout): qs / rs = doubles between consecutive instances' Q / R, 0 = one matrix
-    // shared by the batch; the launchers select the kernels' per-instance instantiations when one of them is set.  The
-    // two fill alignment holes: the kernels' parameter layout (size, every other member's offset) is as without them.
+    // shared by the batch; the launchers select the kernels' per-instance instantiations when one of them is set.  qs
+    // fills the alignment hole after k; rs is followed by 4 bytes of padding.
     int qs;
     int32_t *misc;
-    int prefetch;     // USCKF step: L2-prefetch the record of instance (i + prefetch); 0 = off
     int rs;
     double *mu_out;   // optional instance-major copy of the posterior means (may be mapped host memory), B x out_len
     int out_off, out_len;  // the slice [out_off, out_off + out_len) of the q-vector that goes to mu_out

@@ -1442,33 +1442,18 @@ int launch_msckf_update(int mm, const FilterArgs &a, cudaStream_t s) {
     if (mm != SLB_MM_MSCKF_REPROJ) return set_error(SLB_ERR_INVALID, "msckf: unsupported measurement model");
     if (a.k < 1 || a.k > 10 || a.m > slbd::MS_MMAX || a.m < 2)
         return set_error(SLB_ERR_INVALID, "msckf update: needs 1..10 clones and 2 <= m <= 100");
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const size_t smem = (size_t)slbd::MS_SMEM_DOUBLES * sizeof(double);
-    SLB_CUDA(cudaFuncSetAttribute(slbd::msckf_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int grid = a.B < sms ? a.B : sms;  // one persistent CTA per SM
-    slbd::msckf_update_kernel<<<grid, slbd::MS_T, smem, s>>>(a);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    const int sms = sm_count(), grid = a.B < sms ? a.B : sms;  // one persistent CTA per SM
+    return launch(slbd::msckf_update_kernel, grid, slbd::MS_T, (size_t)slbd::MS_SMEM_DOUBLES * sizeof(double), s, a);
 }
 
 int launch_msckf_update_ekf(int mm, const FilterArgs &a, cudaStream_t s) {
     if (mm != SLB_MM_MSCKF_REPROJ) return set_error(SLB_ERR_INVALID, "msckf: unsupported measurement model");
     if (a.k < 1 || a.k > 10 || a.m > slbd::MS_MMAX || a.m < 2 || (a.m & 1))
         return set_error(SLB_ERR_INVALID, "msckf EKF update: needs 1..10 clones and an even 2 <= m <= 100");
-    int dev = 0, sms = 148;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-    const size_t smem = (size_t)slbd::ME_SMEM_DOUBLES * sizeof(double);
-    SLB_CUDA(cudaFuncSetAttribute(slbd::msckf_ekf_update_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int grid = a.B < sms ? a.B : sms;  // one persistent CTA per SM
-    slbd::msckf_rdiag_kernel<<<1, 256, 0, s>>>(a.R, a.m, a.misc);
-    slbd::msckf_ekf_update_kernel<<<grid, slbd::MS_T, smem, s>>>(a);
-    count_launch(2);
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    const int sms = sm_count(), grid = a.B < sms ? a.B : sms;  // one persistent CTA per SM
+    const int rc = launch(slbd::msckf_rdiag_kernel, 1, 256, 0, s, a.R, a.m, a.misc);
+    if (rc != SLB_OK) return rc;
+    return launch(slbd::msckf_ekf_update_kernel, grid, slbd::MS_T, (size_t)slbd::ME_SMEM_DOUBLES * sizeof(double), s, a);
 }
 
 }  // namespace slb

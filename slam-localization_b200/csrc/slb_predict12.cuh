@@ -476,11 +476,7 @@ int launch_predict12(const FilterArgs &a, cudaStream_t s) {
     constexpr size_t smem = (size_t)WPB * slbd::PRED_SM * sizeof(double);
     auto kern = a.qs ? slbd::predict12_kernel<PM, WPB, ROW0, MU0, CROSS, true>
                      : slbd::predict12_kernel<PM, WPB, ROW0, MU0, CROSS, false>;
-    SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    kern<<<(a.B + WPB - 1) / WPB, WPB * 32, smem, s>>>(a);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(kern, (a.B + WPB - 1) / WPB, WPB * 32, smem, s, a);
 }
 
 }  // namespace slb

@@ -1,5 +1,5 @@
 // slb_ptx.cuh -- the PTX and warp primitives every kernel of the library shares: warp reductions and broadcasts, the
-// mbarrier, TMA bulk copies (global <-> shared, L2 prefetch), 8-byte cp.async (LDGSTS) and the m8n8k4 FP64 DMMA.
+// mbarrier, TMA bulk copies (global <-> shared), 8-byte cp.async (LDGSTS) and the m8n8k4 FP64 DMMA.
 // Each is inline asm (or a shuffle intrinsic), so a -fmad=false translation unit emits the same instructions.
 #pragma once
 #include "slb_math.cuh"
@@ -43,9 +43,6 @@ SLB_DEV void bulk_s2g(void *gdst, const void *ssrc, unsigned bytes) {
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;\n cp.async.bulk.commit_group;\n" ::"l"(gdst),
                  "r"(saddr(ssrc)), "r"(bytes)
                  : "memory");
-}
-SLB_DEV void bulk_prefetch_l2(const void *gsrc, unsigned bytes) {
-    asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;\n" ::"l"(gsrc), "r"(bytes) : "memory");
 }
 SLB_DEV void bulk_store_wait() { asm volatile("cp.async.bulk.wait_group.read 0;\n" ::: "memory"); }
 SLB_DEV void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory"); }

@@ -584,30 +584,22 @@ static int launch_ukf_t(bool predict, bool update, const FilterArgs &a, cudaStre
     constexpr size_t smem = (size_t)(TPB / 32) * slbd::UkfWarp<L, MM::M, G>::DOUBLES * sizeof(double);
     static_assert(smem <= 227 * 1024, "instance records exceed shared memory");
     const int ipb = TPB / G;
-    const int grid = (a.B + ipb - 1) / ipb;
-    auto go = [&](auto kern) -> int {
-        SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        kern<<<grid, TPB, smem, s>>>(a);
-        count_launch();
-        SLB_CUDA(cudaGetLastError());
-        return SLB_OK;
-    };
+    void (*kern)(FilterArgs);
     const bool pin = (predict && a.qs) || (update && a.rs);
     if (update && a.nis) {
-        if (pin) return predict ? go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true, true, true>)
-                                : go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true, true, true>);
-        return predict ? go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true, false, true>)
-                       : go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true, false, true>);
-    }
-    if (pin) {
-        if (predict && update) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true, true>);
-        if (predict) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, false, true>);
-        if (update) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true, true>);
-    }
-    if (predict && update) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true>);
-    if (predict) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, false>);
-    if (update) return go(slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true>);
-    return set_error(SLB_ERR_INVALID, "ukf: nothing to do");
+        if (pin) kern = predict ? slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true, true, true>
+                                : slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true, true, true>;
+        else kern = predict ? slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true, false, true>
+                            : slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true, false, true>;
+    } else if (pin) {
+        if (predict && update) kern = slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true, true>;
+        else if (predict) kern = slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, false, true>;
+        else kern = slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true, true>;
+    } else if (predict && update) kern = slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, true>;
+    else if (predict) kern = slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, true, false>;
+    else if (update) kern = slbd::ukf_kernel<L, PM, MM, G, TPB, MINB, false, true>;
+    else return set_error(SLB_ERR_INVALID, "ukf: nothing to do");
+    return launch(kern, (a.B + ipb - 1) / ipb, TPB, smem, s, a);
 }
 
 int launch_ukf(int layout, int pm, int mm, bool predict, bool update, const FilterArgs &a, cudaStream_t s) {

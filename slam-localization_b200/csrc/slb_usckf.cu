@@ -14,8 +14,6 @@
 //   construction (same algebra as :152-154, without the explicit inverse).
 // update (Usckf.hpp:260-308) and the fused predict+update step: slb_usckf_step.cuh (record resident in shared
 //   memory, blocked square-root-free factorisation on DMMA accumulator tiles, sigma points streamed per 16 columns).
-#include <cstdlib>
-
 #include "slb_predict12.cuh"
 #include "slb_usckf_step.cuh"
 
@@ -129,48 +127,20 @@ static int launch_step_t(const FilterArgs &a, cudaStream_t s) {
     // The PIN instantiation's RP extra doubles per warp (R staged next to z) fit in the slack of the same CTA shape for
     // every built shape: see the static_assert below.
     constexpr size_t pw = (size_t)(PIN ? C::SMP : C::SM) * sizeof(double);
-    constexpr size_t SM_BYTES = 228 * 1024, CTA_MAX = 227 * 1024, RSV = 1024;
-#ifdef SLB_USCKF_WPB
-    constexpr int WPB = SLB_USCKF_WPB;   // experiment knob (compile time)
-#else
+    constexpr size_t SM_BYTES = 228 * 1024, RSV = 1024;
     constexpr int WPB = 2 * (6 * pw + RSV) <= SM_BYTES ? 6 : 4;
-#endif
     constexpr size_t smem = (size_t)WPB * pw;
     constexpr int fit = (int)(SM_BYTES / (smem + RSV));
     constexpr int cap = 12 / WPB < 1 ? 1 : 12 / WPB;
     constexpr int MINB = fit > cap ? cap : fit < 1 ? 1 : fit;
-#ifndef SLB_USCKF_WPB
     {   // per-instance noise must not cost the fused step a CTA
         constexpr size_t pw0 = (size_t)C::SM * sizeof(double);
         constexpr int WPB0 = 2 * (6 * pw0 + RSV) <= SM_BYTES ? 6 : 4;
         constexpr int fit0 = (int)(SM_BYTES / ((size_t)WPB0 * pw0 + RSV));
         static_assert(!PIN || (WPB == WPB0 && fit >= (fit0 < 12 / WPB0 ? fit0 : 12 / WPB0)), "PIN costs occupancy");
     }
-#endif
-    auto kern = slbd::usckf_step_kernel<SLB_PM_USCKF_TEST, NK, NL, PRED, UPD, WPB, MINB, PIN, NIS>;
-    SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    // L2 prefetch distance in instances: SLB_USCKF_PREFETCH waves of (SMs x resident warps); default off (measured: no
-    // gain at 0 / 1 / 2 / 4 waves, and 16 % more DRAM reads at the full fleet size)
-    static const int ahead = [] {
-        const char *e = getenv("SLB_USCKF_PREFETCH");
-        int dev = 0, sms = 148;
-        cudaGetDevice(&dev);
-        cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-        return (e ? atoi(e) : 0) * sms * WPB * MINB;
-    }();
-    FilterArgs b = a;
-    b.prefetch = ahead;
-    // experiment knob: SLB_USCKF_CTAS=1|2 pads the dynamic shared memory so that only that many CTAs fit per SM
-    static const size_t pad = [] {
-        const char *e = getenv("SLB_USCKF_CTAS");
-        const int n = e ? atoi(e) : 0;
-        return n == 1 ? (size_t)(200 * 1024) - smem : n == 2 ? (size_t)(110 * 1024) - smem : (size_t)0;
-    }();
-    if (pad) SLB_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(smem + pad)));
-    kern<<<(a.B + WPB - 1) / WPB, WPB * 32, smem + pad, s>>>(b);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(slbd::usckf_step_kernel<SLB_PM_USCKF_TEST, NK, NL, PRED, UPD, WPB, MINB, PIN, NIS>, (a.B + WPB - 1) / WPB,
+                  WPB * 32, smem, s, a);
 }
 
 template <int NK, int NL, bool NIS>
@@ -203,10 +173,7 @@ int launch_usckf(int pm, int mm, bool predict, bool update, const FilterArgs &a,
 int launch_usckf_clone(int mode, const FilterArgs &a, cudaStream_t s) {
     if (mode != SLB_STATEK_I && mode != SLB_STATEK_L) return SLB_OK;  // default: break (Usckf.hpp:428)
     const int64_t work = (int64_t)a.B * (13 + 288);
-    slbd::usckf_clone_kernel<<<(unsigned)((work + 255) / 256), 256, 0, s>>>(a, mode);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(slbd::usckf_clone_kernel, (unsigned)((work + 255) / 256), 256, 0, s, a, mode);
 }
 
 int launch_usckf_set_measurement(int mode, const FilterArgs &a, cudaStream_t s) {
@@ -215,10 +182,7 @@ int launch_usckf_set_measurement(int mode, const FilterArgs &a, cudaStream_t s) 
     const int len = mode == SLB_STATEK ? a.nk : a.nl;
     if (len == 0) return SLB_OK;
     const int64_t work = (int64_t)a.B * ((N - 36) * N + len);
-    slbd::usckf_set_measurement_kernel<<<(unsigned)((work + 255) / 256), 256, 0, s>>>(a, mode);
-    count_launch();
-    SLB_CUDA(cudaGetLastError());
-    return SLB_OK;
+    return launch(slbd::usckf_set_measurement_kernel, (unsigned)((work + 255) / 256), 256, 0, s, a, mode);
 }
 
 }  // namespace slb

@@ -27,17 +27,6 @@
 #pragma once
 #include "slb_predict12.cuh"
 
-// Experiment knob (compile time): -DSLB_USCKF_CTA_SYNC=1 re-aligns the warps of a CTA a few times per instance so that
-// they walk the (104 KB, fully unrolled) instruction stream together and share instruction-cache lines.
-#ifndef SLB_USCKF_CTA_SYNC
-#define SLB_USCKF_CTA_SYNC 0
-#endif
-#if SLB_USCKF_CTA_SYNC
-#define SLB_CTA_SYNC() __syncthreads()
-#else
-#define SLB_CTA_SYNC() ((void)0)
-#endif
-
 namespace slbd {
 
 template <int NK_, int NL_>
@@ -328,10 +317,7 @@ struct PanelStep {
                 for (int I = J; I < NT; ++I) dmma884(s.c0[I][J], s.c1[I][J], f[I], g);
             }
         }
-        if (Q == 3 || P == C::NPAN - 1) {
-            sigma_group<C, (P >> 2)>(s, mus, Lf, Wg, dv, lane);
-            SLB_CTA_SYNC();
-        }
+        if (Q == 3 || P == C::NPAN - 1) sigma_group<C, (P >> 2)>(s, mus, Lf, Wg, dv, lane);
         PanelStep<C, P + 1>::run(s, mus, Lf, Lraw, Wg, dv, lane);
     }
 };
@@ -574,8 +560,6 @@ __global__ void __launch_bounds__(WPB * 32, MINB) usckf_step_kernel(slb::FilterA
         mbar_expect_tx(bar, (C::PSTR + C::QS) * 8);
         bulk_g2s(Ps, Pg, C::PSTR * 8, bar);
         bulk_g2s(mus, mug, C::QS * 8, bar);
-        // the record a warp of a later wave of CTAs will want: pull it into L2 now (one wave = SMs x resident warps)
-        if (a.prefetch > 0 && inst + a.prefetch < a.B) bulk_prefetch_l2(Pg + (size_t)a.prefetch * a.pstride, C::PSTR * 8);
     }
     // the measurement and the control input are fetched now: with the zero-copy *_step_host they live in mapped host
     // memory and their PCIe latency must not sit in the middle of the step
@@ -600,13 +584,11 @@ __global__ void __launch_bounds__(WPB * 32, MINB) usckf_step_kernel(slb::FilterA
     }
     __syncwarp();
     mbar_wait(bar, 0);
-    SLB_CTA_SYNC();
     int st = 0;
     bool dirty = false;
     if (PRED) {
         st = predict12_block<PM, true, PIN>(ResidentView<C::N>{Ps}, mus + 26, u, a.dt, scr, a.Q, qv, NK + NL, mus + 26, lane, dirty);
     }
-    if (PRED) SLB_CTA_SYNC();
     double m2 = __longlong_as_double(0x7ff8000000000000ll);   // NaN
     if (UPD) st |= usckf_update_smem<NK, NL, PIN>(Ps, mus, scr, zs, Rs, a, lane, dirty, m2);
     if (NIS && lane == 0) a.nis[inst] = m2;
